@@ -2,6 +2,7 @@
 """bench.py -- ray-cell updates/s of the post-flight mapping path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c4] [--configs all|none|c1,c4,..]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (P0 pose integration -> ray set-up -> grid replay) over one batch of
 synthetic logs.  Headline workload: BASELINE config 3 AS WRITTEN -- the 4096-flight optical-flow drift ensemble
@@ -22,6 +23,11 @@ Printed JSON line (rank 0):
   configs      one record per BASELINE configuration c1..c5 at this N (value, e2e, hash[, hash_n1]); c3_weak is
                round 1's N x 4096-flight variant, kept for continuity
   --impl reference   times the reference CPU implementation as the main line (rank 0 only)
+
+--dump-outputs DIR writes, after the timed steps, what the headline's last timed step computed as DIR/<name>.npy
+(float32), so that two builds can be compared output for output on the same seeded logs:
+  c3   grids [k, 400, 400] and poses x, y [k, 3000] of k = 64 flights drawn with a fixed seed from the ensemble (42 MB)
+  c4   grid_rows [512, 16384]: 512 rows of the one grid drawn with a fixed seed (34 MB)
 """
 from __future__ import annotations
 
@@ -42,11 +48,15 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # a run leaves the tree as it found it (it may be read-only)
 
 METRIC = "ray_cell_updates_per_s"
 DATA = "synthetic (seeded logs, SURVEY.md 8(d); ranges on the ToF sensor's 1 mm lattice like a real scan log)"
 LOG_KEYS = ("t_ms", "of_rate_x", "of_rate_y", "h_m", "yaw_deg", "of_q", "ranges")
 M64 = (1 << 64) - 1
+DUMP_SEED = 20240607    # fixed: the sample --dump-outputs writes is the same in every run and at every N
+DUMP_FLIGHTS = 64
+DUMP_ROWS = 512
 
 
 def describe(w, n_gpus, flights_total=None, scaling="strong"):
@@ -78,6 +88,26 @@ def combine_hashes(per_grid: np.ndarray, first_id: int) -> int:
     for i, g in enumerate(per_grid.tolist()):
         h = (h + _mix64(int(g) ^ _mix64(first_id + i))) & M64
     return h
+
+
+def dump_sample(n: int, k: int) -> np.ndarray:
+    """k of the indices [0, n), drawn with DUMP_SEED, ascending."""
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(k, n), replace=False))
+
+
+def write_outputs(cx, out_dir, part):
+    """Gather every rank's piece of the sample on rank 0 (shards are contiguous and in rank order, so the
+    concatenation is in sample order) and write one float32 .npy per array."""
+    parts = [part]
+    if cx.world > 1:
+        parts = [None] * cx.world if cx.rank == 0 else None
+        cx.dist.gather_object(part, parts, dst=0)
+    if cx.rank != 0:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    for name in sorted({k for q in parts for k in q}):
+        a = np.concatenate([q[name] for q in parts if name in q], axis=0).astype(np.float32, copy=False)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -444,6 +474,12 @@ def run_flights(cx, w, first, cnt, total, label, verify_n1, headline=False, vari
     l0 = m.kernel_launches()
     ms = cx.timed(step_device, steps, 0)
     launches = m.kernel_launches() - l0
+    outputs = {}
+    if headline and args.dump_outputs and active:
+        # what the last timed step left on the device, for the flights of the fixed sample that this rank holds
+        ids = dump_sample(total, DUMP_FLIGHTS)
+        mine = torch.as_tensor(ids[(ids >= first) & (ids < first + F)] - first, dtype=torch.long, device=cx.dev)
+        outputs = {"grids": d_grids[mine].float().cpu().numpy(), "x": d_x[mine].cpu().numpy(), "y": d_y[mine].cpu().numpy()}
     kms = [0.0, 0.0, 0.0]
     if active:
         kms, _ = m.profile_collect()
@@ -534,7 +570,7 @@ def run_flights(cx, w, first, cnt, total, label, verify_n1, headline=False, vari
         rec["hash_n1"] = f"{cx.sum_hash(h1):016x}"
         rec["hash_matches_n1"] = rec["hash_n1"] == rec["hash"]
     extra = {"U_rank": U, "kms": kms, "launches": int(launches), "clocks": clk, "steps": steps,
-             "d_pinned": d if (active and headline) else None, "F": F}
+             "d_pinned": d if (active and headline) else None, "F": F, "outputs": outputs}
     return rec, extra
 
 
@@ -565,7 +601,7 @@ def run_p0_variants(cx, w):
     return out
 
 
-def run_c4(cx, verify_n1):
+def run_c4(cx, verify_n1, headline=False):
     """Config 4: ONE 16384^2 grid; every rank owns a band of rows (uqs_row_band), replays the whole log into it,
     one ncclAllGather inside the library assembles the grid on every rank."""
     m, synth, torch, args = cx.m, cx.synth, cx.torch, cx.args
@@ -581,7 +617,7 @@ def run_c4(cx, verify_n1):
     grid = torch.empty((p.H, p.W), dtype=torch.int8, device=cx.dev)
     h_grid = cx.pinned((p.H, p.W), torch.int8) if cx.rank == 0 else None
     torch.cuda.synchronize()
-    steps, warmup = max(2, min(args.steps, 3)), 2
+    steps, warmup = (args.steps, args.warmup) if headline else (max(2, min(args.steps, 3)), 2)
 
     def step_device(want_stats=False, gather=True):
         return m.replay_banded_dev(p, NF, dv["x"].data_ptr(), dv["y"].data_ptr(), dv["yaw"].data_ptr(), dv["ranges"].data_ptr(),
@@ -600,6 +636,11 @@ def run_c4(cx, verify_n1):
     l0 = m.kernel_launches()
     ms = cx.timed(step_device, steps, 0)
     launches = m.kernel_launches() - l0
+    outputs = {}
+    if headline and args.dump_outputs and cx.rank == 0:
+        # every rank holds the whole grid after the gather; rank 0 writes the fixed sample of its rows
+        rows = torch.as_tensor(dump_sample(p.H, DUMP_ROWS), dtype=torch.long, device=cx.dev)
+        outputs = {"grid_rows": grid[rows].float().cpu().numpy()}
     kms, _ = m.profile_collect()
     m.set_profiling(False)
     # the same step without the exchange (what the NCCL gather of the bands costs), and every rank's own kernel time
@@ -639,7 +680,8 @@ def run_c4(cx, verify_n1):
         cx.barrier()
         rec["hash_n1"] = f"{cx.sum_hash(h1):016x}"
         rec["hash_matches_n1"] = rec["hash_n1"] == rec["hash"]
-    extra = {"U_rank": U, "kms": kms, "launches": int(launches), "steps": steps, "n_rays": NF * 32, "n_frames": NF, "cells": p.W * p.H}
+    extra = {"U_rank": U, "kms": kms, "launches": int(launches), "steps": steps, "n_rays": NF * 32, "n_frames": NF, "cells": p.W * p.H,
+             "outputs": outputs}
     return rec, extra
 
 
@@ -773,6 +815,8 @@ def main():
     ap.add_argument("--no-verify-n1", action="store_true", help="skip replaying every job on rank 0 alone for hash_n1")
     ap.add_argument("--engine", type=int, default=0, help="0 auto, 1 sub-tiles, 2 resident (tuning experiments)")
     ap.add_argument("--flight-warps", type=int, default=0, help="warps per resident CTA (0 = library default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of what the headline's last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
@@ -801,7 +845,7 @@ def main():
         n_rays, n_frames_r, cells = F_rank * NF * 32, F_rank * NF, w3.W * w3.W * F_rank
         kernel_name = "k_replay_flights (resident engine)"
     else:
-        head, ex = run_c4(cx, verify)
+        head, ex = run_c4(cx, verify, headline=True)
         configs["c4"] = head
         w4 = synth.CONFIGS["c4"]
         cfg = {"workload": head["workload"], "samples": head["samples"], "frames": head["frames"], "beams_per_sample": 64,
@@ -809,6 +853,10 @@ def main():
                "scaling": "strong", "l2_policy": "log + ray records (>800 MB) exceed the 126 MB L2; no flush needed"}
         n_rays, n_frames_r, cells = ex["n_rays"], ex["n_frames"], ex["cells"] // world
         kernel_name = "k_replay_tiles (sub-tile engine, owned row band)"
+
+    if args.dump_outputs:
+        write_outputs(cx, args.dump_outputs, ex["outputs"])
+    ex["outputs"] = None
 
     # ---- roofline of the dominant kernel (replay), rank 0's share of the job -----------------------------------------------
     roofline = cpu = None

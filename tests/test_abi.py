@@ -43,9 +43,9 @@ def test_header_compiles_as_c99():
     assert r.returncode == 0, r.stderr
 
 
-def test_params_struct_layout_matches_header(pkg):
+def test_params_struct_layout_matches_header(pkg, tmp_path):
     src = '#include <stdio.h>\n#include <stddef.h>\n#include "uqs_mapping.h"\nint main(void){printf("%zu %zu %zu %zu %zu", sizeof(uqs_params), offsetof(uqs_params,res_m), offsetof(uqs_params,lo_free), sizeof(uqs_stats), offsetof(uqs_stats,domain_errors));return 0;}\n'
-    exe = "/tmp/uqs_layout_probe"
+    exe = str(tmp_path / "uqs_layout_probe")
     r = subprocess.run(["gcc", "-I", os.path.join(ROOT, "include"), "-x", "c", "-", "-o", exe], input=src, text=True, capture_output=True)
     assert r.returncode == 0, r.stderr
     out = subprocess.check_output([exe], text=True).split()
