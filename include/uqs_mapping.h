@@ -135,11 +135,12 @@ int  uqs_set_tuning(int subtile_w, int subtile_h, int time_slices);
 int  uqs_set_engine(int engine, int flight_warps);
 /* Lane layout of the resident engine's free-space steps: 0 = the 32 beams of a frame x 1 step per warp
  * instruction, 1 = the 8 beams of one sensor x 4 consecutive steps (fewer shared-memory bank conflicts).
- * -1 = the built-in choice.  Identical bytes either way. */
+ * -1 = the built-in choice.  Identical bytes either way.  uqs_replay_frontier[_dev] ignores this knob. */
 int  uqs_set_fan_layout(int on);
 /* Resident engine with a dedicated decode warp: 0 = every warp decodes every NW-th frame of its flight, 1 = an
  * extra producer warp per CTA does nothing but decode frames into the shared-memory ring, two frames ahead of the
- * consumer warps (4, 8 or 16 of them).  -1 = the built-in choice.  Identical bytes either way. */
+ * consumer warps (4, 8 or 16 of them).  -1 = the built-in choice.  Identical bytes either way.
+ * uqs_replay_frontier[_dev] ignores this knob. */
 int  uqs_set_decode_warp(int on);
 /* Measurement knob: adds `steps` (0..8) to every frame's collision bound K0 (always safe; identical bytes): what one
  * collision-checked step per frame costs the resident engine. */
@@ -270,6 +271,33 @@ int uqs_replay_recentering(const uqs_params* p, int n_frames, const float* x, co
 /* N3: frontier_score_dir() (uav_local_nav.c:356-385) for n queries against one host grid. */
 int uqs_frontier_scores(const uqs_params* p, const int8_t* grid, int n, const float* x, const float* y,
                         const float* yaw_deg, const float* offset_deg, int* scores_out);
+
+/* N3 at the frame a decision was taken: one frontier query (24 bytes, no padding).  Its score is what
+ * frontier_score_dir(x, y, yaw_deg, offset_deg) returns when occ_grid holds flight `flight`'s grid after its frames
+ * 0..frame have been applied -- the map EXPLORE scored against in the control tick of that frame (uav_local_nav.c:
+ * 1715-1736, 2225-2253).  The query carries its own pose (the controller's pose at the tick); pass x[f], y[f], yaw[f]
+ * for the frame's own pose. */
+typedef struct uqs_query {
+  int32_t flight, frame;
+  float   x, y, yaw_deg, offset_deg;
+} uqs_query;
+
+/* uqs_replay_dev plus n_queries frontier queries answered inside the same replay: scores_dev[i] = score of
+ * queries_dev[i] (input order; any order of queries, duplicates and many per frame are fine).  Grids and stats are
+ * byte-identical to uqs_replay_dev with the same arguments (row0 = 0, rows = H: whole grids only); n_queries == 0 is
+ * exactly uqs_replay_dev (scores_dev and queries_dev may then be NULL).  A query with flight outside [0, n_flights) or
+ * frame outside [0, n_frames) returns UQS_ERR_BAD_ARG naming the first such index, before any grid is written (the
+ * check synchronises).  Queries use the fixed origin of p (no recentering).  The engine, sub-tile geometry and time
+ * slicing are chosen as for uqs_replay_dev; the resident engine's probe variant uses the default lane layout, so
+ * uqs_set_fan_layout() and uqs_set_decode_warp() do not apply to this call.  Asynchronous on the current stream. */
+int uqs_replay_frontier_dev(const uqs_params* p, int n_flights, int n_frames,
+                            const float* x_dev, const float* y_dev, const float* yaw_dev, const float* ranges_dev,
+                            int8_t* grids_dev, int accumulate,
+                            int n_queries, const uqs_query* queries_dev, int32_t* scores_dev, uqs_stats* stats);
+/* Host-buffer form (grids start at zero; grids_out may be NULL).  Synchronous. */
+int uqs_replay_frontier(const uqs_params* p, int n_flights, int n_frames, const float* x, const float* y,
+                        const float* yaw_deg, const float* ranges, int8_t* grids_out,
+                        int n_queries, const uqs_query* queries, int32_t* scores_out, uqs_stats* stats);
 
 /* N4: reader of scanlog.bin ("SCLOG2\n" + packed 569-byte scanrec_t records, uav_local_nav.c:1505,1522-1547).
  * Returns the number of qualifying records (> max_records means the buffers were too small), < 0 on error.

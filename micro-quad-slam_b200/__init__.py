@@ -85,6 +85,7 @@ _EXPORTS = [
     "uqs_pose_integrate", "uqs_pose_integrate_dev", "uqs_replay", "uqs_replay_dev", "uqs_replay_flow",
     "uqs_beam_cells", "uqs_frame_bounds", "uqs_sincosf_batch", "uqs_measure_rmw_peak", "uqs_measure_atoms_peak",
     "uqs_beams_from_scans", "uqs_beams_from_scans_dev", "uqs_replay_recentering", "uqs_frontier_scores",
+    "uqs_replay_frontier", "uqs_replay_frontier_dev",
     "uqs_scanlog_read", "uqs_scanlog_count", "uqs_navlog_read", "map_recenter_shift", "map_recentre_if_needed", "frontier_score_dir",
     # multi-GPU
     "uqs_flight_shard", "uqs_row_band", "uqs_comm_unique_id", "uqs_comm_init_rank", "uqs_comm_destroy", "uqs_comm_nranks",
@@ -138,6 +139,8 @@ def lib() -> C.CDLL:
     L.uqs_beams_from_scans.argtypes = [C.c_longlong, vp, C.c_float, vp, vp]
     L.uqs_replay_recentering.argtypes = [C.POINTER(Params), ip, vp, vp, vp, vp, vp, vp, C.POINTER(C.c_int), vp, ip, C.POINTER(Stats)]
     L.uqs_frontier_scores.argtypes = [C.POINTER(Params), vp, ip, vp, vp, vp, vp, vp]
+    L.uqs_replay_frontier.argtypes = [C.POINTER(Params), ip, ip, vp, vp, vp, vp, vp, ip, vp, vp, C.POINTER(Stats)]
+    L.uqs_replay_frontier_dev.argtypes = [C.POINTER(Params), ip, ip, vp, vp, vp, vp, vp, ip, ip, vp, vp, C.POINTER(Stats)]
     L.uqs_scanlog_read.restype = C.c_long
     L.uqs_scanlog_read.argtypes = [C.c_char_p, ip, C.c_long] + [vp] * 11
     L.uqs_scanlog_count.restype = C.c_long
@@ -455,6 +458,52 @@ def frontier_scores(p: Params, grid, x, y, yaw_deg, offset_deg):
     out = np.empty(x.size, np.int32)
     _check(lib().uqs_frontier_scores(C.byref(p), _ptr(g), x.size, _ptr(x), _ptr(y), _ptr(yaw_deg), _ptr(offset_deg), _ptr(out)))
     return out
+
+
+# ``uqs_query``: 24 bytes, no padding (include/uqs_mapping.h)
+QUERY_DTYPE = np.dtype([("flight", "<i4"), ("frame", "<i4"), ("x", "<f4"), ("y", "<f4"), ("yaw_deg", "<f4"),
+                        ("offset_deg", "<f4")])
+
+
+def make_queries(flight, frame, x, y, yaw_deg, offset_deg) -> np.ndarray:
+    """Array of ``uqs_query`` records from six broadcastable columns."""
+    cols = np.broadcast_arrays(*(np.asarray(a) for a in (flight, frame, x, y, yaw_deg, offset_deg)))
+    q = np.empty(cols[0].size, QUERY_DTYPE)
+    for name, c in zip(QUERY_DTYPE.names, cols):
+        q[name] = c.ravel()
+    return q
+
+
+def replay_frontier(p: Params, x, y, yaw_deg, ranges, queries, want_grids: bool = True):
+    """``uqs_replay_frontier``: the replay of ``replay`` plus frontier_score_dir for every query against its flight's
+    grid after frames 0..frame.  Returns (grids [F,H,W] int8 or None, scores [n] int32, stats dict)."""
+    x = _f32(x)
+    if x.ndim == 1:
+        x = x[None]
+    F, N = x.shape
+    y, yaw_deg = _f32(y).reshape(F, N), _f32(yaw_deg).reshape(F, N)
+    ranges = _f32(ranges).reshape(F, N, BEAMS_PER_FRAME)
+    q = np.ascontiguousarray(queries, QUERY_DTYPE)
+    grids = np.empty((F, p.H, p.W), np.int8) if want_grids else None
+    scores = np.empty(q.size, np.int32)
+    st = Stats()
+    _check(lib().uqs_replay_frontier(C.byref(p), F, N, _ptr(x), _ptr(y), _ptr(yaw_deg), _ptr(ranges),
+                                     _ptr(grids) if grids is not None else None, q.size, _ptr(q) if q.size else None,
+                                     _ptr(scores) if q.size else None, C.byref(st)))
+    return grids, scores, st.as_dict()
+
+
+def replay_frontier_dev(p: Params, n_flights: int, n_frames: int, x_ptr: int, y_ptr: int, yaw_ptr: int, ranges_ptr: int,
+                        grids_ptr: int, n_queries: int, queries_ptr: int, scores_ptr: int, accumulate: bool = False,
+                        want_stats: bool = False):
+    """``uqs_replay_frontier_dev`` on raw device pointers (queries: ``QUERY_DTYPE`` records, scores: int32);
+    asynchronous unless stats are asked."""
+    st = Stats()
+    _check(lib().uqs_replay_frontier_dev(C.byref(p), n_flights, n_frames, C.c_void_p(x_ptr), C.c_void_p(y_ptr),
+                                         C.c_void_p(yaw_ptr), C.c_void_p(ranges_ptr), C.c_void_p(grids_ptr),
+                                         1 if accumulate else 0, int(n_queries), C.c_void_p(queries_ptr),
+                                         C.c_void_p(scores_ptr), C.byref(st) if want_stats else None))
+    return st.as_dict() if want_stats else None
 
 
 def navlog_read(path: str) -> dict:

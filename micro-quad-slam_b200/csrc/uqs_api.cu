@@ -151,7 +151,7 @@ static cudaError_t zero_counted(void* p, size_t bytes, cudaStream_t st) {
 
 int replay_device(const DevParams& dp, int n_flights, int n_frames, const float* x, const float* y,
                   const float* yaw, const float* ranges, const uint8_t* kind, int8_t* grids,
-                  int accumulate, int row0, int rows, bool reset_stats) {
+                  int accumulate, int row0, int rows, bool reset_stats, const ProbeSet* probes) {
   cudaStream_t st = g_ctx.stream();
   const int gpf = (n_frames + 31) / 32;
   g_ctx.w->boxes_valid = false;                  // set again below once this call's touched boxes exist
@@ -182,8 +182,11 @@ int replay_device(const DevParams& dp, int n_flights, int n_frames, const float*
     }
     if (generic) {
       if (reset_stats) eg = zero_counted(cnt, 8 * sizeof(unsigned long long), st);
+      if (eg != cudaSuccess) return cuda_fail(eg, "memset stats");
+      ProbeArgs PA;
+      if (probes && (rcg = probe_buckets(*probes, 0, n_flights, n_frames, dp.W, 0, 0, 0, 0, 0, 0, &PA))) return rcg;
       KernelTimer t_rep(2);
-      if (eg == cudaSuccess) eg = generic_launch(dp, n_flights, n_frames, x, y, yaw, ranges, kind, grids, accumulate, row0, rows, cnt, st);
+      eg = generic_launch(dp, n_flights, n_frames, x, y, yaw, ranges, kind, grids, accumulate, row0, rows, cnt, st, probes ? &PA : nullptr);
       t_rep.stop();
       if (eg != cudaSuccess) return cuda_fail(eg, "k_replay_generic launch");
       g_ctx.launches += accumulate ? 1 : 2;
@@ -281,9 +284,7 @@ int replay_device(const DevParams& dp, int n_flights, int n_frames, const float*
   }
 
   int ctas_per_sm = 0;
-  e = cudaFuncSetAttribute(k_replay_tiles, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(k_replay_tiles)");
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, k_replay_tiles, kReplayThreads, smem);
+  e = tiles_prepare(probes != nullptr, smem, &ctas_per_sm);
   if (e != cudaSuccess) return cuda_fail(e, "occupancy(k_replay_tiles)");
   if (ctas_per_sm < 1) { set_error("replay kernel does not fit on an SM (smem %zu)", smem); return UQS_ERR_CUDA; }
 
@@ -382,6 +383,19 @@ int replay_device(const DevParams& dp, int n_flights, int n_frames, const float*
         // cells outside a flight's box are never touched: they are zero in a fresh replay
         if (e == cudaSuccess && !accumulate) e = zero_counted(FA.grids, (size_t)nf * dp.W * dp.H, st);
         if (e != cudaSuccess) return cuda_fail(e, "memset before k_replay_flights");
+        if (probes) {
+          int p_ctas = 0;
+          ProbeArgs PA;
+          if ((rc = probe_buckets(*probes, f0, nf, n_frames, dp.W, 0, 0, 0, 0, 0, 0, &PA))) return rc;
+          if ((e = flights_probe_prepare(fnw, fsmem, &p_ctas)) != cudaSuccess) return cuda_fail(e, "k_replay_flights (probes) attributes");
+          if (p_ctas < 1) { set_error("resident engine (probes): %zu B of shared memory do not fit an SM", fsmem); return UQS_ERR_CUDA; }
+          KernelTimer t_rep(2);
+          e = flights_probe_launch(fnw, (unsigned)std::min<long long>(nf, (long long)p_ctas * g_ctx.sm_count), fsmem, st, FA, PA);
+          t_rep.stop();
+          if (e != cudaSuccess) return cuda_fail(e, "k_replay_flights (probes) launch");
+          g_ctx.launches += 2;
+          continue;
+        }
         const unsigned fgrid = (unsigned)std::min<long long>(nf, (long long)f_ctas * g_ctx.sm_count);
         KernelTimer t_rep(2);
         e = flights_launch(fnw, g_ctx.flight_fan, g_ctx.flight_prod, fgrid, fsmem, st, FA);
@@ -434,9 +448,13 @@ int replay_device(const DevParams& dp, int n_flights, int n_frames, const float*
     if (e != cudaSuccess) return cuda_fail(e, "memset job counter");
     unsigned long long want = (A.total_jobs + kReplayWarps - 1) / kReplayWarps;
     unsigned grid = (unsigned)std::min<unsigned long long>(want, (unsigned long long)ctas_per_sm * g_ctx.sm_count);
+    ProbeArgs PA;
+    if (probes && (rc = probe_buckets(*probes, f0, nf, n_frames, dp.W, slices, gps, sw, sh, nsx, nsy, &PA))) return rc;
     KernelTimer t_rep(2);
-    k_replay_tiles<<<grid, kReplayThreads, smem, st>>>(A);
-    e = cudaGetLastError();
+    e = tiles_launch(probes != nullptr, grid, smem, st, A, probes ? PA : ProbeArgs{});
+    if (e == cudaSuccess && probes && slices > 1 &&     // before slice 0's values are overwritten
+        (rc = probe_resolve_slices(PA, (int)probes->slots(), A.grids, A.maps, dp.W, dp.H, slices, gps)))
+      return rc;
     if (e == cudaSuccess && slices > 1) {
       const size_t cells = (size_t)dp.W * rows * nf;
       k_compose_slices<<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(A.grids, A.maps, nf, dp.W, dp.H, slices, row0, rows);

@@ -177,6 +177,27 @@ __device__ __forceinline__ int beam_endpoint(const DevParams& p, float px, float
 
 __device__ __forceinline__ int sext12(uint32_t v) { return ((int)(v << 20)) >> 20; }
 
+// frontier_score_dir(), uav_local_nav.c:356-385, piece by piece (k_frontier_scores and the probe set-up of
+// uqs_frontier.cu share them).  Ray r (0, +15, -15 degrees, :360) of a query: its angle (:367) ...
+__device__ __forceinline__ float frontier_ray_angle(const DevParams& p, float yaw_deg, float offset_deg, int r) {
+  const float ro = (r == 0) ? 0.0f : (r == 1) ? 15.0f : -15.0f;
+  return __fmul_rn(__fadd_rn(__fadd_rn(yaw_deg, offset_deg), ro), p.deg2rad);
+}
+// ... its first sample distance and step (:361-362: d = step, step + step, ... <= 2.5f) ...
+__device__ __forceinline__ float frontier_step(const DevParams& p) { return __fmul_rn(p.res, 2.0f); }
+constexpr float kFrontierRange = 2.5f;
+// ... the cell of the sample at distance d (:373-375; false = off the grid, which ends the ray) ...
+__device__ __forceinline__ bool frontier_point(const DevParams& p, float x, float y, float d, float ca, float sa, int& gx,
+                                               int& gy) {
+  const float px = __fadd_rn(x, __fmul_rn(d, ca));
+  const float py = __fadd_rn(y, __fmul_rn(d, sa));
+  return world_to_grid(p, px, py, gx, gy);
+}
+// ... and the score's weight of the cell's value (:378-383): unknown +3, free +1, occupied -4
+__device__ __forceinline__ int frontier_weight(int v) {
+  return (v >= -1 && v <= 1) ? 3 : (v > 10) ? -4 : (v < -10) ? 1 : 0;
+}
+
 // q(k) = floor((k*n + m/2) / m) without a divide: n2 = 2n, h2 = 2*(m>>1), inv = ceil(2^31/m).
 // Exact for m <= 1289 (t*m < 2^31 with t <= m*m + m/2); m is capped at kMaxRayCells.
 __device__ __forceinline__ int minor_steps(int k, int n2, int h2, uint32_t inv) {

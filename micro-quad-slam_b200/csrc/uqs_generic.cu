@@ -13,11 +13,13 @@
 
 namespace uqs {
 
+// PROBE: after the rays of frame f, the warp reads the flight's frontier probes of frame f from the grid.
+template <bool PROBE>
 __global__ void __launch_bounds__(128)
 k_replay_generic(const __grid_constant__ DevParams p, int n_flights, int n_frames, const float* __restrict__ x,
                  const float* __restrict__ y, const float* __restrict__ yaw_deg, const float* __restrict__ ranges,
                  const uint8_t* __restrict__ kind, int8_t* __restrict__ grids, int row0, int rows,
-                 unsigned long long* __restrict__ stats /* [4]: U, accepted, skipped, domain */) {
+                 unsigned long long* __restrict__ stats /* [4]: U, accepted, skipped, domain */, ProbeArgs Q) {
   const int flight = (int)((blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5);
   const int lane = threadIdx.x & 31;
   if (flight >= n_flights) return;
@@ -25,6 +27,12 @@ k_replay_generic(const __grid_constant__ DevParams p, int n_flights, int n_frame
   const size_t fbase = (size_t)flight * n_frames;
   unsigned long long cells = 0;
   unsigned accepted = 0, skipped = 0;
+  int pb = 0, pe = 0, next_pf = 0x7fffffff;            // this flight's probes [pb, pe), frame of the next one
+  if (PROBE) {
+    pb = Q.start[flight];
+    pe = Q.start[flight + 1];
+    if (pb < pe) next_pf = Q.probes[pb].x;
+  }
   for (int f = 0; f < n_frames; f++) {
     const size_t fi = fbase + f;
     const float px = x[fi], py = y[fi], third = yaw_deg[fi];
@@ -72,6 +80,17 @@ k_replay_generic(const __grid_constant__ DevParams p, int n_flights, int n_frame
       }
       if (lane == 0) cells += (unsigned long long)m + 1ull;
       __syncwarp();                                                 // the next ray may revisit these cells
+    }
+    if (PROBE) {
+      while (next_pf == f) {                                        // the taken probes are a prefix (frame order)
+        const int i = pb + lane;
+        const int4 pr = i < pe ? Q.probes[i] : make_int4(-1, 0, 0, 0);
+        const bool take = pr.x == f;
+        if (take) Q.values[pr.z] = (uint32_t)(int)grid[pr.y];
+        pb += __popc(__ballot_sync(0xffffffffu, take));
+        next_pf = pb < pe ? Q.probes[pb].x : 0x7fffffff;
+      }
+      __syncwarp();                                                 // frame f + 1 may write the cells just read
     }
   }
   const unsigned acc = __reduce_add_sync(0xffffffffu, accepted), skp = __reduce_add_sync(0xffffffffu, skipped);
@@ -142,10 +161,14 @@ static unsigned sweep_blocks(size_t items) {
 
 cudaError_t generic_launch(const DevParams& dp, int n_flights, int n_frames, const float* x, const float* y, const float* yaw,
                            const float* ranges, const uint8_t* kind, int8_t* grids, int accumulate, int row0, int rows,
-                           unsigned long long* stats, cudaStream_t st) {
+                           unsigned long long* stats, cudaStream_t st, const ProbeArgs* Q) {
   if (!accumulate) k_zero_rows<<<sweep_blocks((size_t)dp.W * rows * n_flights), 256, 0, st>>>(grids, n_flights, dp.W, dp.H, row0, rows);
-  k_replay_generic<<<(unsigned)((n_flights + 3) / 4), 128, 0, st>>>(dp, n_flights, n_frames, x, y, yaw, ranges, kind, grids, row0,
-                                                                   rows, stats);
+  if (Q)
+    k_replay_generic<true><<<(unsigned)((n_flights + 3) / 4), 128, 0, st>>>(dp, n_flights, n_frames, x, y, yaw, ranges, kind, grids,
+                                                                           row0, rows, stats, *Q);
+  else
+    k_replay_generic<false><<<(unsigned)((n_flights + 3) / 4), 128, 0, st>>>(dp, n_flights, n_frames, x, y, yaw, ranges, kind, grids,
+                                                                            row0, rows, stats, ProbeArgs{});
   return cudaGetLastError();
 }
 

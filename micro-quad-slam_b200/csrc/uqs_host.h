@@ -25,6 +25,7 @@ struct DevBuf {
 // stream override, used by the host-buffer pipeline to keep two chunks' kernels in flight)
 struct Work {
   DevBuf rays, frames, groups, counters, inc, scan, order, maps, boxes;
+  DevBuf probe_slots, probe_keys, probe_sorted, probe_start, probe_tmp;   // frontier probes and buckets (uqs_frontier.cu)
   int order_nsx = 0, order_nsy = 0;             // geometry the cached tile order was built for
   cudaStream_t stream = nullptr;
   int* h_dims = nullptr;                        // mapped host words the box kernel publishes its maxima to
@@ -33,7 +34,8 @@ struct Work {
   void release() {
     if (h_dims) cudaFreeHost(h_dims);
     h_dims = nullptr;
-    DevBuf* all[] = { &rays, &frames, &groups, &counters, &inc, &scan, &order, &maps, &boxes };
+    DevBuf* all[] = { &rays, &frames, &groups, &counters, &inc, &scan, &order, &maps, &boxes, &probe_slots, &probe_keys, &probe_sorted,
+                      &probe_start, &probe_tmp };
     order_nsx = order_nsy = 0;
     for (DevBuf* b : all) b->release();
   }
@@ -99,15 +101,34 @@ void set_error(const char* fmt, ...);
 int cuda_fail(cudaError_t e, const char* what);
 int check_ready();
 int make_dev_params(const uqs_params* p, DevParams* d);
+// Frontier queries answered inside a replay (uqs_frontier.cu).  Query q owns the probe slots (q*3 + r)*s_max + k: ray
+// r's k-th sample, cells[slot] = its cell or -1 (past the grid's edge).  values[slot] receives the cell's value at the
+// query's frame.
+struct ProbeSet {
+  int n_queries = 0, s_max = 0;
+  const uqs_query* queries = nullptr;
+  const int* cells = nullptr;
+  uint32_t* values = nullptr;
+  size_t slots() const { return (size_t)n_queries * 3 * s_max; }
+};
+// Sort the probes of flights [f0, f0 + nf) into buckets (launch-local flight ids): per flight when slices == 0,
+// per (flight, time slice, sub-tile) otherwise.  Asynchronous on the current stream.
+int probe_buckets(const ProbeSet& Q, int f0, int nf, int n_frames, int W, int slices, int groups_per_slice, int sw,
+                  int sh, int nsx, int nsy, ProbeArgs* out);
+// value = map word of slice s >= 1 applied after slice 0's value and the maps of slices 1..s-1 (before k_compose_slices)
+int probe_resolve_slices(const ProbeArgs& A, int n_probes_max, const int8_t* grids, const uint32_t* maps, int W, int H,
+                         int slices, int groups_per_slice);
+
+// probes == nullptr: the plain replay.  With probes the engine and geometry are chosen exactly as without them.
 int replay_device(const DevParams& dp, int n_flights, int n_frames, const float* x, const float* y,
                   const float* yaw, const float* ranges, const uint8_t* kind, int8_t* grids,
-                  int accumulate, int row0, int rows, bool reset_stats);
+                  int accumulate, int row0, int rows, bool reset_stats, const ProbeSet* probes = nullptr);
 int fetch_stats(uqs_stats* stats, uint64_t frames);
 int ensure_inv_table();
 // uqs_generic.cu: the unrestricted replay and the start-grid range check
 cudaError_t generic_launch(const DevParams& dp, int n_flights, int n_frames, const float* x, const float* y, const float* yaw,
                            const float* ranges, const uint8_t* kind, int8_t* grids, int accumulate, int row0, int rows,
-                           unsigned long long* stats, cudaStream_t st);
+                           unsigned long long* stats, cudaStream_t st, const ProbeArgs* Q = nullptr);
 cudaError_t range_check_launch(const int8_t* grids, int n_flights, int W, int H, int row0, int rows, int lo_min, int lo_max,
                                unsigned long long* bad, cudaStream_t st);
 int fetch_stats_mask(uqs_stats* stats, uint64_t frames, unsigned mask);

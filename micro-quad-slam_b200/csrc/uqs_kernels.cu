@@ -672,8 +672,12 @@ __device__ __forceinline__ void apply_queued(const TileConsts& A, const TileRegi
 
 extern __shared__ __align__(16) unsigned char uqs_smem[];
 
+// PROBE: also serves the job's frontier probes (bucket (flight, slice, sub-tile), frame order).  A probe of frame p is
+// read when every ray of frames <= p that reaches the sub-tile has been applied: before the rays of the first hit frame
+// g > p are queued (after a flush of the queue, which may still hold rays of frames < g), or when the job ends.
+template <bool PROBE>
 __global__ void __launch_bounds__(kReplayThreads)
-k_replay_tiles(ReplayArgs A) {
+k_replay_tiles(ReplayArgs A, ProbeArgs Q) {
   const int lane = threadIdx.x & 31;
   const int wic = threadIdx.x >> 5;
   int8_t* tile = reinterpret_cast<int8_t*>(uqs_smem) + (size_t)wic * A.tile_bytes;
@@ -754,6 +758,40 @@ k_replay_tiles(ReplayArgs A) {
       qhead = (qhead + count) & (kQueueEntries - 1);
       qn -= count;
     };
+    int pb = 0, pe = 0, next_pf = 0x7fffffff;          // this job's probes [pb, pe), frame of the next one
+    if (PROBE) {
+      const int b = (flight * S + slice) * subs_per_grid + sub;
+      pb = Q.start[b];
+      pe = Q.start[b + 1];
+      if (pb < pe) next_pf = Q.probes[pb].x;
+    }
+    // read every probe of a frame < fmax (lanes take consecutive probes; the ones taken are a prefix: frame order)
+    auto serve = [&](int fmax) {
+      if (next_pf >= fmax) return;
+      while (qn > 0) flush();
+      __syncwarp();
+      while (next_pf < fmax) {
+        const int i = pb + lane;
+        const int4 pr = i < pe ? Q.probes[i] : make_int4(0x7fffffff, 0, 0, 0);
+        const bool take = pr.x < fmax;
+        if (take) {
+          const int gy = pr.y / A.W, gx = pr.y - gy * A.W;
+          uint32_t v;
+          if (map) {
+            const uint32_t cell = tile_s + ((uint32_t)((gy - Y0) * A.pitch_cells + (gx - X0)) << 2);
+            UQS_CHECK(cell, 4u, DR.tile);
+            v = lds_u32(cell);
+          } else {
+            const uint32_t cell = tile_s + (uint32_t)((gy - Y0) * A.pitch + (gx - X0));
+            UQS_CHECK(cell, 1u, DR.tile);
+            v = (uint32_t)lds_s8(cell);
+          }
+          Q.values[pr.z] = v;
+        }
+        pb += __popc(__ballot_sync(0xffffffffu, take));
+        next_pf = pb < pe ? Q.probes[pb].x : 0x7fffffff;
+      }
+    };
     for (int g0 = g_begin; g0 < g_end; g0 += 32) {
       bool ghit = false;
       if (g0 + lane < g_end) {
@@ -776,6 +814,7 @@ k_replay_tiles(ReplayArgs A) {
           fmask &= fmask - 1;
           const uint2 rec = rec_next;
           if (fmask) rec_next = __ldg(&rays[(size_t)(f0 + __ffs(fmask) - 1) * 32 + lane]);
+          if (PROBE) serve(f0 + fi);
           const int gx0 = (int)(__shfl_sync(0xffffffffu, fr.x, fi) & 0xffffu);
           const int gy0 = (int)(__shfl_sync(0xffffffffu, fr.y, fi) & 0xffffu);
           const int ex = gx0 + sext12(rec.x), ey = gy0 + sext12(rec.x >> 12);
@@ -797,6 +836,7 @@ k_replay_tiles(ReplayArgs A) {
     }
     while (qn > 0) flush();
     __syncwarp();
+    if (PROBE) serve(0x7fffffff);                       // frames no ray of which reached the sub-tile
 
     // ---- write the sub-tile back: values into the grid, maps into the slice scratch ---------
     if (map) {
@@ -904,9 +944,13 @@ __device__ __forceinline__ Beam decode_beam(uint2 rec, uint2 org, int P, int bx0
 // touched by exactly one lane, whichever layout enumerates them.
 // PROD = 1: warp specialisation -- an extra (NW+1)-th warp does nothing but decode frames into the ring, two frames
 // ahead of the NW consumer warps, and joins the per-frame barrier; the consumers never decode or load raw records.
-template <int NW, int FAN, int PROD>
+// PROBE: also serves the flight's frontier probes (bucket = flight, frame order).  The barrier that ends frame f orders
+// it before frame f + 1, so the probes of frame f are read right after it, followed by one more barrier (only when f
+// has probes: the condition is the same in every thread).  Cells outside the resident box are read from the grid in
+// HBM, which the kernel only writes at the end: they still hold their start value.
+template <int NW, int FAN, int PROD, bool PROBE = false>
 __global__ void __launch_bounds__((NW + PROD) * 32, (NW <= 4) ? (PROD ? 6 : UQS_MINB) : ((NW <= 8) ? 4 : ((NW <= 16) ? 2 : 1)))
-k_replay_flights(FlightArgs A) {
+k_replay_flights(FlightArgs A, ProbeArgs Q) {
   constexpr int NT = (NW + PROD) * 32;          // threads per CTA
   const bool producer = PROD && (threadIdx.x >> 5) == NW;
   int8_t* grid_s = reinterpret_cast<int8_t*>(uqs_smem);
@@ -938,7 +982,19 @@ k_replay_flights(FlightArgs A) {
     // everything outside keeps its value in HBM (zero unless accumulating)
     const int4 box = A.boxes[flight];
     const int bx0 = box.x, by0 = box.y, bw = box.z - box.x, bh = box.w - box.y;
-    if (bw <= 0 || bh <= 0) { __syncthreads(); continue; }
+    const int8_t* grid_hbm = A.grids + (size_t)flight * A.W * A.H;
+    int pb = 0, pe = 0, next_pf = 0x7fffffff;          // this flight's probes [pb, pe), frame of the next one
+    if (PROBE) {
+      pb = Q.start[flight];
+      pe = Q.start[flight + 1];
+      if (pb < pe) next_pf = Q.probes[pb].x;
+    }
+    if (bw <= 0 || bh <= 0) {                           // no accepted ray: every probe reads the start grid
+      if (PROBE)
+        for (int i = pb + threadIdx.x; i < pe; i += NT) { const int4 pr = Q.probes[i]; Q.values[pr.z] = (uint32_t)(int)grid_hbm[pr.y]; }
+      __syncthreads();
+      continue;
+    }
     int8_t* grid_g = A.grids + (size_t)flight * A.W * A.H + (size_t)by0 * A.W + bx0;
     const bool vec = (((A.W | bx0 | bw) & 3) == 0) && ((reinterpret_cast<size_t>(grid_g) & 3) == 0);
 
@@ -1226,6 +1282,27 @@ k_replay_flights(FlightArgs A) {
         raw_org = __ldg(reinterpret_cast<const uint2*>(&frames[gn]));
       }
       __syncthreads();
+      if (PROBE) {
+        while (next_pf == f) {                      // the taken probes are a prefix of [pb, pe) (frame order)
+          const int i = pb + (int)threadIdx.x;
+          const int4 pr = i < pe ? Q.probes[i] : make_int4(-1, 0, 0, 0);
+          const bool take = pr.x == f;
+          if (take) {
+            const int gy = pr.y / A.W, gx = pr.y - gy * A.W;
+            int v;
+            if (gx >= bx0 && gx < bx0 + bw && gy >= by0 && gy < by0 + bh) {
+              const uint32_t cell = grid_sa + (uint32_t)((gy - by0) * P + (gx - bx0));
+              UQS_CHECK(cell, 1u, RG);
+              v = lds_s8(cell);
+            } else {
+              v = (int)grid_hbm[pr.y];
+            }
+            Q.values[pr.z] = (uint32_t)v;
+          }
+          pb += __syncthreads_count(take);           // also keeps frame f + 1 from writing before every read is done
+          next_pf = pb < pe ? Q.probes[pb].x : 0x7fffffff;
+        }
+      }
     }
 
     if (vec) {
@@ -1272,7 +1349,7 @@ __global__ void k_flight_boxes(int n_flights, int groups_per_flight, const uint2
   }
 }
 
-static void (*flight_kernel(int nw, int fan, int prod))(FlightArgs) {
+static void (*flight_kernel(int nw, int fan, int prod))(FlightArgs, ProbeArgs) {
   if (prod) return nw == 4 ? k_replay_flights<4, 0, 1> : (nw == 8 ? k_replay_flights<8, 0, 1> : (nw == 32 ? k_replay_flights<16, 0, 1> : k_replay_flights<16, 0, 1>));
   if (fan) return nw == 4 ? k_replay_flights<4, 1, 0> : (nw == 8 ? k_replay_flights<8, 1, 0> : (nw == 32 ? k_replay_flights<32, 1, 0> : k_replay_flights<16, 1, 0>));
   return nw == 4 ? k_replay_flights<4, 0, 0> : (nw == 8 ? k_replay_flights<8, 0, 0> : (nw == 32 ? k_replay_flights<32, 0, 0> : k_replay_flights<16, 0, 0>));
@@ -1303,7 +1380,36 @@ cudaError_t flights_prepare(int nw, int fan, int prod, size_t smem, int* ctas_pe
 }
 
 cudaError_t flights_launch(int nw, int fan, int prod, unsigned grid, size_t smem, cudaStream_t st, const FlightArgs& A) {
-  flight_kernel(nw, fan, prod)<<<grid, flight_threads(nw, prod), smem, st>>>(A);
+  flight_kernel(nw, fan, prod)<<<grid, flight_threads(nw, prod), smem, st>>>(A, ProbeArgs{});
+  return cudaGetLastError();
+}
+
+// the probe variant exists for the default layout only (the fan layout and the decode warp were measured and rejected)
+static void (*flight_probe_kernel(int nw))(FlightArgs, ProbeArgs) {
+  return nw == 4 ? k_replay_flights<4, 0, 0, true> : (nw == 8 ? k_replay_flights<8, 0, 0, true> : (nw == 32 ? k_replay_flights<32, 0, 0, true> : k_replay_flights<16, 0, 0, true>));
+}
+
+cudaError_t flights_probe_prepare(int nw, size_t smem, int* ctas_per_sm) {
+  cudaError_t e = cudaFuncSetAttribute(flight_probe_kernel(nw), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, flight_probe_kernel(nw), flight_threads(nw, 0), smem);
+}
+
+cudaError_t flights_probe_launch(int nw, unsigned grid, size_t smem, cudaStream_t st, const FlightArgs& A, const ProbeArgs& Q) {
+  flight_probe_kernel(nw)<<<grid, flight_threads(nw, 0), smem, st>>>(A, Q);
+  return cudaGetLastError();
+}
+
+cudaError_t tiles_prepare(bool probe, size_t smem, int* ctas_per_sm) {
+  void (*k)(ReplayArgs, ProbeArgs) = probe ? k_replay_tiles<true> : k_replay_tiles<false>;
+  cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, k, kReplayThreads, smem);
+}
+
+cudaError_t tiles_launch(bool probe, unsigned grid, size_t smem, cudaStream_t st, const ReplayArgs& A, const ProbeArgs& Q) {
+  if (probe) k_replay_tiles<true><<<grid, kReplayThreads, smem, st>>>(A, Q);
+  else       k_replay_tiles<false><<<grid, kReplayThreads, smem, st>>>(A, Q);
   return cudaGetLastError();
 }
 

@@ -47,6 +47,16 @@ struct FlightArgs {
   int accumulate;
 };
 
+// Frontier probes served inside a replay (uqs_frontier.cu): one cell a query's score reads, at the moment its owner
+// has applied exactly the frames <= `frame`.  Sorted by (bucket, frame); bucket b holds [start[b], start[b+1]):
+// per flight for the resident and unrestricted engines, per (flight, time slice, sub-tile) for the sub-tile engine.
+struct ProbeArgs {
+  const int4* probes;       // {frame, cell = gy*W + gx, slot, flight (launch-local)}
+  const int* start;         // [n_buckets + 1]
+  uint32_t* values;         // [slot]: the cell's value, or its 32-bit map word in a time-slice map tile
+  int n_buckets;
+};
+
 struct ScanState;
 
 __global__ void k_pose_increments(long long total, int n_samples, const uint32_t* t_ms,
@@ -72,9 +82,13 @@ __global__ void k_records_to_cells(long long n_frames, const uint4* frames, cons
                                    int32_t* cells, int32_t* origin);
 __global__ void k_sincosf(size_t n, const float* a, float* s, float* c);
 __global__ void k_world_to_grid_one(DevParams p, float wx, float wy, int* out);
-__global__ void k_replay_tiles(ReplayArgs A);
+// the sub-tile engine (k_replay_tiles), plain or serving probes
+cudaError_t tiles_prepare(bool probe, size_t smem, int* ctas_per_sm);
+cudaError_t tiles_launch(bool probe, unsigned grid, size_t smem, cudaStream_t st, const ReplayArgs& A, const ProbeArgs& Q);
 __global__ void k_compose_slices(int8_t* grids, const uint32_t* maps, int n_flights, int W, int H, int S, int row0,
                                  int rows);
+cudaError_t flights_probe_prepare(int nw, size_t smem, int* ctas_per_sm);
+cudaError_t flights_probe_launch(int nw, unsigned grid, size_t smem, cudaStream_t st, const FlightArgs& A, const ProbeArgs& Q);
 cudaError_t flight_boxes_launch(int n_flights, int groups_per_flight, const uint2* groups, int W, int H, int4* boxes,
                                 int* dims, int* host_dims_dev, cudaStream_t st);
 cudaError_t flights_prepare(int nw, int fan, int prod, size_t smem, int* ctas_per_sm);

@@ -112,26 +112,18 @@ __global__ void k_frontier_scores(DevParams p, const int8_t* __restrict__ grid, 
                                   unsigned long long* __restrict__ domain_errors) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  const float max_range = 2.5f;                                    // :361
-  const float step = __fmul_rn(p.res, 2.0f);                       // :362
-  int unknown = 0, freec = 0, occ = 0;
+  const float step = frontier_step(p);
+  int score = 0;
   for (int r = 0; r < 3; r++) {
-    const float ro = (r == 0) ? 0.0f : (r == 1) ? 15.0f : -15.0f;  // :360
-    const float ang = __fmul_rn(__fadd_rn(__fadd_rn(yaw_deg[i], offset_deg[i]), ro), p.deg2rad);   // :367
     float sa, ca;
-    if (!sincosf_glibc(ang, sa, ca)) { atomicAdd(domain_errors, 1ull); continue; }
-    for (float d = step; d <= max_range; d = __fadd_rn(d, step)) {  // :371
-      const float px = __fadd_rn(x[i], __fmul_rn(d, ca));
-      const float py = __fadd_rn(y[i], __fmul_rn(d, sa));
+    if (!sincosf_glibc(frontier_ray_angle(p, yaw_deg[i], offset_deg[i], r), sa, ca)) { atomicAdd(domain_errors, 1ull); continue; }
+    for (float d = step; d <= kFrontierRange; d = __fadd_rn(d, step)) {   // :371
       int gx, gy;
-      if (!world_to_grid(p, px, py, gx, gy)) break;                // :375
-      const int v = (int)grid[(size_t)gy * p.W + gx];
-      if (v >= -1 && v <= 1) unknown++;                            // :378-380
-      else if (v > 10) occ++;
-      else if (v < -10) freec++;
+      if (!frontier_point(p, x[i], y[i], d, ca, sa, gx, gy)) break;
+      score += frontier_weight((int)grid[(size_t)gy * p.W + gx]);
     }
   }
-  scores[i] = unknown * 3 + freec * 1 - occ * 4;                   // :383
+  scores[i] = score;                                               // unknown*3 + free - occ*4, :383
 }
 
 }  // namespace uqs
