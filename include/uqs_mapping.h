@@ -142,8 +142,8 @@ int  uqs_set_fan_layout(int on);
  * consumer warps (4, 8 or 16 of them).  -1 = the built-in choice.  Identical bytes either way.
  * uqs_replay_frontier[_dev] ignores this knob. */
 int  uqs_set_decode_warp(int on);
-/* Measurement knob: adds `steps` (0..8) to every frame's collision bound K0 (always safe; identical bytes): what one
- * collision-checked step per frame costs the resident engine. */
+/* Measurement knob: adds `steps` (0..8) to every frame's collision bound K0, capped at the frame's longest beam
+ * (always safe; identical bytes): what one collision-checked step per frame costs the resident engine. */
 int  uqs_set_k0_bias(int steps);
 /* Experiment knob for the layouts above: row pitch of the resident box in 32-bit words, modulo 32
  * (-1 = the built-in odd pitch).  Identical bytes for any value. */
@@ -242,8 +242,8 @@ int uqs_beam_cells(const uqs_params* p, int n_frames,
                    const float* x, const float* y, const float* yaw_deg, const float* ranges,
                    int32_t* cells_out, int32_t* origin_out);
 /* Parity hook for the collision bound of the resident engine: per frame, K0 (two beams of the frame can share
- * a cell only at steps k < K0; -1 when the frame's pose is off the grid) and whether the frame's beams were
- * found in circular angular order.  Host pointers. */
+ * a cell only at steps k < K0; -1 when the frame's pose is off the grid) as the resident engine receives it,
+ * uqs_set_k0_bias included, and whether the frame's beams were found in circular angular order.  Host pointers. */
 int uqs_frame_bounds(const uqs_params* p, int n_frames, const float* x, const float* y, const float* yaw_deg,
                      const float* ranges, int32_t* k0_out, int32_t* sorted_out);
 

@@ -843,8 +843,8 @@ int uqs_beam_cells(const uqs_params* p, int n_frames, const float* x, const floa
 }
 
 /* Parity hook for the collision bound: K0 and the angular-order flag of every frame, as k_ray_setup writes
- * them for the resident engine.  tests/ verify by brute force that no two beams of a frame share a cell at any
- * step >= K0 and that flagged frames really are in circular angular order. */
+ * them for the resident engine, K0 including the bias of uqs_set_k0_bias.  tests/ verify by brute force that no two
+ * beams of a frame share a cell at any step >= K0 and that flagged frames really are in circular angular order. */
 int uqs_frame_bounds(const uqs_params* p, int n_frames, const float* x, const float* y, const float* yaw,
                      const float* ranges, int32_t* k0_out, int32_t* sorted_out) {
   int rc = check_ready();
@@ -865,7 +865,7 @@ int uqs_frame_bounds(const uqs_params* p, int n_frames, const float* x, const fl
   cudaError_t e = cudaMemsetAsync(g_ctx.w->counters.p, 0, 64, st);
   if (e != cudaSuccess) return cuda_fail(e, "memset");
   k_ray_setup<<<(unsigned)gpf, 1024, 0, st>>>(dp, n_frames, (float*)g_ctx.in_x.p, (float*)g_ctx.in_y.p,
-                                              (float*)g_ctx.in_yaw.p, (float*)g_ctx.in_ranges.p, nullptr, 1,
+                                              (float*)g_ctx.in_yaw.p, (float*)g_ctx.in_ranges.p, nullptr, 1 + g_ctx.k0_bias,
                                               (const uint32_t*)g_ctx.inv_table.p, (uint4*)g_ctx.w->frames.p, (uint2*)g_ctx.w->groups.p,
                                               (uint2*)g_ctx.w->rays.p, (unsigned long long*)g_ctx.w->counters.p);
   e = cudaGetLastError();

@@ -399,7 +399,7 @@ k_ray_setup(const __grid_constant__ DevParams p, int n_frames, const float* __re
           int kk = 1;                                                   // the start cell is shared by all beams
           // no shared cell once k*gap > 1: steps 0..floor(1/gap) may collide (the float slack only enlarges it)
           if (has_dir && __popc(dir) >= 2) kk = (gap > 1e-4f) ? (int)(1.0f / (gap - 2e-5f)) + 1 : 0x7fffffff;
-          k0 = min(__reduce_max_sync(0xffffffffu, kk) + (want_k0 - 1), mmax + 1);      // want_k0 - 1: measurement bias (K0 may only be too large)
+          k0 = min(__reduce_max_sync(0xffffffffu, kk), mmax + 1);
         } else {
           // beams out of angular order (very short rays quantise coarsely): exact all-pairs bound
 #pragma unroll 4
@@ -417,6 +417,10 @@ k_ray_setup(const __grid_constant__ DevParams p, int n_frames, const float* __re
           k0 = __reduce_max_sync(0xffffffffu, k0);
         }
       }
+      // want_k0 - 1: measurement bias (uqs_set_k0_bias), added after the cap at mmax + 1 so that it cannot overflow the
+      // 0x7fffffff of parallel beams, and capped the same way (a larger K0 is always safe: more collision-checked steps)
+      const int bias = want_k0 - 1;
+      k0 = min(k0, mmax + 1 - bias) + bias;
     }
 
     xmin = __reduce_min_sync(0xffffffffu, xmin);
