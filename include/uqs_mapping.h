@@ -263,10 +263,30 @@ int uqs_beams_from_scans_dev(long long n_frames, const uint8_t* raw_dev, float m
 
 /* N2: replay ONE log exactly as log_tick() does with recentering enabled (uav_local_nav.c:1629-1635:
  * map_recentre_if_needed(pose) before every update).  origin_out = final map origin; events_out receives
- * up to max_events {frame, sx_cells, sy_cells} triples. */
+ * up to max_events {frame, sx_cells, sy_cells} triples, *n_events_out the number of events (any count).
+ * Host buffers; uqs_replay_recentering_dev with one flight. */
 int uqs_replay_recentering(const uqs_params* p, int n_frames, const float* x, const float* y, const float* yaw_deg,
                            const float* ranges, int8_t* grid_out, float origin_out[2], int* n_events_out,
                            int* events_out, int max_events, uqs_stats* stats);
+
+/* N2 for many flights: every flight replayed exactly as log_tick() does with recentering enabled
+ * (map_recentre_if_needed(x[f], y[f]) before frame f's update), each from an all-zero grid at origin (p->origin_x,
+ * p->origin_y).  grids_dev: [n_flights][H][W], each flight's final map in its final window.
+ * origins_dev: [n_flights][2] final origins.  n_events_dev: [n_flights] events per flight.
+ * events_dev (may be NULL): [n_flights][max_events][3] {frame, sx, sy}, the first max_events of each flight (entries
+ * past a flight's count are not written).  Stats as for uqs_replay_dev.  Asynchronous unless stats is given (the
+ * recenter plan itself synchronises once, to size its event list).
+ * NULL buffers, non-positive sizes, max_events < 0, or max_events > 0 with events_dev == NULL return UQS_ERR_BAD_ARG
+ * before anything is written; so does engine 2 (uqs_set_engine): the resident engine has no recentering variant.
+ * Engines 0 and 1 replay the flights in one pass of the sub-tile engine when the inputs suit it (rays of at most 1024
+ * cells, 0 inside [lo_min, lo_max], no time slices for this call -- or uqs_set_tuning(.., .., 1) -- and the cells the
+ * flights reach across their windows within 32767 x 32767); otherwise, and with engine 3, each flight's log is replayed
+ * segment by segment between its events.  uqs_set_fan_layout(), uqs_set_decode_warp() and uqs_set_k0_bias() do not
+ * apply to this call. */
+int uqs_replay_recentering_dev(const uqs_params* p, int n_flights, int n_frames,
+                               const float* x_dev, const float* y_dev, const float* yaw_dev, const float* ranges_dev,
+                               int8_t* grids_dev, float* origins_dev, int32_t* n_events_dev,
+                               int32_t* events_dev, int max_events, uqs_stats* stats);
 
 /* N3: frontier_score_dir() (uav_local_nav.c:356-385) for n queries against one host grid. */
 int uqs_frontier_scores(const uqs_params* p, const int8_t* grid, int n, const float* x, const float* y,

@@ -85,7 +85,7 @@ _EXPORTS = [
     "uqs_pose_integrate", "uqs_pose_integrate_dev", "uqs_replay", "uqs_replay_dev", "uqs_replay_flow",
     "uqs_beam_cells", "uqs_frame_bounds", "uqs_sincosf_batch", "uqs_measure_rmw_peak", "uqs_measure_atoms_peak",
     "uqs_beams_from_scans", "uqs_beams_from_scans_dev", "uqs_replay_recentering", "uqs_frontier_scores",
-    "uqs_replay_frontier", "uqs_replay_frontier_dev",
+    "uqs_replay_frontier", "uqs_replay_frontier_dev", "uqs_replay_recentering_dev",
     "uqs_scanlog_read", "uqs_scanlog_count", "uqs_navlog_read", "map_recenter_shift", "map_recentre_if_needed", "frontier_score_dir",
     # multi-GPU
     "uqs_flight_shard", "uqs_row_band", "uqs_comm_unique_id", "uqs_comm_init_rank", "uqs_comm_destroy", "uqs_comm_nranks",
@@ -138,6 +138,7 @@ def lib() -> C.CDLL:
     L.uqs_measure_atoms_peak.argtypes = [C.POINTER(C.c_double)]
     L.uqs_beams_from_scans.argtypes = [C.c_longlong, vp, C.c_float, vp, vp]
     L.uqs_replay_recentering.argtypes = [C.POINTER(Params), ip, vp, vp, vp, vp, vp, vp, C.POINTER(C.c_int), vp, ip, C.POINTER(Stats)]
+    L.uqs_replay_recentering_dev.argtypes = [C.POINTER(Params), ip, ip] + [vp] * 8 + [ip, C.POINTER(Stats)]
     L.uqs_frontier_scores.argtypes = [C.POINTER(Params), vp, ip, vp, vp, vp, vp, vp]
     L.uqs_replay_frontier.argtypes = [C.POINTER(Params), ip, ip, vp, vp, vp, vp, vp, ip, vp, vp, C.POINTER(Stats)]
     L.uqs_replay_frontier_dev.argtypes = [C.POINTER(Params), ip, ip, vp, vp, vp, vp, vp, ip, ip, vp, vp, C.POINTER(Stats)]
@@ -449,6 +450,43 @@ def replay_recentering(p: Params, x, y, yaw_deg, ranges):
     _check(lib().uqs_replay_recentering(C.byref(p), n, _ptr(x), _ptr(y), _ptr(yaw_deg), _ptr(ranges), _ptr(grid), _ptr(origin),
                                         C.byref(n_ev), _ptr(ev), 256, C.byref(st)))
     return grid, (float(origin[0]), float(origin[1])), ev[:min(n_ev.value, 256)].copy(), st.as_dict()
+
+
+def replay_recentering_dev(p: Params, n_flights: int, n_frames: int, x_ptr: int, y_ptr: int, yaw_ptr: int, ranges_ptr: int,
+                           grids_ptr: int, origins_ptr: int, n_events_ptr: int, events_ptr: int = 0, max_events: int = 0,
+                           want_stats: bool = False):
+    """``uqs_replay_recentering_dev`` on raw device pointers (e.g. ``tensor.data_ptr()``): grids int8 [F,H,W], origins
+    float32 [F,2], n_events int32 [F], events int32 [F,max_events,3] (0 = none); asynchronous unless stats are asked."""
+    st = Stats()
+    _check(lib().uqs_replay_recentering_dev(C.byref(p), n_flights, n_frames, C.c_void_p(x_ptr), C.c_void_p(y_ptr),
+                                            C.c_void_p(yaw_ptr), C.c_void_p(ranges_ptr), C.c_void_p(grids_ptr),
+                                            C.c_void_p(origins_ptr), C.c_void_p(n_events_ptr),
+                                            C.c_void_p(events_ptr) if events_ptr else None, int(max_events),
+                                            C.byref(st) if want_stats else None))
+    return st.as_dict() if want_stats else None
+
+
+def replay_recentering_flights(p: Params, x, y, yaw_deg, ranges, max_events: int = 64):
+    """N2 for many flights from host arrays (x, y, yaw [F,N], ranges [F,N,32]), staged through torch on the current
+    device -> (grids [F,H,W] int8, origins [F,2] float32, n_events [F] int32, events [F,max_events,3] int32, stats).
+    events[f, k] is meaningful for k < min(n_events[f], max_events)."""
+    import torch
+    x = _f32(x)
+    if x.ndim == 1:
+        x = x[None]
+    F, N = x.shape
+    dev = torch.device("cuda", torch.cuda.current_device())
+    t = [torch.from_numpy(a).to(dev) for a in (x, _f32(y).reshape(F, N), _f32(yaw_deg).reshape(F, N),
+                                               _f32(ranges).reshape(F, N, BEAMS_PER_FRAME))]
+    grids = torch.empty((F, p.H, p.W), dtype=torch.int8, device=dev)
+    origins = torch.empty((F, 2), dtype=torch.float32, device=dev)
+    n_ev = torch.empty(F, dtype=torch.int32, device=dev)
+    events = torch.zeros((F, max(max_events, 0), 3), dtype=torch.int32, device=dev)
+    torch.cuda.synchronize()
+    st = replay_recentering_dev(p, F, N, *(a.data_ptr() for a in t), grids.data_ptr(), origins.data_ptr(), n_ev.data_ptr(),
+                                events.data_ptr() if max_events > 0 else 0, max_events, want_stats=True)
+    torch.cuda.synchronize()
+    return grids.cpu().numpy(), origins.cpu().numpy(), n_ev.cpu().numpy(), events.cpu().numpy(), st
 
 
 def frontier_scores(p: Params, grid, x, y, yaw_deg, offset_deg):

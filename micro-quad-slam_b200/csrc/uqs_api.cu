@@ -149,50 +149,11 @@ static cudaError_t zero_counted(void* p, size_t bytes, cudaStream_t st) {
   return zero_async(p, bytes, st);
 }
 
-int replay_device(const DevParams& dp, int n_flights, int n_frames, const float* x, const float* y,
-                  const float* yaw, const float* ranges, const uint8_t* kind, int8_t* grids,
-                  int accumulate, int row0, int rows, bool reset_stats, const ProbeSet* probes) {
-  cudaStream_t st = g_ctx.stream();
+// Sub-tile engine geometry and time slices of a replay of n_flights x n_frames over `rows` rows (replay_device; the
+// recentering call asks it whether a call would be time-sliced)
+void tile_geometry(const DevParams& dp, int n_flights, int n_frames, int rows, int* psw, int* psh, int* pnsx, int* pnsy,
+                   int* pslices) {
   const int gpf = (n_frames + 31) / 32;
-  g_ctx.w->boxes_valid = false;                  // set again below once this call's touched boxes exist
-  {
-    const int rc0 = ensure_inv_table();
-    if (rc0) return rc0;
-  }
-  // Inputs outside what the fast engines assume go to the unrestricted kernel (uqs_generic.cu): rays that can be
-  // longer than kMaxRayCells cells, a clamp range that excludes 0, or -- when accumulating -- a start grid with
-  // values outside [lo_min, lo_max] (checked on the device; the reference clamps such a cell on its next update).
-  {
-    const int side = std::max(dp.W, dp.H);
-    const bool long_rays = side > kMaxRayCells + 1 && (kind != nullptr || !(dp.max_range / dp.res + 3.0f <= (float)kMaxRayCells));
-    bool generic = g_ctx.engine == 3 || long_rays || dp.lo_min > 0 || dp.lo_max < 0;
-    int rcg;
-    if ((rcg = g_ctx.w->counters.ensure(64 * sizeof(unsigned long long)))) return rcg;
-    unsigned long long* cnt = (unsigned long long*)g_ctx.w->counters.p;
-    cudaError_t eg = cudaSuccess;
-    if (!generic && accumulate) {
-      unsigned long long bad = 0;
-      eg = zero_counted(cnt + 40, sizeof(unsigned long long), st);
-      if (eg == cudaSuccess) eg = range_check_launch(grids, n_flights, dp.W, dp.H, row0, rows, dp.lo_min, dp.lo_max, cnt + 40, st);
-      if (eg == cudaSuccess) eg = cudaMemcpyAsync(&bad, cnt + 40, sizeof(bad), cudaMemcpyDeviceToHost, st);
-      if (eg == cudaSuccess) eg = cudaStreamSynchronize(st);
-      if (eg != cudaSuccess) return cuda_fail(eg, "start-grid range check");
-      g_ctx.launches += 1;
-      generic = bad != 0;
-    }
-    if (generic) {
-      if (reset_stats) eg = zero_counted(cnt, 8 * sizeof(unsigned long long), st);
-      if (eg != cudaSuccess) return cuda_fail(eg, "memset stats");
-      ProbeArgs PA;
-      if (probes && (rcg = probe_buckets(*probes, 0, n_flights, n_frames, dp.W, 0, 0, 0, 0, 0, 0, &PA))) return rcg;
-      KernelTimer t_rep(2);
-      eg = generic_launch(dp, n_flights, n_frames, x, y, yaw, ranges, kind, grids, accumulate, row0, rows, cnt, st, probes ? &PA : nullptr);
-      t_rep.stop();
-      if (eg != cudaSuccess) return cuda_fail(eg, "k_replay_generic launch");
-      g_ctx.launches += accumulate ? 1 : 2;
-      return UQS_OK;
-    }
-  }
   // Sub-tile engine geometry.  With plenty of (flight, tile) jobs, ~80-cell tiles and no time slicing.
   // With few (one long log, one small flight) the chip would idle: cut the log into S time slices,
   // replayed concurrently as clamp-add maps on 40-cell tiles and composed afterwards (exact).
@@ -239,11 +200,61 @@ int replay_device(const DevParams& dp, int n_flights, int n_frames, const float*
       choose_tiles(dp.W, rows, slice_tile, &sw, &sh, &nsx, &nsy);
     }
   }
-  int pitch = (sw + 3) & ~3;
-  if (((pitch >> 2) & 1) == 0) pitch += 4;            // odd word pitch: column walks hit 32 banks
   const int pitch_cells = sw | 1;
   if (slices > 1 && g_ctx.tune_slices == 0 && ((size_t)pitch_cells * sh * 4 + kReplayQueueBytes) * kReplayWarps > 227u * 1024u)
     slices = 1;                                        // a forced large sub-tile leaves no room for 32-bit map cells
+  *psw = sw; *psh = sh; *pnsx = nsx; *pnsy = nsy; *pslices = slices;
+}
+
+int replay_device(const DevParams& dp, int n_flights, int n_frames, const float* x, const float* y,
+                  const float* yaw, const float* ranges, const uint8_t* kind, int8_t* grids,
+                  int accumulate, int row0, int rows, bool reset_stats, const ProbeSet* probes) {
+  cudaStream_t st = g_ctx.stream();
+  const int gpf = (n_frames + 31) / 32;
+  g_ctx.w->boxes_valid = false;                  // set again below once this call's touched boxes exist
+  {
+    const int rc0 = ensure_inv_table();
+    if (rc0) return rc0;
+  }
+  // Inputs outside what the fast engines assume go to the unrestricted kernel (uqs_generic.cu): rays that can be
+  // longer than kMaxRayCells cells, a clamp range that excludes 0, or -- when accumulating -- a start grid with
+  // values outside [lo_min, lo_max] (checked on the device; the reference clamps such a cell on its next update).
+  {
+    const int side = std::max(dp.W, dp.H);
+    const bool long_rays = side > kMaxRayCells + 1 && (kind != nullptr || !(dp.max_range / dp.res + 3.0f <= (float)kMaxRayCells));
+    bool generic = g_ctx.engine == 3 || long_rays || dp.lo_min > 0 || dp.lo_max < 0;
+    int rcg;
+    if ((rcg = g_ctx.w->counters.ensure(64 * sizeof(unsigned long long)))) return rcg;
+    unsigned long long* cnt = (unsigned long long*)g_ctx.w->counters.p;
+    cudaError_t eg = cudaSuccess;
+    if (!generic && accumulate) {
+      unsigned long long bad = 0;
+      eg = zero_counted(cnt + 40, sizeof(unsigned long long), st);
+      if (eg == cudaSuccess) eg = range_check_launch(grids, n_flights, dp.W, dp.H, row0, rows, dp.lo_min, dp.lo_max, cnt + 40, st);
+      if (eg == cudaSuccess) eg = cudaMemcpyAsync(&bad, cnt + 40, sizeof(bad), cudaMemcpyDeviceToHost, st);
+      if (eg == cudaSuccess) eg = cudaStreamSynchronize(st);
+      if (eg != cudaSuccess) return cuda_fail(eg, "start-grid range check");
+      g_ctx.launches += 1;
+      generic = bad != 0;
+    }
+    if (generic) {
+      if (reset_stats) eg = zero_counted(cnt, 8 * sizeof(unsigned long long), st);
+      if (eg != cudaSuccess) return cuda_fail(eg, "memset stats");
+      ProbeArgs PA;
+      if (probes && (rcg = probe_buckets(*probes, 0, n_flights, n_frames, dp.W, 0, 0, 0, 0, 0, 0, &PA))) return rcg;
+      KernelTimer t_rep(2);
+      eg = generic_launch(dp, n_flights, n_frames, x, y, yaw, ranges, kind, grids, accumulate, row0, rows, cnt, st, probes ? &PA : nullptr);
+      t_rep.stop();
+      if (eg != cudaSuccess) return cuda_fail(eg, "k_replay_generic launch");
+      g_ctx.launches += accumulate ? 1 : 2;
+      return UQS_OK;
+    }
+  }
+  int sw, sh, nsx, nsy, slices;
+  tile_geometry(dp, n_flights, n_frames, rows, &sw, &sh, &nsx, &nsy, &slices);
+  int pitch = (sw + 3) & ~3;
+  if (((pitch >> 2) & 1) == 0) pitch += 4;            // odd word pitch: column walks hit 32 banks
+  const int pitch_cells = sw | 1;
   const int gps = (gpf + slices - 1) / slices;          // 32-frame groups per slice
   const int tile_bytes = slices > 1 ? std::max(pitch * sh, pitch_cells * sh * 4) : pitch * sh;
   size_t smem = (size_t)tile_bytes * kReplayWarps + (size_t)kReplayQueueBytes * kReplayWarps;   // tiles + candidate queues
@@ -292,12 +303,11 @@ int replay_device(const DevParams& dp, int n_flights, int n_frames, const float*
     const int nf = std::min(chunk, n_flights - f0);
     const size_t fo = (size_t)f0 * n_frames;
     KernelTimer t_setup(1);
-    k_ray_setup<<<dim3((unsigned)gpf, (unsigned)nf), 1024, 0, st>>>(
-        dp, n_frames, x + fo, y + fo, yaw + fo,
+    e = ray_setup_launch(
+        dim3((unsigned)gpf, (unsigned)nf), st, dp, n_frames, x + fo, y + fo, yaw + fo,
         dp.ranges_u16 ? reinterpret_cast<const float*>(reinterpret_cast<const uint16_t*>(ranges) + fo * 32) : ranges + fo * 32,
         kind ? kind + fo : nullptr, may_reside ? 1 + g_ctx.k0_bias : 0,
         (const uint32_t*)g_ctx.inv_table.p, (uint4*)g_ctx.w->frames.p, (uint2*)g_ctx.w->groups.p, (uint2*)g_ctx.w->rays.p, counters);
-    e = cudaGetLastError();
     t_setup.stop();
     if (e != cudaSuccess) return cuda_fail(e, "k_ray_setup launch");
 
@@ -461,6 +471,84 @@ int replay_device(const DevParams& dp, int n_flights, int n_frames, const float*
       e = cudaGetLastError();
       g_ctx.launches += 1;
     }
+    t_rep.stop();
+    if (e != cudaSuccess) return cuda_fail(e, "k_replay_tiles launch");
+    g_ctx.launches += 2;
+  }
+  return UQS_OK;
+}
+
+// Recentred flights through the sub-tile engine (uqs_replay_recentering_dev, route A): the ray set-up places every
+// frame's records in its flight's global frame, and the sub-tiles cover the largest global extent gw x gh of the call.
+// Grids start at zero; stats are reset.  The caller has checked that the inputs suit the sub-tile engine.
+int replay_device_recentering(const DevParams& dp, int n_flights, int n_frames, const float* x, const float* y,
+                              const float* yaw, const float* ranges, int8_t* grids, const PlanEvent* events,
+                              const int* ev_start, const int2* s_min, int gw, int gh) {
+  cudaStream_t st = g_ctx.stream();
+  const int gpf = (n_frames + 31) / 32;
+  g_ctx.w->boxes_valid = false;
+  int rc;
+  if ((rc = ensure_inv_table())) return rc;
+  int sw, sh, nsx, nsy;
+  choose_tiles(gw, gh, 80, &sw, &sh, &nsx, &nsy);
+  int pitch = (sw + 3) & ~3;
+  if (((pitch >> 2) & 1) == 0) pitch += 4;
+  const size_t smem = ((size_t)pitch * sh + kReplayQueueBytes) * kReplayWarps;
+  if (smem > 227u * 1024u) {
+    set_error("sub-tile %dx%d needs %zu B of shared memory per CTA (> 227 KB)", sw, sh, smem);
+    return UQS_ERR_BAD_ARG;
+  }
+  const size_t per_flight = (size_t)n_frames * (32 * sizeof(uint2) + sizeof(uint4)) + (size_t)gpf * sizeof(uint2);
+  int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)n_flights, g_ctx.scratch_budget / std::max<size_t>(per_flight, 1)));
+  chunk = std::min(chunk, 65535);                       // flights are gridDim.y of the ray set-up
+  if ((rc = g_ctx.w->rays.ensure((size_t)chunk * n_frames * 32 * sizeof(uint2))) ||
+      (rc = g_ctx.w->frames.ensure((size_t)chunk * n_frames * sizeof(uint4))) ||
+      (rc = g_ctx.w->groups.ensure((size_t)chunk * gpf * sizeof(uint2))) ||
+      (rc = g_ctx.w->counters.ensure(64 * sizeof(unsigned long long))))
+    return rc;
+  unsigned long long* counters = (unsigned long long*)g_ctx.w->counters.p;
+  cudaError_t e = zero_counted(counters, 8 * sizeof(unsigned long long), st);
+  if (e == cudaSuccess) e = zero_counted(grids, (size_t)n_flights * dp.W * dp.H, st);   // cells no sub-tile writes read 0
+  if (e != cudaSuccess) return cuda_fail(e, "memset before the recentering replay");
+  int ctas_per_sm = 0;
+  if ((e = tiles_recenter_prepare(smem, &ctas_per_sm)) != cudaSuccess) return cuda_fail(e, "occupancy(k_replay_tiles)");
+  if (ctas_per_sm < 1) { set_error("replay kernel does not fit on an SM (smem %zu)", smem); return UQS_ERR_CUDA; }
+  for (int f0 = 0; f0 < n_flights; f0 += chunk) {
+    const int nf = std::min(chunk, n_flights - f0);
+    const size_t fo = (size_t)f0 * n_frames;
+    KernelTimer t_setup(1);
+    e = ray_setup_recenter_launch(dim3((unsigned)gpf, (unsigned)nf), st, dp, n_frames, x + fo, y + fo, yaw + fo, ranges + fo * 32,
+                                  (const uint32_t*)g_ctx.inv_table.p, (uint4*)g_ctx.w->frames.p, (uint2*)g_ctx.w->groups.p,
+                                  (uint2*)g_ctx.w->rays.p, counters, events, ev_start + f0, s_min + f0);
+    t_setup.stop();
+    if (e != cudaSuccess) return cuda_fail(e, "k_ray_setup launch");
+    ReplayArgs A = {};
+    A.tile_order = nullptr;
+    A.n_flights = nf;
+    A.frames = (const uint4*)g_ctx.w->frames.p;
+    A.groups = (const uint2*)g_ctx.w->groups.p;
+    A.rays = (const uint2*)g_ctx.w->rays.p;
+    A.grids = grids + (size_t)f0 * dp.W * dp.H;
+    A.job_counter = counters + 8;
+    A.total_jobs = (unsigned long long)nf * nsx * nsy;
+    A.slices = 1; A.groups_per_slice = gpf; A.pitch_cells = sw | 1;
+    A.maps = nullptr;
+    A.n_frames = n_frames; A.groups_per_flight = gpf;
+    A.W = gw; A.H = gh; A.row0 = 0; A.rows = gh;
+    A.sw = sw; A.sh = sh; A.nsx = nsx; A.nsy = nsy;
+    A.pitch = pitch; A.tile_bytes = pitch * sh;
+    A.lo_free = dp.lo_free; A.lo_occ = dp.lo_occ; A.lo_min = dp.lo_min; A.lo_max = dp.lo_max;
+    A.end_nohit = dp.end_nohit;
+    A.accumulate = 0;
+    RecenterArgs R;
+    R.events = events; R.ev_start = ev_start + f0; R.s_min = s_min + f0;
+    R.W = dp.W; R.H = dp.H;
+    e = zero_counted(A.job_counter, sizeof(unsigned long long), st);
+    if (e != cudaSuccess) return cuda_fail(e, "memset job counter");
+    const unsigned long long want = (A.total_jobs + kReplayWarps - 1) / kReplayWarps;
+    const unsigned grid = (unsigned)std::min<unsigned long long>(want, (unsigned long long)ctas_per_sm * g_ctx.sm_count);
+    KernelTimer t_rep(2);
+    e = tiles_recenter_launch(grid, smem, st, A, R);
     t_rep.stop();
     if (e != cudaSuccess) return cuda_fail(e, "k_replay_tiles launch");
     g_ctx.launches += 2;
@@ -824,10 +912,10 @@ int uqs_beam_cells(const uqs_params* p, int n_frames, const float* x, const floa
     return rc;
   cudaError_t e = cudaMemsetAsync(g_ctx.w->counters.p, 0, 64, st);
   if (e != cudaSuccess) return cuda_fail(e, "memset");
-  k_ray_setup<<<(unsigned)gpf, 1024, 0, st>>>(dp, n_frames, (float*)g_ctx.in_x.p, (float*)g_ctx.in_y.p,
-                                              (float*)g_ctx.in_yaw.p, (float*)g_ctx.in_ranges.p, nullptr, 0,
-                                              (const uint32_t*)g_ctx.inv_table.p, (uint4*)g_ctx.w->frames.p, (uint2*)g_ctx.w->groups.p,
-                                              (uint2*)g_ctx.w->rays.p, (unsigned long long*)g_ctx.w->counters.p);
+  e = ray_setup_launch(dim3((unsigned)gpf), st, dp, n_frames, (float*)g_ctx.in_x.p, (float*)g_ctx.in_y.p, (float*)g_ctx.in_yaw.p,
+                       (float*)g_ctx.in_ranges.p, nullptr, 0, (const uint32_t*)g_ctx.inv_table.p, (uint4*)g_ctx.w->frames.p,
+                       (uint2*)g_ctx.w->groups.p, (uint2*)g_ctx.w->rays.p, (unsigned long long*)g_ctx.w->counters.p);
+  if (e != cudaSuccess) return cuda_fail(e, "k_ray_setup launch");
   int32_t* d_cells = (int32_t*)g_ctx.out_grids.p;
   int32_t* d_origin = d_cells + n * 64;
   k_records_to_cells<<<(unsigned)((n * 32 + 255) / 256), 256, 0, st>>>((long long)n, (uint4*)g_ctx.w->frames.p,
@@ -864,11 +952,10 @@ int uqs_frame_bounds(const uqs_params* p, int n_frames, const float* x, const fl
     return rc;
   cudaError_t e = cudaMemsetAsync(g_ctx.w->counters.p, 0, 64, st);
   if (e != cudaSuccess) return cuda_fail(e, "memset");
-  k_ray_setup<<<(unsigned)gpf, 1024, 0, st>>>(dp, n_frames, (float*)g_ctx.in_x.p, (float*)g_ctx.in_y.p,
-                                              (float*)g_ctx.in_yaw.p, (float*)g_ctx.in_ranges.p, nullptr, 1 + g_ctx.k0_bias,
-                                              (const uint32_t*)g_ctx.inv_table.p, (uint4*)g_ctx.w->frames.p, (uint2*)g_ctx.w->groups.p,
-                                              (uint2*)g_ctx.w->rays.p, (unsigned long long*)g_ctx.w->counters.p);
-  e = cudaGetLastError();
+  e = ray_setup_launch(dim3((unsigned)gpf), st, dp, n_frames, (float*)g_ctx.in_x.p, (float*)g_ctx.in_y.p, (float*)g_ctx.in_yaw.p,
+                       (float*)g_ctx.in_ranges.p, nullptr, 1 + g_ctx.k0_bias, (const uint32_t*)g_ctx.inv_table.p,
+                       (uint4*)g_ctx.w->frames.p, (uint2*)g_ctx.w->groups.p, (uint2*)g_ctx.w->rays.p,
+                       (unsigned long long*)g_ctx.w->counters.p);
   if (e != cudaSuccess) return cuda_fail(e, "k_ray_setup launch");
   std::vector<uint4> fr(n);
   e = cudaMemcpyAsync(fr.data(), g_ctx.w->frames.p, n * sizeof(uint4), cudaMemcpyDeviceToHost, st);

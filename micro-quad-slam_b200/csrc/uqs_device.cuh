@@ -142,7 +142,19 @@ __device__ __forceinline__ int lrintf_as_int(float q) {
   return (int)r;
 }
 
-// world_to_grid(), uav_local_nav.c:205-214
+// world_to_grid(), uav_local_nav.c:205-214, with the map origin (ox, oy) (map_origin_x/y, which recentering moves)
+__device__ __forceinline__ bool world_to_grid_at(const DevParams& p, float ox, float oy, float wx, float wy, int& gx,
+                                                 int& gy) {
+  const float ddx = __fsub_rn(wx, ox);
+  const float ddy = __fsub_rn(wy, oy);
+  const int ix = (int)((unsigned)lrintf_as_int(__fdiv_rn(ddx, p.res)) + (unsigned)p.halfW);
+  const int iy = (int)((unsigned)lrintf_as_int(__fdiv_rn(ddy, p.res)) + (unsigned)p.halfH);
+  gx = ix;
+  gy = iy;
+  return !(ix < 0 || ix >= p.W || iy < 0 || iy >= p.H);
+}
+
+// world_to_grid(), uav_local_nav.c:205-214, with the origin of p
 __device__ __forceinline__ bool world_to_grid(const DevParams& p, float wx, float wy, int& gx,
                                               int& gy) {
   const float ddx = __fsub_rn(wx, p.ox);

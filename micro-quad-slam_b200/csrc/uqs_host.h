@@ -26,6 +26,7 @@ struct DevBuf {
 struct Work {
   DevBuf rays, frames, groups, counters, inc, scan, order, maps, boxes;
   DevBuf probe_slots, probe_keys, probe_sorted, probe_start, probe_tmp;   // frontier probes and buckets (uqs_frontier.cu)
+  DevBuf plan_info, plan_start, plan_events, plan_tmp;                   // recenter plans (uqs_next.cu)
   int order_nsx = 0, order_nsy = 0;             // geometry the cached tile order was built for
   cudaStream_t stream = nullptr;
   int* h_dims = nullptr;                        // mapped host words the box kernel publishes its maxima to
@@ -35,7 +36,7 @@ struct Work {
     if (h_dims) cudaFreeHost(h_dims);
     h_dims = nullptr;
     DevBuf* all[] = { &rays, &frames, &groups, &counters, &inc, &scan, &order, &maps, &boxes, &probe_slots, &probe_keys, &probe_sorted,
-                      &probe_start, &probe_tmp };
+                      &probe_start, &probe_tmp, &plan_info, &plan_start, &plan_events, &plan_tmp };
     order_nsx = order_nsy = 0;
     for (DevBuf* b : all) b->release();
   }
@@ -124,6 +125,13 @@ int replay_device(const DevParams& dp, int n_flights, int n_frames, const float*
                   const float* yaw, const float* ranges, const uint8_t* kind, int8_t* grids,
                   int accumulate, int row0, int rows, bool reset_stats, const ProbeSet* probes = nullptr);
 int fetch_stats(uqs_stats* stats, uint64_t frames);
+// sub-tile geometry and time slices replay_device chooses for a call
+void tile_geometry(const DevParams& dp, int n_flights, int n_frames, int rows, int* sw, int* sh, int* nsx, int* nsy,
+                   int* slices);
+// recentred flights through the sub-tile engine, records in each flight's global frame (gw x gh: the largest extent)
+int replay_device_recentering(const DevParams& dp, int n_flights, int n_frames, const float* x, const float* y,
+                              const float* yaw, const float* ranges, int8_t* grids, const PlanEvent* events,
+                              const int* ev_start, const int2* s_min, int gw, int gh);
 int ensure_inv_table();
 // uqs_generic.cu: the unrestricted replay and the start-grid range check
 cudaError_t generic_launch(const DevParams& dp, int n_flights, int n_frames, const float* x, const float* y, const float* yaw,

@@ -251,17 +251,22 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
 // kind == nullptr: every entry is a frame (pose + 32 ranges).
 // kind[i] == 1   : entry i is one raw ray raycast_update(x0,y0,x1,y1,hit) stored as
 //                  x=x0, y=y0, yaw=x1, ranges[0]=y1, ranges[1]=hit (drop-in symbol only).
+// RECENTER: frame f of a flight is set up as log_tick() maps it after map_recentre_if_needed(): world_to_grid() with
+// the origin of the flight's last event at a frame <= f, in window coordinates (its off-grid test included); only then
+// are the cells moved into the flight's global frame by S - s_min of that event.  dx, dy do not change.
+template <bool RECENTER>
 __global__ void __launch_bounds__(1024, 2)
 k_ray_setup(const __grid_constant__ DevParams p, int n_frames, const float* __restrict__ x,
             const float* __restrict__ y, const float* __restrict__ yaw_deg,
             const float* __restrict__ ranges, const uint8_t* __restrict__ kind, int want_k0,
             const uint32_t* __restrict__ inv_table, uint4* __restrict__ frames, uint2* __restrict__ groups, uint2* __restrict__ rays,
-            unsigned long long* __restrict__ stats /* [4]: U, accepted, skipped, domain */) {
+            unsigned long long* __restrict__ stats /* [4]: U, accepted, skipped, domain */,
+            const PlanEvent* __restrict__ events, const int* __restrict__ ev_start, const int2* __restrict__ s_min) {
   __shared__ __align__(128) float s_rng[32 * 32];
   __shared__ __align__(8) unsigned long long s_bar;
   __shared__ int s_box[4][32];
   __shared__ unsigned s_cnt[2][32];
-  __shared__ int s_org[32][2];
+  __shared__ int s_org[32][RECENTER ? 6 : 2];      // start cell (+ the frame's origin and its offset into the global frame)
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int flight = blockIdx.y, g = blockIdx.x, groups_per_flight = gridDim.x;
   const int f = g * 32 + w;
@@ -293,7 +298,30 @@ k_ray_setup(const __grid_constant__ DevParams p, int n_frames, const float* __re
   if (w == 31) {
     int ox = -1, oy = -1;
     const int fo = g * 32 + lane;
-    if (fo < n_frames && !world_to_grid(p, x[fbase + fo], y[fbase + fo], ox, oy)) ox = oy = -1;
+    if (!RECENTER) {
+      if (fo < n_frames && !world_to_grid(p, x[fbase + fo], y[fbase + fo], ox, oy)) ox = oy = -1;
+    } else {
+      float mx = p.ox, my = p.oy;                                  // the origin at frame fo, and S - s_min
+      int offx = 0, offy = 0;
+      if (fo < n_frames) {
+        const int eb = ev_start[flight];
+        int lo = eb, hi = ev_start[flight + 1];                    // first event of a frame > fo
+        while (lo < hi) {
+          const int mid = (lo + hi) >> 1;
+          if (events[mid].frame <= fo) lo = mid + 1; else hi = mid;
+        }
+        int sx = 0, sy = 0;
+        if (lo > eb) { const PlanEvent& e = events[lo - 1]; mx = e.ox; my = e.oy; sx = e.Sx; sy = e.Sy; }
+        const int2 smin = s_min[flight];
+        offx = sx - smin.x;
+        offy = sy - smin.y;
+        if (!world_to_grid_at(p, mx, my, x[fbase + fo], y[fbase + fo], ox, oy)) ox = oy = -1;
+      }
+      s_org[lane][2] = __float_as_int(mx);
+      s_org[lane][3] = __float_as_int(my);
+      s_org[lane][4] = offx;
+      s_org[lane][5] = offy;
+    }
     s_org[lane][0] = ox;
     s_org[lane][1] = oy;
   }
@@ -323,14 +351,20 @@ k_ray_setup(const __grid_constant__ DevParams p, int n_frames, const float* __re
   __syncthreads();
 
   if (live) {
-    const int gx0 = s_org[w][0], gy0 = s_org[w][1];
-    const bool have_o = gx0 >= 0;
+    const bool have_o = s_org[w][0] >= 0;
+    // window cells; in the global frame for RECENTER (-1 stays the off-grid mark)
+    const int gx0 = s_org[w][0] + (RECENTER && have_o ? s_org[w][RECENTER ? 4 : 0] : 0);
+    const int gy0 = s_org[w][1] + (RECENTER && have_o ? s_org[w][RECENTER ? 5 : 0] : 0);
     uint32_t w0 = 0, w1 = 0;
     if (st < 0) {
       domain = 1;
     } else if (st > 0 && have_o) {
       int gx1, gy1;
-      if (world_to_grid(p, ex, ey, gx1, gy1)) {
+      const bool on_grid = RECENTER ? world_to_grid_at(p, __int_as_float(s_org[w][RECENTER ? 2 : 0]),
+                                                       __int_as_float(s_org[w][RECENTER ? 3 : 0]), ex, ey, gx1, gy1)
+                                    : world_to_grid(p, ex, ey, gx1, gy1);
+      if (on_grid) {
+        if (RECENTER) { gx1 += s_org[w][RECENTER ? 4 : 0]; gy1 += s_org[w][RECENTER ? 5 : 0]; }
         const int dx = gx1 - gx0, dy = gy1 - gy0;
         const int m = max(abs(dx), abs(dy));
         if (m > kMaxRayCells) {
@@ -458,6 +492,23 @@ k_ray_setup(const __grid_constant__ DevParams p, int n_frames, const float* __re
       if (t) atomicAdd(&stats[lane], t);
     }
   }
+}
+
+cudaError_t ray_setup_launch(dim3 grid, cudaStream_t st, const DevParams& p, int n_frames, const float* x, const float* y,
+                             const float* yaw_deg, const float* ranges, const uint8_t* kind, int want_k0,
+                             const uint32_t* inv_table, uint4* frames, uint2* groups, uint2* rays, unsigned long long* stats) {
+  k_ray_setup<false><<<grid, 1024, 0, st>>>(p, n_frames, x, y, yaw_deg, ranges, kind, want_k0, inv_table, frames, groups, rays,
+                                            stats, nullptr, nullptr, nullptr);
+  return cudaGetLastError();
+}
+
+cudaError_t ray_setup_recenter_launch(dim3 grid, cudaStream_t st, const DevParams& p, int n_frames, const float* x,
+                                      const float* y, const float* yaw_deg, const float* ranges, const uint32_t* inv_table,
+                                      uint4* frames, uint2* groups, uint2* rays, unsigned long long* stats,
+                                      const PlanEvent* events, const int* ev_start, const int2* s_min) {
+  k_ray_setup<true><<<grid, 1024, 0, st>>>(p, n_frames, x, y, yaw_deg, ranges, nullptr, 0, inv_table, frames, groups, rays,
+                                           stats, events, ev_start, s_min);
+  return cudaGetLastError();
 }
 
 // Parity hook: end cell of every beam from the records (cells [-1,-1] when skipped).
@@ -679,9 +730,15 @@ extern __shared__ __align__(16) unsigned char uqs_smem[];
 // PROBE: also serves the job's frontier probes (bucket (flight, slice, sub-tile), frame order).  A probe of frame p is
 // read when every ray of frames <= p that reaches the sub-tile has been applied: before the rays of the first hit frame
 // g > p are queued (after a flush of the queue, which may still hold rays of frames < g), or when the job ends.
-template <bool PROBE>
+// RECENTER: the flights were recentred (R) and the records are in each flight's global frame; A.W x A.H is the largest
+// global extent of the launch, which the sub-tiles cover.  Every global cell outside the flight's current window is 0,
+// so a recenter event only zeroes the sub-tile's cells that have left the window: the warp applies the events of
+// frames <= f before queueing frame f's rays (after a flush: the queue may hold rays of earlier frames) and the rest
+// at job end.  A sub-tile no ray reached stays 0 and is not written back (the grids were zeroed); the others write
+// their cells inside the final window to the flight's grid.  Value tiles only: no accumulation, no time slices.
+template <bool PROBE, bool RECENTER = false>
 __global__ void __launch_bounds__(kReplayThreads)
-k_replay_tiles(ReplayArgs A, ProbeArgs Q) {
+k_replay_tiles(ReplayArgs A, ProbeArgs Q, RecenterArgs R) {
   const int lane = threadIdx.x & 31;
   const int wic = threadIdx.x >> 5;
   int8_t* tile = reinterpret_cast<int8_t*>(uqs_smem) + (size_t)wic * A.tile_bytes;
@@ -713,9 +770,9 @@ k_replay_tiles(ReplayArgs A, ProbeArgs Q) {
     const int X0 = (sub % A.nsx) * A.sw, Y0 = A.row0 + (sub / A.nsx) * A.sh;
     const int X1 = min(X0 + A.sw, A.W), Y1 = min(Y0 + A.sh, A.row0 + A.rows);
     const int tw = X1 - X0, th = Y1 - Y0;
-    int8_t* grid = A.grids + (size_t)flight * A.W * A.H;
-    const bool vec = ((A.W | X0 | tw) & 3) == 0 && ((reinterpret_cast<size_t>(grid) & 3) == 0);
-    const bool map = slice > 0;
+    int8_t* grid = RECENTER ? A.grids + (size_t)flight * R.W * R.H : A.grids + (size_t)flight * A.W * A.H;
+    const bool vec = !RECENTER && ((A.W | X0 | tw) & 3) == 0 && ((reinterpret_cast<size_t>(grid) & 3) == 0);
+    const bool map = !RECENTER && slice > 0;
     TileRegions DR;
     DR.tile.lo = tile_s;
     DR.tile.hi = tile_s + (uint32_t)(map ? A.pitch_cells * th * 4 : A.pitch * th);
@@ -796,6 +853,39 @@ k_replay_tiles(ReplayArgs A, ProbeArgs Q) {
         next_pf = pb < pe ? Q.probes[pb].x : 0x7fffffff;
       }
     };
+    // RECENTER: the flight's events [ei, ee), the frame of the next one, the current window's corner in the tile frame
+    int ei = 0, ee = 0, next_ef = 0x7fffffff, smx = 0, smy = 0, wx0 = 0, wy0 = 0;
+    bool touched = false;
+    if (RECENTER) {
+      ei = R.ev_start[flight];
+      ee = R.ev_start[flight + 1];
+      if (ei < ee) next_ef = R.events[ei].frame;
+      const int2 sm = R.s_min[flight];
+      smx = sm.x; smy = sm.y;
+      wx0 = -smx; wy0 = -smy;                                      // S = 0 before the first event
+    }
+    // apply every event of a frame <= fmax
+    auto advance = [&](int fmax) {
+      while (next_ef <= fmax) {
+        const PlanEvent& e = R.events[ei];
+        wx0 = e.Sx - smx;
+        wy0 = e.Sy - smy;
+        ei++;
+        next_ef = ei < ee ? R.events[ei].frame : 0x7fffffff;
+        if (!touched || (X0 >= wx0 && X1 <= wx0 + R.W && Y0 >= wy0 && Y1 <= wy0 + R.H)) continue;
+        while (qn > 0) flush();
+        __syncwarp();
+        for (int i = lane; i < tw * th; i += 32) {
+          const int r = i / tw, c = i - r * tw;
+          const int u = X0 + c - wx0, v = Y0 + r - wy0;
+          if (u < 0 || u >= R.W || v < 0 || v >= R.H) {
+            UQS_CHECK(tile_s + (uint32_t)(r * A.pitch + c), 1u, DR.tile);
+            tile[r * A.pitch + c] = 0;
+          }
+        }
+        __syncwarp();
+      }
+    };
     for (int g0 = g_begin; g0 < g_end; g0 += 32) {
       bool ghit = false;
       if (g0 + lane < g_end) {
@@ -819,6 +909,7 @@ k_replay_tiles(ReplayArgs A, ProbeArgs Q) {
           const uint2 rec = rec_next;
           if (fmask) rec_next = __ldg(&rays[(size_t)(f0 + __ffs(fmask) - 1) * 32 + lane]);
           if (PROBE) serve(f0 + fi);
+          if (RECENTER) advance(f0 + fi);
           const int gx0 = (int)(__shfl_sync(0xffffffffu, fr.x, fi) & 0xffffu);
           const int gy0 = (int)(__shfl_sync(0xffffffffu, fr.y, fi) & 0xffffu);
           const int ex = gx0 + sext12(rec.x), ey = gy0 + sext12(rec.x >> 12);
@@ -834,6 +925,7 @@ k_replay_tiles(ReplayArgs A, ProbeArgs Q) {
             sts_u32(at + 8u * kQueueEntries, (uint32_t)gx0 | ((uint32_t)gy0 << 16));
           }
           qn += __popc(nm);
+          touched = true;
           if (qn >= 32) flush();                               // at most 63 queued before, at most 31 after
         }
       }
@@ -841,9 +933,16 @@ k_replay_tiles(ReplayArgs A, ProbeArgs Q) {
     while (qn > 0) flush();
     __syncwarp();
     if (PROBE) serve(0x7fffffff);                       // frames no ray of which reached the sub-tile
+    if (RECENTER) advance(0x7ffffffe);                   // events after the last frame that reached the sub-tile
 
     // ---- write the sub-tile back: values into the grid, maps into the slice scratch ---------
-    if (map) {
+    if (RECENTER) {
+      for (int i = lane; touched && i < tw * th; i += 32) {
+        const int r = i / tw, c = i - r * tw;
+        const int u = X0 + c - wx0, v = Y0 + r - wy0;
+        if (u >= 0 && u < R.W && v >= 0 && v < R.H) grid[(size_t)v * R.W + u] = tile[r * A.pitch + c];
+      }
+    } else if (map) {
       uint32_t* out = A.maps + ((size_t)flight * (S - 1) + (slice - 1)) * A.W * A.H;
       for (int i = lane; i < tw * th; i += 32) {
         const int r = i / tw, c = i - r * tw;
@@ -1405,15 +1504,26 @@ cudaError_t flights_probe_launch(int nw, unsigned grid, size_t smem, cudaStream_
 }
 
 cudaError_t tiles_prepare(bool probe, size_t smem, int* ctas_per_sm) {
-  void (*k)(ReplayArgs, ProbeArgs) = probe ? k_replay_tiles<true> : k_replay_tiles<false>;
+  void (*k)(ReplayArgs, ProbeArgs, RecenterArgs) = probe ? k_replay_tiles<true> : k_replay_tiles<false>;
   cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, k, kReplayThreads, smem);
 }
 
 cudaError_t tiles_launch(bool probe, unsigned grid, size_t smem, cudaStream_t st, const ReplayArgs& A, const ProbeArgs& Q) {
-  if (probe) k_replay_tiles<true><<<grid, kReplayThreads, smem, st>>>(A, Q);
-  else       k_replay_tiles<false><<<grid, kReplayThreads, smem, st>>>(A, Q);
+  if (probe) k_replay_tiles<true><<<grid, kReplayThreads, smem, st>>>(A, Q, RecenterArgs{});
+  else       k_replay_tiles<false><<<grid, kReplayThreads, smem, st>>>(A, Q, RecenterArgs{});
+  return cudaGetLastError();
+}
+
+cudaError_t tiles_recenter_prepare(size_t smem, int* ctas_per_sm) {
+  cudaError_t e = cudaFuncSetAttribute(k_replay_tiles<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, k_replay_tiles<false, true>, kReplayThreads, smem);
+}
+
+cudaError_t tiles_recenter_launch(unsigned grid, size_t smem, cudaStream_t st, const ReplayArgs& A, const RecenterArgs& R) {
+  k_replay_tiles<false, true><<<grid, kReplayThreads, smem, st>>>(A, ProbeArgs{}, R);
   return cudaGetLastError();
 }
 

@@ -57,6 +57,22 @@ struct ProbeArgs {
   int n_buckets;
 };
 
+// Recentering (uqs_next.cu).  One recenter event of a flight: the shift (sx, sy) applied before `frame` is mapped, the
+// map origin after it (binary32, as uav_local_nav.c:346-347 leaves it) and S, the sum of every shift applied so far.
+// A flight's cells are numbered in its global frame, global = window cell + S; the replay's grids hold global cells
+// minus the flight's smallest S (s_min), so that they start at 0.
+struct __align__(16) PlanEvent {
+  int frame, sx, sy, pad;
+  int Sx, Sy;
+  float ox, oy;
+};
+struct RecenterArgs {
+  const PlanEvent* events;  // every flight's events in frame order
+  const int* ev_start;      // [n_flights + 1] (launch-local flights): flight f's events are [ev_start[f], ev_start[f+1])
+  const int2* s_min;        // [n_flights] the flight's smallest S
+  int W, H;                 // the window: the map the drone holds
+};
+
 struct ScanState;
 
 __global__ void k_pose_increments(long long total, int n_samples, const uint32_t* t_ms,
@@ -73,11 +89,16 @@ size_t pose_scan_state_bytes();
 cudaError_t zero_async(void* p, size_t bytes, cudaStream_t st);   // zero fill by a kernel (never a copy engine)
 int pose_scan_threads();
 
-__global__ void k_ray_setup(const __grid_constant__ DevParams p, int n_frames, const float* x,
-                            const float* y, const float* yaw_deg, const float* ranges,
-                            const uint8_t* kind, int want_k0, const uint32_t* inv_table, uint4* frames, uint2* groups,
-                            uint2* rays,
-                            unsigned long long* stats);
+// k_ray_setup: the ray and frame records of a chunk of flights (grid = (groups per flight, flights))
+cudaError_t ray_setup_launch(dim3 grid, cudaStream_t st, const DevParams& p, int n_frames, const float* x, const float* y,
+                             const float* yaw_deg, const float* ranges, const uint8_t* kind, int want_k0,
+                             const uint32_t* inv_table, uint4* frames, uint2* groups, uint2* rays, unsigned long long* stats);
+// the same for recentred flights: each frame is set up against its flight's origin at that frame, and its records are
+// in the flight's global frame (events, ev_start and s_min as in RecenterArgs)
+cudaError_t ray_setup_recenter_launch(dim3 grid, cudaStream_t st, const DevParams& p, int n_frames, const float* x,
+                                      const float* y, const float* yaw_deg, const float* ranges, const uint32_t* inv_table,
+                                      uint4* frames, uint2* groups, uint2* rays, unsigned long long* stats,
+                                      const PlanEvent* events, const int* ev_start, const int2* s_min);
 __global__ void k_records_to_cells(long long n_frames, const uint4* frames, const uint2* rays,
                                    int32_t* cells, int32_t* origin);
 __global__ void k_sincosf(size_t n, const float* a, float* s, float* c);
@@ -85,6 +106,9 @@ __global__ void k_world_to_grid_one(DevParams p, float wx, float wy, int* out);
 // the sub-tile engine (k_replay_tiles), plain or serving probes
 cudaError_t tiles_prepare(bool probe, size_t smem, int* ctas_per_sm);
 cudaError_t tiles_launch(bool probe, unsigned grid, size_t smem, cudaStream_t st, const ReplayArgs& A, const ProbeArgs& Q);
+// the sub-tile engine replaying recentred flights: tiles cover the flights' global frames (no probes, no time slices)
+cudaError_t tiles_recenter_prepare(size_t smem, int* ctas_per_sm);
+cudaError_t tiles_recenter_launch(unsigned grid, size_t smem, cudaStream_t st, const ReplayArgs& A, const RecenterArgs& R);
 __global__ void k_compose_slices(int8_t* grids, const uint32_t* maps, int n_flights, int W, int H, int S, int row0,
                                  int rows);
 cudaError_t flights_probe_prepare(int nw, size_t smem, int* ctas_per_sm);

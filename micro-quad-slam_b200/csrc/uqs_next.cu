@@ -3,6 +3,8 @@
 //   N2  map recentering                      map_recenter_shift / map_recentre_if_needed,  uav_local_nav.c:308-353
 //   N3  frontier scoring (grid consumer)     frontier_score_dir,                           uav_local_nav.c:356-385
 // Same rules as the hot path: one rounding per C operator, glibc sincosf restated, no host arithmetic.
+#include <algorithm>
+#include <climits>
 #include <cmath>
 #include <cstdio>
 #include <vector>
@@ -50,8 +52,6 @@ __global__ void k_scans_to_beams(long long n, const uint8_t* __restrict__ raw, f
 // ---------------------------------------------------------------------------------------------
 // N2: recentering
 // ---------------------------------------------------------------------------------------------
-struct RecenterEvent { int frame, sx, sy; float ox, oy; };     // shift applied BEFORE `frame` is mapped
-
 // map_recentre_if_needed(), :324-349, decision only: returns true and the shift when one is due
 __device__ __forceinline__ bool recenter_decide(float res, float size_m, float ox, float oy, float x, float y,
                                                 int& sx, int& sy) {
@@ -67,21 +67,64 @@ __device__ __forceinline__ bool recenter_decide(float res, float size_m, float o
   return !(sx == 0 && sy == 0);
 }
 
-// one thread walks one log in order (the decision depends on poses and the running origin only)
-__global__ void k_recenter_plan(int n_frames, const float* __restrict__ x, const float* __restrict__ y, float res,
-                                float size_m, float ox, float oy, RecenterEvent* events, int max_events, int* n_events) {
-  if (blockIdx.x != 0 || threadIdx.x != 0) return;
+// One thread per flight walks its poses in order: the decision depends on the poses and the running origin only, so
+// the whole plan exists before any replay.  Pass 1 (WRITE = false): info[f] = {events, min Sx, min Sy, max Sx, max Sy}
+// (S = 0 included: the first window) and s_min[f].  Pass 2: the events, at ev_start[f].  S is summed in 64 bits and
+// its extremes saturate at +-2^30 (such a flight cannot take the sub-tile route anyway).
+constexpr int kPlanInfo = 5;
+template <bool WRITE>
+__global__ void k_recenter_plan(int n_flights, int n_frames, const float* __restrict__ x, const float* __restrict__ y,
+                                float res, float size_m, float ox, float oy, int* __restrict__ info, int2* __restrict__ s_min,
+                                const int* __restrict__ ev_start, PlanEvent* __restrict__ events) {
+  const int f = blockIdx.x * blockDim.x + threadIdx.x;
+  if (f >= n_flights) return;
+  const float* xf = x + (size_t)f * n_frames;
+  const float* yf = y + (size_t)f * n_frames;
+  PlanEvent* out = WRITE ? events + ev_start[f] : nullptr;
+  long long Sx = 0, Sy = 0, lo_x = 0, lo_y = 0, hi_x = 0, hi_y = 0;
   int n = 0;
-  for (int f = 0; f < n_frames; f++) {
+  for (int i = 0; i < n_frames; i++) {
     int sx, sy;
-    if (recenter_decide(res, size_m, ox, oy, x[f], y[f], sx, sy)) {
+    if (recenter_decide(res, size_m, ox, oy, __ldg(&xf[i]), __ldg(&yf[i]), sx, sy)) {
       ox = __fadd_rn(ox, __fmul_rn((float)sx, res));                     // :346-347
       oy = __fadd_rn(oy, __fmul_rn((float)sy, res));
-      if (n < max_events) events[n] = { f, sx, sy, ox, oy };
+      Sx += sx;
+      Sy += sy;
+      if (WRITE) {
+        out[n] = { i, sx, sy, 0, (int)Sx, (int)Sy, ox, oy };
+      } else {
+        lo_x = min(lo_x, Sx); lo_y = min(lo_y, Sy);
+        hi_x = max(hi_x, Sx); hi_y = max(hi_y, Sy);
+      }
       n++;
     }
   }
-  *n_events = n;
+  if (!WRITE) {
+    const long long cap = 1ll << 30;
+    int* o = info + (size_t)f * kPlanInfo;
+    o[0] = n;
+    o[1] = (int)max(lo_x, -cap); o[2] = (int)max(lo_y, -cap);
+    o[3] = (int)min(hi_x, cap);  o[4] = (int)min(hi_y, cap);
+    s_min[f] = make_int2(o[1], o[2]);
+  }
+}
+
+// per flight: the final origin, the event count and the first max_events {frame, sx, sy}
+__global__ void k_recenter_outputs(int n_flights, const int* __restrict__ ev_start, const PlanEvent* __restrict__ events,
+                                   float ox, float oy, float* __restrict__ origins, int32_t* __restrict__ n_events,
+                                   int32_t* __restrict__ events_out, int max_events) {
+  const int f = blockIdx.x * blockDim.x + threadIdx.x;
+  if (f >= n_flights) return;
+  const int eb = ev_start[f], n = ev_start[f + 1] - eb;
+  origins[2 * f] = n ? events[eb + n - 1].ox : ox;
+  origins[2 * f + 1] = n ? events[eb + n - 1].oy : oy;
+  n_events[f] = n;
+  for (int k = 0; k < n && k < max_events; k++) {
+    int32_t* e = events_out + ((size_t)f * max_events + k) * 3;
+    e[0] = events[eb + k].frame;
+    e[1] = events[eb + k].sx;
+    e[2] = events[eb + k].sy;
+  }
 }
 
 __global__ void k_recenter_decide_one(float res, float size_m, float ox, float oy, float x, float y, int* out) {
@@ -203,9 +246,122 @@ int uqs_frontier_scores(const uqs_params* p, const int8_t* grid /* host, [H][W] 
   return UQS_OK;
 }
 
-/* N2: one log replayed with the reference's recentering honoured (log_tick order, :1629-1635:
- * recentre check first, then the update).  origin_out = final map origin; events_out (may be NULL, capacity
- * max_events) gets {frame, sx, sy} triples. */
+/* N2 for many flights.  Route A, the sub-tile engine in each flight's global frame, when the inputs suit it: rays of
+ * at most kMaxRayCells cells, 0 inside the clamp range, no time slices for this call, global extents that fit the
+ * records' 16-bit cells, engine 0 or 1.  Route B otherwise: per flight, the log between two events through
+ * replay_device at that segment's origin, then the shift, with the stats summed on the device. */
+int uqs_replay_recentering_dev(const uqs_params* p, int n_flights, int n_frames, const float* x, const float* y,
+                               const float* yaw, const float* ranges, int8_t* grids, float* origins, int32_t* n_events,
+                               int32_t* events, int max_events, uqs_stats* stats) {
+  int rc = check_ready();
+  if (rc) return rc;
+  DevParams dp;
+  if ((rc = make_dev_params(p, &dp))) return rc;
+  if (n_flights <= 0 || n_frames <= 0 || !x || !y || !yaw || !ranges || !grids || !origins || !n_events || max_events < 0 ||
+      (max_events > 0 && !events)) {
+    set_error("uqs_replay_recentering_dev: NULL pointer or bad size");
+    return UQS_ERR_BAD_ARG;
+  }
+  if (g_ctx.engine == 2) {
+    set_error("uqs_replay_recentering_dev: engine 2 (resident) has no recentering variant; use 0, 1 or 3");
+    return UQS_ERR_BAD_ARG;
+  }
+  cudaStream_t st = g_ctx.stream();
+  Work& W = *g_ctx.w;
+  const size_t info_bytes = ((size_t)n_flights * kPlanInfo * sizeof(int) + 15) & ~(size_t)15;
+  if ((rc = W.plan_info.ensure(info_bytes + (size_t)n_flights * sizeof(int2))) ||
+      (rc = W.plan_start.ensure(((size_t)n_flights + 1) * sizeof(int))))
+    return rc;
+  int* d_info = (int*)W.plan_info.p;
+  int2* d_smin = (int2*)((char*)W.plan_info.p + info_bytes);
+  int* d_start = (int*)W.plan_start.p;
+  const unsigned blocks = (unsigned)((n_flights + 127) / 128);
+  k_recenter_plan<false><<<blocks, 128, 0, st>>>(n_flights, n_frames, x, y, p->res_m, p->size_m, p->origin_x, p->origin_y,
+                                                 d_info, d_smin, nullptr, nullptr);
+  std::vector<int> info((size_t)n_flights * kPlanInfo);
+  cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess) e = cudaMemcpyAsync(info.data(), d_info, info.size() * sizeof(int), cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  if (e != cudaSuccess) return cuda_fail(e, "k_recenter_plan");
+  g_ctx.launches += 1;
+  std::vector<int> start((size_t)n_flights + 1);
+  long long total = 0, span_x = 0, span_y = 0;
+  for (int f = 0; f < n_flights; f++) {
+    const int* o = &info[(size_t)f * kPlanInfo];
+    start[f] = (int)total;
+    total += o[0];
+    span_x = std::max(span_x, (long long)o[3] - o[1]);
+    span_y = std::max(span_y, (long long)o[4] - o[2]);
+    if (total > INT_MAX) { set_error("more than %d recenter events in one call", INT_MAX); return UQS_ERR_BAD_ARG; }
+  }
+  start[n_flights] = (int)total;
+  if ((rc = W.plan_events.ensure(std::max<size_t>(1, (size_t)total) * sizeof(PlanEvent)))) return rc;
+  PlanEvent* d_ev = (PlanEvent*)W.plan_events.p;
+  e = cudaMemcpyAsync(d_start, start.data(), start.size() * sizeof(int), cudaMemcpyHostToDevice, st);
+  if (e != cudaSuccess) return cuda_fail(e, "plan H2D");
+  k_recenter_plan<true><<<blocks, 128, 0, st>>>(n_flights, n_frames, x, y, p->res_m, p->size_m, p->origin_x, p->origin_y,
+                                                nullptr, nullptr, d_start, d_ev);
+  k_recenter_outputs<<<blocks, 128, 0, st>>>(n_flights, d_start, d_ev, p->origin_x, p->origin_y, origins, n_events, events,
+                                             max_events);
+  if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "k_recenter_plan");
+  g_ctx.launches += 2;
+
+  const int side = std::max(dp.W, dp.H);
+  const bool long_rays = side > kMaxRayCells + 1 && !(dp.max_range / dp.res + 3.0f <= (float)kMaxRayCells);
+  int sw, sh, nsx, nsy, slices;
+  tile_geometry(dp, n_flights, n_frames, dp.H, &sw, &sh, &nsx, &nsy, &slices);
+  const long long gw = span_x + dp.W, gh = span_y + dp.H;
+  const bool route_a = !long_rays && dp.lo_min <= 0 && dp.lo_max >= 0 && slices == 1 && gw <= 0x7fff && gh <= 0x7fff &&
+                       (g_ctx.engine == 0 || g_ctx.engine == 1);
+  if (route_a) {
+    if ((rc = replay_device_recentering(dp, n_flights, n_frames, x, y, yaw, ranges, grids, d_ev, d_start, d_smin, (int)gw,
+                                        (int)gh)))
+      return rc;
+  } else {
+    std::vector<PlanEvent> ev((size_t)total);
+    if (total) {
+      e = cudaMemcpyAsync(ev.data(), d_ev, (size_t)total * sizeof(PlanEvent), cudaMemcpyDeviceToHost, st);
+      if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+      if (e != cudaSuccess) return cuda_fail(e, "events D2H");
+    }
+    const size_t cells = (size_t)p->W * p->H;
+    if ((rc = W.plan_tmp.ensure(cells)) || (rc = W.counters.ensure(64 * sizeof(unsigned long long)))) return rc;
+    int8_t* tmp = (int8_t*)W.plan_tmp.p;
+    e = zero_async(W.counters.p, 8 * sizeof(unsigned long long), st);
+    if (e == cudaSuccess) e = zero_async(grids, (size_t)n_flights * cells, st);
+    if (e != cudaSuccess) return cuda_fail(e, "memset before the segment replay");
+    g_ctx.launches += 2;
+    for (int f = 0; f < n_flights; f++) {
+      uqs_params q = *p;
+      int8_t* g = grids + (size_t)f * cells;
+      const size_t base = (size_t)f * n_frames;
+      int f0 = 0;
+      for (int k = start[f]; k <= start[f + 1]; k++) {
+        const int f1 = k < start[f + 1] ? ev[k].frame : n_frames;
+        if (f1 > f0) {
+          DevParams dq;
+          if ((rc = make_dev_params(&q, &dq))) return rc;
+          if ((rc = replay_device(dq, 1, f1 - f0, x + base + f0, y + base + f0, yaw + base + f0, ranges + (base + f0) * 32,
+                                  nullptr, g, 1, 0, p->H, false)))
+            return rc;
+        }
+        if (k < start[f + 1]) {
+          k_recenter_shift<<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(g, tmp, p->W, p->H, ev[k].sx, ev[k].sy);
+          e = cudaGetLastError();
+          if (e == cudaSuccess) e = cudaMemcpyAsync(g, tmp, cells, cudaMemcpyDeviceToDevice, st);
+          if (e != cudaSuccess) return cuda_fail(e, "k_recenter_shift");
+          q.origin_x = ev[k].ox;
+          q.origin_y = ev[k].oy;
+          g_ctx.launches += 1;
+        }
+        f0 = f1;
+      }
+    }
+  }
+  return fetch_stats(stats, (uint64_t)n_flights * n_frames);
+}
+
+/* N2, one log from host buffers: uqs_replay_recentering_dev with one flight. */
 int uqs_replay_recentering(const uqs_params* p, int n_frames, const float* x, const float* y, const float* yaw_deg,
                            const float* ranges, int8_t* grid_out, float origin_out[2], int* n_events_out,
                            int* events_out, int max_events, uqs_stats* stats) {
@@ -216,63 +372,32 @@ int uqs_replay_recentering(const uqs_params* p, int n_frames, const float* x, co
   if (n_frames <= 0 || !x || !y || !yaw_deg || !ranges || !grid_out) { set_error("uqs_replay_recentering: bad argument"); return UQS_ERR_BAD_ARG; }
   cudaStream_t st = g_ctx.stream();
   const size_t cells = (size_t)p->W * p->H, n = (size_t)n_frames;
-  const int cap = 4096;
+  const int cap = events_out ? std::max(max_events, 0) : 0;
   if ((rc = stage(g_ctx.in_x, x, n * 4)) || (rc = stage(g_ctx.in_y, y, n * 4)) || (rc = stage(g_ctx.in_yaw, yaw_deg, n * 4)) ||
-      (rc = stage(g_ctx.in_ranges, ranges, n * 128)) || (rc = g_ctx.out_grids.ensure(2 * cells)) ||
-      (rc = g_ctx.in_t.ensure(cap * sizeof(RecenterEvent) + 16)))
+      (rc = stage(g_ctx.in_ranges, ranges, n * 128)) || (rc = g_ctx.out_grids.ensure(cells + 16)) ||
+      (rc = g_ctx.in_t.ensure((size_t)std::max(cap, 1) * 12)))
     return rc;
-  RecenterEvent* d_ev = (RecenterEvent*)g_ctx.in_t.p;
-  int* d_n = (int*)((char*)g_ctx.in_t.p + cap * sizeof(RecenterEvent));
-  k_recenter_plan<<<1, 1, 0, st>>>(n_frames, (float*)g_ctx.in_x.p, (float*)g_ctx.in_y.p, p->res_m, p->size_m, p->origin_x,
-                                   p->origin_y, d_ev, cap, d_n);
+  int8_t* d_grid = (int8_t*)g_ctx.out_grids.p;
+  float* d_origin = (float*)(d_grid + ((cells + 3) & ~(size_t)3));
+  int32_t* d_n = (int32_t*)(d_origin + 2);
+  uqs_stats local;
+  if ((rc = uqs_replay_recentering_dev(p, 1, n_frames, (float*)g_ctx.in_x.p, (float*)g_ctx.in_y.p, (float*)g_ctx.in_yaw.p,
+                                       (float*)g_ctx.in_ranges.p, d_grid, d_origin, d_n, cap ? (int32_t*)g_ctx.in_t.p : nullptr,
+                                       cap, stats ? stats : &local)))
+    return rc;
+  float origin[2];
   int n_ev = 0;
-  cudaError_t e = cudaGetLastError();
-  if (e == cudaSuccess) e = cudaMemcpyAsync(&n_ev, d_n, 4, cudaMemcpyDeviceToHost, st);
+  cudaError_t e = cudaMemcpyAsync(grid_out, d_grid, cells, cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(origin, d_origin, sizeof(origin), cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(&n_ev, d_n, sizeof(int), cudaMemcpyDeviceToHost, st);
   if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-  if (e != cudaSuccess) return cuda_fail(e, "k_recenter_plan");
-  if (n_ev > cap) { set_error("%d recenter events exceed the supported %d", n_ev, cap); return UQS_ERR_BAD_ARG; }
-  std::vector<RecenterEvent> ev((size_t)n_ev);
-  if (n_ev) {
-    e = cudaMemcpy(ev.data(), d_ev, (size_t)n_ev * sizeof(RecenterEvent), cudaMemcpyDeviceToHost);
-    if (e != cudaSuccess) return cuda_fail(e, "events D2H");
+  if (e == cudaSuccess && cap) {
+    e = cudaMemcpyAsync(events_out, g_ctx.in_t.p, (size_t)std::min(n_ev, cap) * 12, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
   }
-  int8_t* g0 = (int8_t*)g_ctx.out_grids.p;
-  int8_t* g1 = g0 + cells;
-  if ((e = cudaMemsetAsync(g0, 0, cells, st)) != cudaSuccess) return cuda_fail(e, "memset grid");
-  uqs_params q = *p;
-  uqs_stats total = { 0, 0, 0, 0, 0 }, part;
-  int f0 = 0;
-  for (int k = 0; k <= n_ev; k++) {
-    const int f1 = (k < n_ev) ? ev[k].frame : n_frames;
-    if (f1 > f0) {
-      DevParams dq;
-      if ((rc = make_dev_params(&q, &dq))) return rc;
-      if ((rc = replay_device(dq, 1, f1 - f0, (float*)g_ctx.in_x.p + f0, (float*)g_ctx.in_y.p + f0, (float*)g_ctx.in_yaw.p + f0,
-                              (float*)g_ctx.in_ranges.p + (size_t)f0 * 32, nullptr, g0, 1, 0, p->H, true)))
-        return rc;
-      rc = fetch_stats(&part, (uint64_t)(f1 - f0));
-      if (rc) return rc;
-      total.ray_cell_updates += part.ray_cell_updates; total.rays_accepted += part.rays_accepted;
-      total.rays_skipped += part.rays_skipped; total.frames += part.frames;
-    }
-    if (k < n_ev) {
-      k_recenter_shift<<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(g0, g1, p->W, p->H, ev[k].sx, ev[k].sy);
-      if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "k_recenter_shift");
-      std::swap(g0, g1);
-      q.origin_x = ev[k].ox;
-      q.origin_y = ev[k].oy;
-      g_ctx.launches += 1;
-    }
-    f0 = f1;
-  }
-  e = cudaMemcpyAsync(grid_out, g0, cells, cudaMemcpyDeviceToHost, st);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-  if (e != cudaSuccess) return cuda_fail(e, "grid D2H");
-  if (origin_out) { origin_out[0] = q.origin_x; origin_out[1] = q.origin_y; }
+  if (e != cudaSuccess) return cuda_fail(e, "uqs_replay_recentering D2H");
+  if (origin_out) { origin_out[0] = origin[0]; origin_out[1] = origin[1]; }
   if (n_events_out) *n_events_out = n_ev;
-  if (events_out)
-    for (int k = 0; k < n_ev && k < max_events; k++) { events_out[3 * k] = ev[k].frame; events_out[3 * k + 1] = ev[k].sx; events_out[3 * k + 2] = ev[k].sy; }
-  if (stats) *stats = total;
   return UQS_OK;
 }
 
