@@ -307,7 +307,8 @@ typedef struct uqs_query {
  * byte-identical to uqs_replay_dev with the same arguments (row0 = 0, rows = H: whole grids only); n_queries == 0 is
  * exactly uqs_replay_dev (scores_dev and queries_dev may then be NULL).  A query with flight outside [0, n_flights) or
  * frame outside [0, n_frames) returns UQS_ERR_BAD_ARG naming the first such index, before any grid is written (the
- * check synchronises).  Queries use the fixed origin of p (no recentering).  The engine, sub-tile geometry and time
+ * check synchronises).  Queries use the fixed origin of p (no recentering; uqs_replay_recentering_frontier_dev scores
+ * queries against recentred maps).  The engine, sub-tile geometry and time
  * slicing are chosen as for uqs_replay_dev; the resident engine's probe variant uses the default lane layout, so
  * uqs_set_fan_layout() and uqs_set_decode_warp() do not apply to this call.  Asynchronous on the current stream. */
 int uqs_replay_frontier_dev(const uqs_params* p, int n_flights, int n_frames,
@@ -318,6 +319,33 @@ int uqs_replay_frontier_dev(const uqs_params* p, int n_flights, int n_frames,
 int uqs_replay_frontier(const uqs_params* p, int n_flights, int n_frames, const float* x, const float* y,
                         const float* yaw_deg, const float* ranges, int8_t* grids_out,
                         int n_queries, const uqs_query* queries, int32_t* scores_out, uqs_stats* stats);
+
+/* N2 + N3: uqs_replay_recentering_dev plus n_queries frontier queries answered inside the same replay, each against
+ * its flight's recentred map at its frame.  scores_dev[i] is what frontier_score_dir(x, y, yaw_deg, offset_deg) of
+ * queries_dev[i] returns when occ_grid holds flight `flight`'s map after log_tick() of frames 0..frame -- each frame
+ * map_recentre_if_needed(x[f], y[f]) then map_update_from_beams -- and map_origin_x/y is that flight's origin at that
+ * point: a query at a frame with an event sees the shifted window and the new origin, its samples go through
+ * world_to_grid() in window coordinates and the first sample outside the window ends its ray, as in control_tick()
+ * (uav_local_nav.c:1873, 1715-1736, 2225-2253).  Scores come back in input order; any order of queries, duplicates and
+ * many per frame are fine.  Grids, origins, event counts, event lists and stats are byte-identical to
+ * uqs_replay_recentering_dev with the same arguments, and n_queries == 0 is exactly that call (queries_dev and
+ * scores_dev may then be NULL).  A query with flight outside [0, n_flights) or frame outside [0, n_frames) returns
+ * UQS_ERR_BAD_ARG naming the first such index before anything is written (the check synchronises); so do NULL
+ * buffers, bad sizes, engine 2 and more probes than uqs_replay_frontier_dev accepts.  Queries never change the route,
+ * engine or geometry of the call: on the sub-tile route the probes are read in each flight's global frame, an event of
+ * frame e applied before every probe of a frame >= e and a probe of frame p read before every event of a frame > p; on
+ * the segment route each segment's replay serves the queries of its frames.  uqs_set_fan_layout(),
+ * uqs_set_decode_warp() and uqs_set_k0_bias() do not apply.  Asynchronous unless stats is given (the recenter plan and,
+ * on the segment route, the grouping of queries by segment synchronise). */
+int uqs_replay_recentering_frontier_dev(const uqs_params* p, int n_flights, int n_frames,
+                                        const float* x_dev, const float* y_dev, const float* yaw_dev, const float* ranges_dev,
+                                        int8_t* grids_dev, float* origins_dev, int32_t* n_events_dev, int32_t* events_dev,
+                                        int max_events, int n_queries, const uqs_query* queries_dev, int32_t* scores_dev,
+                                        uqs_stats* stats);
+/* Host-buffer form: grids_out [n_flights][H][W] and origins_out [n_flights][2] may be NULL.  Synchronous. */
+int uqs_replay_recentering_frontier(const uqs_params* p, int n_flights, int n_frames, const float* x, const float* y,
+                                    const float* yaw_deg, const float* ranges, int8_t* grids_out, float* origins_out,
+                                    int n_queries, const uqs_query* queries, int32_t* scores_out, uqs_stats* stats);
 
 /* N4: reader of scanlog.bin ("SCLOG2\n" + packed 569-byte scanrec_t records, uav_local_nav.c:1505,1522-1547).
  * Returns the number of qualifying records (> max_records means the buffers were too small), < 0 on error.

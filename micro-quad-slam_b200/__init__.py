@@ -86,6 +86,7 @@ _EXPORTS = [
     "uqs_beam_cells", "uqs_frame_bounds", "uqs_sincosf_batch", "uqs_measure_rmw_peak", "uqs_measure_atoms_peak",
     "uqs_beams_from_scans", "uqs_beams_from_scans_dev", "uqs_replay_recentering", "uqs_frontier_scores",
     "uqs_replay_frontier", "uqs_replay_frontier_dev", "uqs_replay_recentering_dev",
+    "uqs_replay_recentering_frontier", "uqs_replay_recentering_frontier_dev",
     "uqs_scanlog_read", "uqs_scanlog_count", "uqs_navlog_read", "map_recenter_shift", "map_recentre_if_needed", "frontier_score_dir",
     # multi-GPU
     "uqs_flight_shard", "uqs_row_band", "uqs_comm_unique_id", "uqs_comm_init_rank", "uqs_comm_destroy", "uqs_comm_nranks",
@@ -142,6 +143,8 @@ def lib() -> C.CDLL:
     L.uqs_frontier_scores.argtypes = [C.POINTER(Params), vp, ip, vp, vp, vp, vp, vp]
     L.uqs_replay_frontier.argtypes = [C.POINTER(Params), ip, ip, vp, vp, vp, vp, vp, ip, vp, vp, C.POINTER(Stats)]
     L.uqs_replay_frontier_dev.argtypes = [C.POINTER(Params), ip, ip, vp, vp, vp, vp, vp, ip, ip, vp, vp, C.POINTER(Stats)]
+    L.uqs_replay_recentering_frontier_dev.argtypes = [C.POINTER(Params), ip, ip] + [vp] * 8 + [ip, ip, vp, vp, C.POINTER(Stats)]
+    L.uqs_replay_recentering_frontier.argtypes = [C.POINTER(Params), ip, ip] + [vp] * 6 + [ip, vp, vp, C.POINTER(Stats)]
     L.uqs_scanlog_read.restype = C.c_long
     L.uqs_scanlog_read.argtypes = [C.c_char_p, ip, C.c_long] + [vp] * 11
     L.uqs_scanlog_count.restype = C.c_long
@@ -541,6 +544,45 @@ def replay_frontier_dev(p: Params, n_flights: int, n_frames: int, x_ptr: int, y_
                                          C.c_void_p(yaw_ptr), C.c_void_p(ranges_ptr), C.c_void_p(grids_ptr),
                                          1 if accumulate else 0, int(n_queries), C.c_void_p(queries_ptr),
                                          C.c_void_p(scores_ptr), C.byref(st) if want_stats else None))
+    return st.as_dict() if want_stats else None
+
+
+def replay_recentering_frontier(p: Params, x, y, yaw_deg, ranges, queries, want_grids: bool = True):
+    """``uqs_replay_recentering_frontier``: the replay of ``replay_recentering_flights`` plus frontier_score_dir for every
+    query against its flight's recentred map at its frame, in the window of the origin the flight had then.  Returns
+    (grids [F,H,W] int8 or None, origins [F,2] float32 or None, scores [n] int32, stats dict)."""
+    x = _f32(x)
+    if x.ndim == 1:
+        x = x[None]
+    F, N = x.shape
+    y, yaw_deg = _f32(y).reshape(F, N), _f32(yaw_deg).reshape(F, N)
+    ranges = _f32(ranges).reshape(F, N, BEAMS_PER_FRAME)
+    q = np.ascontiguousarray(queries, QUERY_DTYPE)
+    grids = np.empty((F, p.H, p.W), np.int8) if want_grids else None
+    origins = np.empty((F, 2), np.float32) if want_grids else None
+    scores = np.empty(q.size, np.int32)
+    st = Stats()
+    _check(lib().uqs_replay_recentering_frontier(C.byref(p), F, N, _ptr(x), _ptr(y), _ptr(yaw_deg), _ptr(ranges),
+                                                 _ptr(grids) if grids is not None else None,
+                                                 _ptr(origins) if origins is not None else None, q.size,
+                                                 _ptr(q) if q.size else None, _ptr(scores) if q.size else None, C.byref(st)))
+    return grids, origins, scores, st.as_dict()
+
+
+def replay_recentering_frontier_dev(p: Params, n_flights: int, n_frames: int, x_ptr: int, y_ptr: int, yaw_ptr: int,
+                                    ranges_ptr: int, grids_ptr: int, origins_ptr: int, n_events_ptr: int, events_ptr: int,
+                                    max_events: int, n_queries: int, queries_ptr: int, scores_ptr: int,
+                                    want_stats: bool = False):
+    """``uqs_replay_recentering_frontier_dev`` on raw device pointers: the buffers of ``replay_recentering_dev`` plus
+    queries (``QUERY_DTYPE`` records) and scores (int32); asynchronous unless stats are asked."""
+    st = Stats()
+    _check(lib().uqs_replay_recentering_frontier_dev(C.byref(p), n_flights, n_frames, C.c_void_p(x_ptr), C.c_void_p(y_ptr),
+                                                     C.c_void_p(yaw_ptr), C.c_void_p(ranges_ptr), C.c_void_p(grids_ptr),
+                                                     C.c_void_p(origins_ptr), C.c_void_p(n_events_ptr),
+                                                     C.c_void_p(events_ptr) if events_ptr else None, int(max_events),
+                                                     int(n_queries), C.c_void_p(queries_ptr) if queries_ptr else None,
+                                                     C.c_void_p(scores_ptr) if scores_ptr else None,
+                                                     C.byref(st) if want_stats else None))
     return st.as_dict() if want_stats else None
 
 

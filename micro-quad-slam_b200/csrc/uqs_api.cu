@@ -480,10 +480,11 @@ int replay_device(const DevParams& dp, int n_flights, int n_frames, const float*
 
 // Recentred flights through the sub-tile engine (uqs_replay_recentering_dev, route A): the ray set-up places every
 // frame's records in its flight's global frame, and the sub-tiles cover the largest global extent gw x gh of the call.
-// Grids start at zero; stats are reset.  The caller has checked that the inputs suit the sub-tile engine.
+// Grids start at zero; stats are reset.  The caller has checked that the inputs suit the sub-tile engine.  probes: cells
+// in each flight's global frame (gw wide), served by the (flight, sub-tile) that owns them.
 int replay_device_recentering(const DevParams& dp, int n_flights, int n_frames, const float* x, const float* y,
                               const float* yaw, const float* ranges, int8_t* grids, const PlanEvent* events,
-                              const int* ev_start, const int2* s_min, int gw, int gh) {
+                              const int* ev_start, const int2* s_min, int gw, int gh, const ProbeSet* probes) {
   cudaStream_t st = g_ctx.stream();
   const int gpf = (n_frames + 31) / 32;
   g_ctx.w->boxes_valid = false;
@@ -511,7 +512,7 @@ int replay_device_recentering(const DevParams& dp, int n_flights, int n_frames, 
   if (e == cudaSuccess) e = zero_counted(grids, (size_t)n_flights * dp.W * dp.H, st);   // cells no sub-tile writes read 0
   if (e != cudaSuccess) return cuda_fail(e, "memset before the recentering replay");
   int ctas_per_sm = 0;
-  if ((e = tiles_recenter_prepare(smem, &ctas_per_sm)) != cudaSuccess) return cuda_fail(e, "occupancy(k_replay_tiles)");
+  if ((e = tiles_recenter_prepare(probes != nullptr, smem, &ctas_per_sm)) != cudaSuccess) return cuda_fail(e, "occupancy(k_replay_tiles)");
   if (ctas_per_sm < 1) { set_error("replay kernel does not fit on an SM (smem %zu)", smem); return UQS_ERR_CUDA; }
   for (int f0 = 0; f0 < n_flights; f0 += chunk) {
     const int nf = std::min(chunk, n_flights - f0);
@@ -547,8 +548,10 @@ int replay_device_recentering(const DevParams& dp, int n_flights, int n_frames, 
     if (e != cudaSuccess) return cuda_fail(e, "memset job counter");
     const unsigned long long want = (A.total_jobs + kReplayWarps - 1) / kReplayWarps;
     const unsigned grid = (unsigned)std::min<unsigned long long>(want, (unsigned long long)ctas_per_sm * g_ctx.sm_count);
+    ProbeArgs PA;
+    if (probes && (rc = probe_buckets(*probes, f0, nf, n_frames, gw, 1, gpf, sw, sh, nsx, nsy, &PA))) return rc;
     KernelTimer t_rep(2);
-    e = tiles_recenter_launch(grid, smem, st, A, R);
+    e = tiles_recenter_launch(probes != nullptr, grid, smem, st, A, probes ? PA : ProbeArgs{}, R);
     t_rep.stop();
     if (e != cudaSuccess) return cuda_fail(e, "k_replay_tiles launch");
     g_ctx.launches += 2;

@@ -198,12 +198,13 @@ __device__ __forceinline__ float frontier_ray_angle(const DevParams& p, float ya
 // ... its first sample distance and step (:361-362: d = step, step + step, ... <= 2.5f) ...
 __device__ __forceinline__ float frontier_step(const DevParams& p) { return __fmul_rn(p.res, 2.0f); }
 constexpr float kFrontierRange = 2.5f;
-// ... the cell of the sample at distance d (:373-375; false = off the grid, which ends the ray) ...
-__device__ __forceinline__ bool frontier_point(const DevParams& p, float x, float y, float d, float ca, float sa, int& gx,
-                                               int& gy) {
+// ... the cell of the sample at distance d in the window of map origin (ox, oy) (:373-375; false = off the window, which
+// ends the ray) ...
+__device__ __forceinline__ bool frontier_point(const DevParams& p, float ox, float oy, float x, float y, float d, float ca,
+                                               float sa, int& gx, int& gy) {
   const float px = __fadd_rn(x, __fmul_rn(d, ca));
   const float py = __fadd_rn(y, __fmul_rn(d, sa));
-  return world_to_grid(p, px, py, gx, gy);
+  return world_to_grid_at(p, ox, oy, px, py, gx, gy);
 }
 // ... and the score's weight of the cell's value (:378-383): unknown +3, free +1, occupied -4
 __device__ __forceinline__ int frontier_weight(int v) {

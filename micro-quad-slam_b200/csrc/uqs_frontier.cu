@@ -9,8 +9,12 @@
 //   (replay engines)     each probe's value read by the cell's owner between frame `frame` and the next (PROBE = true)
 //   k_probe_slices       time-sliced sub-tile replays: map words -> values, before k_compose_slices
 //   k_frontier_reduce    one thread per query: unknown*3 + free - occ*4 over its probes
+// Recentred flights (uqs_replay_recentering_frontier_dev, uqs_next.cu): k_frontier_probes<true> samples each query at its
+// flight's origin at the query's frame; k_segment_keys / k_segment_gather group the queries by segment between events
+// for the segment route.
 #include <climits>
 #include <cmath>
+#include <vector>
 
 #include <cub/device/device_radix_sort.cuh>
 
@@ -19,12 +23,36 @@
 namespace uqs {
 
 // One thread per (query, ray): the cell of every sample d = step, 2 step, ... <= 2.5 (binary32 accumulation of d, :371)
-// until the first off-grid point (:375); the ray's remaining slots are empty (-1).
+// until the first off-window point (:375); the ray's remaining slots are empty (-1).  RECENTER: slot j holds query
+// O.order[j] (or j), sampled in the window of its flight's last event at a frame <= its own (world_to_grid at that
+// origin, off-window test included) and, with O.s_min, then moved into the flight's global frame, O.gw wide.
+struct ProbeOrigins {
+  const PlanEvent* events;
+  const int* ev_start;
+  const int2* s_min;
+  const int* order;
+  int gw;
+};
+template <bool RECENTER>
 __global__ void k_frontier_probes(DevParams p, int n_queries, int s_max, const uqs_query* __restrict__ queries,
-                                  int* __restrict__ cells, unsigned long long* __restrict__ domain_errors) {
+                                  int* __restrict__ cells, unsigned long long* __restrict__ domain_errors, ProbeOrigins O) {
   const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= (long long)n_queries * 3) return;
-  const uqs_query q = queries[t / 3];
+  const int j = (int)(t / 3);
+  const uqs_query q = queries[RECENTER && O.order ? O.order[j] : j];
+  float ox = p.ox, oy = p.oy;
+  int offx = 0, offy = 0, width = p.W;
+  if (RECENTER) {
+    const int eb = O.ev_start[q.flight];
+    const int e = last_event_at(O.events, eb, O.ev_start[q.flight + 1], q.frame);
+    if (e >= eb) { ox = O.events[e].ox; oy = O.events[e].oy; }
+    if (O.s_min) {
+      const int2 sm = O.s_min[q.flight];
+      offx = (e >= eb ? O.events[e].Sx : 0) - sm.x;
+      offy = (e >= eb ? O.events[e].Sy : 0) - sm.y;
+      width = O.gw;
+    }
+  }
   int* out = cells + t * s_max;
   int k = 0;
   float sa, ca;
@@ -34,8 +62,8 @@ __global__ void k_frontier_probes(DevParams p, int n_queries, int s_max, const u
     const float step = frontier_step(p);
     for (float d = step; d <= kFrontierRange && k < s_max; d = __fadd_rn(d, step)) {
       int gx, gy;
-      if (!frontier_point(p, q.x, q.y, d, ca, sa, gx, gy)) break;
-      out[k++] = gy * p.W + gx;
+      if (!frontier_point(p, ox, oy, q.x, q.y, d, ca, sa, gx, gy)) break;
+      out[k++] = (gy + offy) * width + gx + offx;
     }
   }
   for (; k < s_max; k++) out[k] = -1;
@@ -112,14 +140,45 @@ __global__ void k_probe_slices(ProbeArgs Q, int n_max, const int8_t* __restrict_
 }
 
 __global__ void k_frontier_reduce(int n_queries, int s_max, const int* __restrict__ cells, const uint32_t* __restrict__ values,
-                                  int32_t* __restrict__ scores) {
+                                  const int* __restrict__ order, int32_t* __restrict__ scores) {
   const int q = blockIdx.x * blockDim.x + threadIdx.x;
   if (q >= n_queries) return;
   const size_t s0 = (size_t)q * 3 * s_max;
   int score = 0;
   for (int k = 0; k < 3 * s_max; k++)
     if (cells[s0 + k] >= 0) score += frontier_weight((int)values[s0 + k]);
-  scores[q] = score;
+  scores[order ? order[q] : q] = score;
+}
+
+// query i -> (segment of its frame, i): segment e + 1 + flight follows the flight's last event e at a frame <= its own
+__global__ void k_segment_keys(int n, const uqs_query* __restrict__ queries, const PlanEvent* __restrict__ events,
+                               const int* __restrict__ ev_start, unsigned long long* __restrict__ keys, int* __restrict__ idx) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uqs_query q = queries[i];
+  const int e = last_event_at(events, ev_start[q.flight], ev_start[q.flight + 1], q.frame);
+  keys[i] = (unsigned long long)(e + 1 + q.flight);
+  idx[i] = i;
+}
+
+// sorted (segment, query) -> the segment-local queries, their input indices and the segment starts
+__global__ void k_segment_gather(int n, const unsigned long long* __restrict__ keys, const int* __restrict__ idx,
+                                 const uqs_query* __restrict__ queries, const PlanEvent* __restrict__ events,
+                                 const int* __restrict__ ev_start, int n_segments, uqs_query* __restrict__ local,
+                                 int* __restrict__ order, int* __restrict__ start) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int seg = (int)keys[i];
+  uqs_query q = queries[idx[i]];
+  const int e = seg - 1 - q.flight;
+  q.frame -= e >= ev_start[q.flight] ? events[e].frame : 0;
+  q.flight = 0;
+  local[i] = q;
+  order[i] = idx[i];
+  const int bp = i ? (int)keys[i - 1] : -1;
+  for (int b = bp + 1; b <= seg; b++) start[b] = i;
+  if (i == n - 1)
+    for (int b = seg + 1; b <= n_segments; b++) start[b] = n;
 }
 
 static unsigned blocks_for(long long n, int threads) { return (unsigned)((n + threads - 1) / threads); }
@@ -189,6 +248,119 @@ static int frontier_samples(float res) {
   return n;
 }
 
+int frontier_queries_begin(const char* who, const uqs_params* p, int n_flights, int n_frames, int n_queries,
+                           const uqs_query* queries, ProbeSet* Q, unsigned long long** dom) {
+  const int s_max = frontier_samples(p->res_m);
+  if (s_max < 0 || (long long)n_queries * 3 * s_max >= INT_MAX) {
+    set_error("%s: %d queries of %d samples per ray exceed the supported probe count", who, n_queries, s_max);
+    return UQS_ERR_BAD_ARG;
+  }
+  cudaStream_t st = g_ctx.stream();
+  int rc;
+  if ((rc = g_ctx.w->counters.ensure(64 * sizeof(unsigned long long)))) return rc;
+  *dom = (unsigned long long*)g_ctx.w->counters.p + 48;
+  int* first_bad = (int*)((unsigned long long*)g_ctx.w->counters.p + 49);
+  // the queries are checked before anything is written
+  int h_bad = INT_MAX;
+  cudaError_t e = cudaMemcpyAsync(first_bad, &h_bad, sizeof(int), cudaMemcpyHostToDevice, st);
+  if (e == cudaSuccess) {
+    k_query_check<<<blocks_for(n_queries, 256), 256, 0, st>>>(n_queries, queries, n_flights, n_frames, first_bad);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) e = cudaMemcpyAsync(&h_bad, first_bad, sizeof(int), cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  if (e != cudaSuccess) return cuda_fail(e, "k_query_check");
+  g_ctx.launches += 1;
+  if (h_bad != INT_MAX) {
+    uqs_query q;
+    e = cudaMemcpy(&q, queries + h_bad, sizeof(q), cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) return cuda_fail(e, "query D2H");
+    set_error("query %d: flight %d outside [0, %d) or frame %d outside [0, %d)", h_bad, q.flight, n_flights, q.frame, n_frames);
+    return UQS_ERR_BAD_ARG;
+  }
+  Q->n_queries = n_queries;
+  Q->s_max = s_max;
+  Q->queries = queries;
+  const size_t slots = Q->slots();
+  if ((rc = g_ctx.w->probe_slots.ensure(slots * 8 + 16))) return rc;
+  int* cells = (int*)g_ctx.w->probe_slots.p;
+  Q->cells = cells;
+  Q->values = (uint32_t*)(cells + slots);
+  if ((e = zero_async(*dom, sizeof(unsigned long long), st)) != cudaSuccess) return cuda_fail(e, "memset");
+  return UQS_OK;
+}
+
+int frontier_probes_recentered(const DevParams& dp, const ProbeSet& Q, const uqs_query* queries, const int* order,
+                               const PlanEvent* events, const int* ev_start, const int2* s_min, int gw,
+                               unsigned long long* dom) {
+  const ProbeOrigins O = { events, ev_start, s_min, order, gw };
+  k_frontier_probes<true><<<blocks_for((long long)Q.n_queries * 3, 128), 128, 0, g_ctx.stream()>>>(
+      dp, Q.n_queries, Q.s_max, queries, Q.cells, dom, O);
+  const cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return cuda_fail(e, "k_frontier_probes");
+  g_ctx.launches += 1;
+  return UQS_OK;
+}
+
+int frontier_queries_by_segment(int n_queries, const uqs_query* queries, const PlanEvent* events, const int* ev_start,
+                                int n_segments, uqs_query* local, int* order, std::vector<int>* seg_start) {
+  cudaStream_t st = g_ctx.stream();
+  Work& w = *g_ctx.w;
+  const int n = n_queries;
+  int end_bit = 1;
+  while (end_bit < 64 && ((unsigned long long)n_segments >> end_bit) != 0) end_bit++;
+  size_t tmp_bytes = 0;
+  unsigned long long *k_in = nullptr, *k_out = nullptr;
+  int *i_in = nullptr, *i_out = nullptr;
+  cudaError_t e = cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, k_in, k_out, i_in, i_out, n, 0, end_bit, st);
+  if (e != cudaSuccess) return cuda_fail(e, "segment sort sizing");
+  int rc;
+  if ((rc = w.probe_keys.ensure((size_t)n * 24)) || (rc = w.probe_tmp.ensure(tmp_bytes)) ||
+      (rc = w.probe_start.ensure(((size_t)n_segments + 1) * sizeof(int))))
+    return rc;
+  k_in = (unsigned long long*)w.probe_keys.p;
+  k_out = k_in + n;
+  i_in = (int*)(k_out + n);
+  i_out = i_in + n;
+  int* d_start = (int*)w.probe_start.p;
+  k_segment_keys<<<blocks_for(n, 256), 256, 0, st>>>(n, queries, events, ev_start, k_in, i_in);
+  e = cudaGetLastError();
+  if (e == cudaSuccess) e = cub::DeviceRadixSort::SortPairs(w.probe_tmp.p, tmp_bytes, k_in, k_out, i_in, i_out, n, 0, end_bit, st);
+  if (e == cudaSuccess) {
+    k_segment_gather<<<blocks_for(n, 256), 256, 0, st>>>(n, k_out, i_out, queries, events, ev_start, n_segments, local, order,
+                                                         d_start);
+    e = cudaGetLastError();
+  }
+  seg_start->resize((size_t)n_segments + 1);
+  if (e == cudaSuccess)
+    e = cudaMemcpyAsync(seg_start->data(), d_start, seg_start->size() * sizeof(int), cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  if (e != cudaSuccess) return cuda_fail(e, "frontier queries by segment");
+  g_ctx.launches += 3;
+  return UQS_OK;
+}
+
+int frontier_queries_end(const ProbeSet& Q, const int* order, int32_t* scores, unsigned long long* dom, uqs_stats* stats,
+                         uint64_t frames) {
+  cudaStream_t st = g_ctx.stream();
+  cudaError_t e = cudaSuccess;
+  if (Q.s_max > 0)
+    k_frontier_reduce<<<blocks_for(Q.n_queries, 128), 128, 0, st>>>(Q.n_queries, Q.s_max, Q.cells, Q.values, order, scores);
+  else e = zero_async(scores, (size_t)Q.n_queries * sizeof(int32_t), st);
+  if (e == cudaSuccess) e = cudaGetLastError();
+  if (e != cudaSuccess) return cuda_fail(e, "k_frontier_reduce");
+  g_ctx.launches += 1;
+  if (!stats) return UQS_OK;
+  int rc;
+  if ((rc = fetch_stats(stats, frames))) return rc;
+  unsigned long long hdom = 0;
+  e = cudaMemcpyAsync(&hdom, dom, sizeof(hdom), cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  if (e != cudaSuccess) return cuda_fail(e, "frontier domain D2H");
+  if (hdom) { set_error("%llu frontier rays outside the restated sincosf domain", hdom); return UQS_ERR_DOMAIN; }
+  return UQS_OK;
+}
+
 }  // namespace uqs
 
 using namespace uqs;
@@ -211,65 +383,22 @@ int uqs_replay_frontier_dev(const uqs_params* p, int n_flights, int n_frames, co
     if ((rc = replay_device(dp, n_flights, n_frames, x, y, yaw, ranges, nullptr, grids, accumulate, 0, p->H, true))) return rc;
     return fetch_stats(stats, (uint64_t)n_flights * n_frames);
   }
-  const int s_max = frontier_samples(p->res_m);
-  if (s_max < 0 || (long long)n_queries * 3 * s_max >= INT_MAX) {
-    set_error("uqs_replay_frontier_dev: %d queries of %d samples per ray exceed the supported probe count", n_queries, s_max);
-    return UQS_ERR_BAD_ARG;
-  }
-  cudaStream_t st = g_ctx.stream();
-  if ((rc = g_ctx.w->counters.ensure(64 * sizeof(unsigned long long)))) return rc;
-  unsigned long long* dom = (unsigned long long*)g_ctx.w->counters.p + 48;
-  int* first_bad = (int*)((unsigned long long*)g_ctx.w->counters.p + 49);
-  // the queries are checked before anything is written
-  int h_bad = INT_MAX;
-  cudaError_t e = cudaMemcpyAsync(first_bad, &h_bad, sizeof(int), cudaMemcpyHostToDevice, st);
-  if (e == cudaSuccess) {
-    k_query_check<<<blocks_for(n_queries, 256), 256, 0, st>>>(n_queries, queries, n_flights, n_frames, first_bad);
-    e = cudaGetLastError();
-  }
-  if (e == cudaSuccess) e = cudaMemcpyAsync(&h_bad, first_bad, sizeof(int), cudaMemcpyDeviceToHost, st);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-  if (e != cudaSuccess) return cuda_fail(e, "k_query_check");
-  g_ctx.launches += 1;
-  if (h_bad != INT_MAX) {
-    uqs_query q;
-    e = cudaMemcpy(&q, queries + h_bad, sizeof(q), cudaMemcpyDeviceToHost);
-    if (e != cudaSuccess) return cuda_fail(e, "query D2H");
-    set_error("query %d: flight %d outside [0, %d) or frame %d outside [0, %d)", h_bad, q.flight, n_flights, q.frame, n_frames);
-    return UQS_ERR_BAD_ARG;
-  }
   ProbeSet Q;
-  Q.n_queries = n_queries;
-  Q.s_max = s_max;
-  Q.queries = queries;
-  const size_t slots = Q.slots();
-  if ((rc = g_ctx.w->probe_slots.ensure(slots * 8 + 16))) return rc;
-  int* cells = (int*)g_ctx.w->probe_slots.p;
-  Q.cells = cells;
-  Q.values = (uint32_t*)(cells + slots);
-  if ((e = zero_async(dom, sizeof(unsigned long long), st)) != cudaSuccess) return cuda_fail(e, "memset");
-  if (s_max > 0) {
-    k_frontier_probes<<<blocks_for((long long)n_queries * 3, 128), 128, 0, st>>>(dp, n_queries, s_max, queries, cells, dom);
-    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "k_frontier_probes");
+  unsigned long long* dom = nullptr;
+  if ((rc = frontier_queries_begin("uqs_replay_frontier_dev", p, n_flights, n_frames, n_queries, queries, &Q, &dom))) return rc;
+  if (Q.s_max > 0) {
+    k_frontier_probes<false><<<blocks_for((long long)n_queries * 3, 128), 128, 0, g_ctx.stream()>>>(dp, n_queries, Q.s_max, queries,
+                                                                                                   Q.cells, dom,
+                                                                                                   ProbeOrigins{});
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "k_frontier_probes");
     g_ctx.launches += 2;
   }
   // (a step longer than 2.5 m samples nothing: every score is 0 and the replay is the plain one)
   if ((rc = replay_device(dp, n_flights, n_frames, x, y, yaw, ranges, nullptr, grids, accumulate, 0, p->H, true,
-                          s_max > 0 ? &Q : nullptr)))
+                          Q.s_max > 0 ? &Q : nullptr)))
     return rc;
-  if (s_max > 0) k_frontier_reduce<<<blocks_for(n_queries, 128), 128, 0, st>>>(n_queries, s_max, cells, Q.values, scores);
-  else e = zero_async(scores, (size_t)n_queries * sizeof(int32_t), st);
-  if (e == cudaSuccess) e = cudaGetLastError();
-  if (e != cudaSuccess) return cuda_fail(e, "k_frontier_reduce");
-  g_ctx.launches += 1;
-  if (!stats) return UQS_OK;
-  if ((rc = fetch_stats(stats, (uint64_t)n_flights * n_frames))) return rc;
-  unsigned long long hdom = 0;
-  e = cudaMemcpyAsync(&hdom, dom, sizeof(hdom), cudaMemcpyDeviceToHost, st);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-  if (e != cudaSuccess) return cuda_fail(e, "frontier domain D2H");
-  if (hdom) { set_error("%llu frontier rays outside the restated sincosf domain", hdom); return UQS_ERR_DOMAIN; }
-  return UQS_OK;
+  return frontier_queries_end(Q, nullptr, scores, dom, stats, (uint64_t)n_flights * n_frames);
 }
 
 int uqs_replay_frontier(const uqs_params* p, int n_flights, int n_frames, const float* x, const float* y, const float* yaw,

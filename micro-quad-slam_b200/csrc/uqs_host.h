@@ -26,6 +26,7 @@ struct DevBuf {
 struct Work {
   DevBuf rays, frames, groups, counters, inc, scan, order, maps, boxes;
   DevBuf probe_slots, probe_keys, probe_sorted, probe_start, probe_tmp;   // frontier probes and buckets (uqs_frontier.cu)
+  DevBuf probe_local;                                                    // queries grouped by recentering segment
   DevBuf plan_info, plan_start, plan_events, plan_tmp;                   // recenter plans (uqs_next.cu)
   int order_nsx = 0, order_nsy = 0;             // geometry the cached tile order was built for
   cudaStream_t stream = nullptr;
@@ -36,7 +37,7 @@ struct Work {
     if (h_dims) cudaFreeHost(h_dims);
     h_dims = nullptr;
     DevBuf* all[] = { &rays, &frames, &groups, &counters, &inc, &scan, &order, &maps, &boxes, &probe_slots, &probe_keys, &probe_sorted,
-                      &probe_start, &probe_tmp, &plan_info, &plan_start, &plan_events, &plan_tmp };
+                      &probe_start, &probe_tmp, &probe_local, &plan_info, &plan_start, &plan_events, &plan_tmp };
     order_nsx = order_nsy = 0;
     for (DevBuf* b : all) b->release();
   }
@@ -108,7 +109,7 @@ int make_dev_params(const uqs_params* p, DevParams* d);
 struct ProbeSet {
   int n_queries = 0, s_max = 0;
   const uqs_query* queries = nullptr;
-  const int* cells = nullptr;
+  int* cells = nullptr;
   uint32_t* values = nullptr;
   size_t slots() const { return (size_t)n_queries * 3 * s_max; }
 };
@@ -128,10 +129,31 @@ int fetch_stats(uqs_stats* stats, uint64_t frames);
 // sub-tile geometry and time slices replay_device chooses for a call
 void tile_geometry(const DevParams& dp, int n_flights, int n_frames, int rows, int* sw, int* sh, int* nsx, int* nsy,
                    int* slices);
-// recentred flights through the sub-tile engine, records in each flight's global frame (gw x gh: the largest extent)
+// recentred flights through the sub-tile engine, records in each flight's global frame (gw x gh: the largest extent);
+// probes (or nullptr) with cells in that frame
 int replay_device_recentering(const DevParams& dp, int n_flights, int n_frames, const float* x, const float* y,
                               const float* yaw, const float* ranges, int8_t* grids, const PlanEvent* events,
-                              const int* ev_start, const int2* s_min, int gw, int gh);
+                              const int* ev_start, const int2* s_min, int gw, int gh, const ProbeSet* probes = nullptr);
+// Frontier queries of a call (uqs_frontier.cu).  frontier_queries_begin: UQS_ERR_BAD_ARG naming the first query whose
+// flight or frame is out of range (synchronises; nothing written), the probe-count limit, then the probe slots of
+// every query (Q->s_max == 0: no samples, every score is 0) and a zeroed domain-error counter (*dom).
+int frontier_queries_begin(const char* who, const uqs_params* p, int n_flights, int n_frames, int n_queries,
+                           const uqs_query* queries, ProbeSet* Q, unsigned long long** dom);
+// Probe cells of recentred flights: each query's samples in the window of its flight's last event at a frame <= its
+// own (events, ev_start as in RecenterArgs, whole call), then moved by S - s_min of that event into the flight's
+// global frame (gw wide) when s_min is given.  Slot j of Q holds query order[j] (order == nullptr: query j).
+int frontier_probes_recentered(const DevParams& dp, const ProbeSet& Q, const uqs_query* queries, const int* order,
+                               const PlanEvent* events, const int* ev_start, const int2* s_min, int gw,
+                               unsigned long long* dom);
+// Queries grouped by segment (the frames from one event of a flight, or its start, to the next): segment k + 1 + f
+// follows flight f's event k (k = ev_start[f] - 1: its start).  local[j] = query order[j] with flight 0 and its frame
+// counted from the segment's first frame; (*seg_start)[s] = first j of segment s (n_segments + 1 entries).
+// Synchronises once.
+int frontier_queries_by_segment(int n_queries, const uqs_query* queries, const PlanEvent* events, const int* ev_start,
+                                int n_segments, uqs_query* local, int* order, std::vector<int>* seg_start);
+// scores[order ? order[j] : j] = unknown*3 + free - occ*4 over slot j's probes; then, with stats, the domain check
+int frontier_queries_end(const ProbeSet& Q, const int* order, int32_t* scores, unsigned long long* dom, uqs_stats* stats,
+                         uint64_t frames);
 int ensure_inv_table();
 // uqs_generic.cu: the unrestricted replay and the start-grid range check
 cudaError_t generic_launch(const DevParams& dp, int n_flights, int n_frames, const float* x, const float* y, const float* yaw,

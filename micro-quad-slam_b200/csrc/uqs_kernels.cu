@@ -305,13 +305,9 @@ k_ray_setup(const __grid_constant__ DevParams p, int n_frames, const float* __re
       int offx = 0, offy = 0;
       if (fo < n_frames) {
         const int eb = ev_start[flight];
-        int lo = eb, hi = ev_start[flight + 1];                    // first event of a frame > fo
-        while (lo < hi) {
-          const int mid = (lo + hi) >> 1;
-          if (events[mid].frame <= fo) lo = mid + 1; else hi = mid;
-        }
+        const int k = last_event_at(events, eb, ev_start[flight + 1], fo);
         int sx = 0, sy = 0;
-        if (lo > eb) { const PlanEvent& e = events[lo - 1]; mx = e.ox; my = e.oy; sx = e.Sx; sy = e.Sy; }
+        if (k >= eb) { const PlanEvent& e = events[k]; mx = e.ox; my = e.oy; sx = e.Sx; sy = e.Sy; }
         const int2 smin = s_min[flight];
         offx = sx - smin.x;
         offy = sy - smin.y;
@@ -736,6 +732,11 @@ extern __shared__ __align__(16) unsigned char uqs_smem[];
 // frames <= f before queueing frame f's rays (after a flush: the queue may hold rays of earlier frames) and the rest
 // at job end.  A sub-tile no ray reached stays 0 and is not written back (the grids were zeroed); the others write
 // their cells inside the final window to the flight's grid.  Value tiles only: no accumulation, no time slices.
+// PROBE and RECENTER (probes in the flight's global frame): before queueing hit frame g, and at job end, the warp takes
+// the probes of frames < g and the events of frames <= g in frame order -- an event of frame e before every probe of a
+// frame >= e, a probe of frame p before every event of a frame > p -- so a probe never reads a cell that left the window
+// and came back before its frame with its old value, and reads a cell that leaves the window after its frame before it
+// is zeroed.
 template <bool PROBE, bool RECENTER = false>
 __global__ void __launch_bounds__(kReplayThreads)
 k_replay_tiles(ReplayArgs A, ProbeArgs Q, RecenterArgs R) {
@@ -886,6 +887,14 @@ k_replay_tiles(ReplayArgs A, ProbeArgs Q, RecenterArgs R) {
         __syncwarp();
       }
     };
+    // PROBE and RECENTER: probes of frames < fmax and events of frames <= fmax (< 0x7fffffff), in frame order
+    auto catch_up = [&](int fmax) {
+      for (;;) {
+        if (next_ef <= fmax && next_ef <= next_pf) advance(next_ef);
+        else if (next_pf < fmax) serve(min(next_ef, fmax));
+        else break;
+      }
+    };
     for (int g0 = g_begin; g0 < g_end; g0 += 32) {
       bool ghit = false;
       if (g0 + lane < g_end) {
@@ -908,8 +917,12 @@ k_replay_tiles(ReplayArgs A, ProbeArgs Q, RecenterArgs R) {
           fmask &= fmask - 1;
           const uint2 rec = rec_next;
           if (fmask) rec_next = __ldg(&rays[(size_t)(f0 + __ffs(fmask) - 1) * 32 + lane]);
-          if (PROBE) serve(f0 + fi);
-          if (RECENTER) advance(f0 + fi);
+          if (PROBE && RECENTER) {
+            catch_up(f0 + fi);
+          } else {
+            if (PROBE) serve(f0 + fi);
+            if (RECENTER) advance(f0 + fi);
+          }
           const int gx0 = (int)(__shfl_sync(0xffffffffu, fr.x, fi) & 0xffffu);
           const int gy0 = (int)(__shfl_sync(0xffffffffu, fr.y, fi) & 0xffffu);
           const int ex = gx0 + sext12(rec.x), ey = gy0 + sext12(rec.x >> 12);
@@ -932,8 +945,12 @@ k_replay_tiles(ReplayArgs A, ProbeArgs Q, RecenterArgs R) {
     }
     while (qn > 0) flush();
     __syncwarp();
-    if (PROBE) serve(0x7fffffff);                       // frames no ray of which reached the sub-tile
-    if (RECENTER) advance(0x7ffffffe);                   // events after the last frame that reached the sub-tile
+    if (PROBE && RECENTER) {
+      catch_up(0x7ffffffe);
+    } else {
+      if (PROBE) serve(0x7fffffff);                     // frames no ray of which reached the sub-tile
+      if (RECENTER) advance(0x7ffffffe);                 // events after the last frame that reached the sub-tile
+    }
 
     // ---- write the sub-tile back: values into the grid, maps into the slice scratch ---------
     if (RECENTER) {
@@ -1516,14 +1533,17 @@ cudaError_t tiles_launch(bool probe, unsigned grid, size_t smem, cudaStream_t st
   return cudaGetLastError();
 }
 
-cudaError_t tiles_recenter_prepare(size_t smem, int* ctas_per_sm) {
-  cudaError_t e = cudaFuncSetAttribute(k_replay_tiles<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+cudaError_t tiles_recenter_prepare(bool probe, size_t smem, int* ctas_per_sm) {
+  void (*k)(ReplayArgs, ProbeArgs, RecenterArgs) = probe ? k_replay_tiles<true, true> : k_replay_tiles<false, true>;
+  cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
-  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, k_replay_tiles<false, true>, kReplayThreads, smem);
+  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, k, kReplayThreads, smem);
 }
 
-cudaError_t tiles_recenter_launch(unsigned grid, size_t smem, cudaStream_t st, const ReplayArgs& A, const RecenterArgs& R) {
-  k_replay_tiles<false, true><<<grid, kReplayThreads, smem, st>>>(A, ProbeArgs{}, R);
+cudaError_t tiles_recenter_launch(bool probe, unsigned grid, size_t smem, cudaStream_t st, const ReplayArgs& A,
+                                  const ProbeArgs& Q, const RecenterArgs& R) {
+  if (probe) k_replay_tiles<true, true><<<grid, kReplayThreads, smem, st>>>(A, Q, R);
+  else       k_replay_tiles<false, true><<<grid, kReplayThreads, smem, st>>>(A, ProbeArgs{}, R);
   return cudaGetLastError();
 }
 

@@ -66,6 +66,15 @@ struct __align__(16) PlanEvent {
   int Sx, Sy;
   float ox, oy;
 };
+// the index of a flight's last event at a frame <= f among its events [eb, ee) (frame order), eb - 1 when there is none
+__device__ __forceinline__ int last_event_at(const PlanEvent* events, int eb, int ee, int f) {
+  int lo = eb, hi = ee;                                 // first event of a frame > f
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (events[mid].frame <= f) lo = mid + 1; else hi = mid;
+  }
+  return lo - 1;
+}
 struct RecenterArgs {
   const PlanEvent* events;  // every flight's events in frame order
   const int* ev_start;      // [n_flights + 1] (launch-local flights): flight f's events are [ev_start[f], ev_start[f+1])
@@ -106,9 +115,11 @@ __global__ void k_world_to_grid_one(DevParams p, float wx, float wy, int* out);
 // the sub-tile engine (k_replay_tiles), plain or serving probes
 cudaError_t tiles_prepare(bool probe, size_t smem, int* ctas_per_sm);
 cudaError_t tiles_launch(bool probe, unsigned grid, size_t smem, cudaStream_t st, const ReplayArgs& A, const ProbeArgs& Q);
-// the sub-tile engine replaying recentred flights: tiles cover the flights' global frames (no probes, no time slices)
-cudaError_t tiles_recenter_prepare(size_t smem, int* ctas_per_sm);
-cudaError_t tiles_recenter_launch(unsigned grid, size_t smem, cudaStream_t st, const ReplayArgs& A, const RecenterArgs& R);
+// the sub-tile engine replaying recentred flights: tiles cover the flights' global frames (no time slices), plain or
+// serving probes whose cells are in those global frames
+cudaError_t tiles_recenter_prepare(bool probe, size_t smem, int* ctas_per_sm);
+cudaError_t tiles_recenter_launch(bool probe, unsigned grid, size_t smem, cudaStream_t st, const ReplayArgs& A,
+                                  const ProbeArgs& Q, const RecenterArgs& R);
 __global__ void k_compose_slices(int8_t* grids, const uint32_t* maps, int n_flights, int W, int H, int S, int row0,
                                  int rows);
 cudaError_t flights_probe_prepare(int nw, size_t smem, int* ctas_per_sm);

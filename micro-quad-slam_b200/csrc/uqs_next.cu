@@ -162,7 +162,7 @@ __global__ void k_frontier_scores(DevParams p, const int8_t* __restrict__ grid, 
     if (!sincosf_glibc(frontier_ray_angle(p, yaw_deg[i], offset_deg[i], r), sa, ca)) { atomicAdd(domain_errors, 1ull); continue; }
     for (float d = step; d <= kFrontierRange; d = __fadd_rn(d, step)) {   // :371
       int gx, gy;
-      if (!frontier_point(p, x[i], y[i], d, ca, sa, gx, gy)) break;
+      if (!frontier_point(p, p.ox, p.oy, x[i], y[i], d, ca, sa, gx, gy)) break;
       score += frontier_weight((int)grid[(size_t)gy * p.W + gx]);
     }
   }
@@ -249,23 +249,14 @@ int uqs_frontier_scores(const uqs_params* p, const int8_t* grid /* host, [H][W] 
 /* N2 for many flights.  Route A, the sub-tile engine in each flight's global frame, when the inputs suit it: rays of
  * at most kMaxRayCells cells, 0 inside the clamp range, no time slices for this call, global extents that fit the
  * records' 16-bit cells, engine 0 or 1.  Route B otherwise: per flight, the log between two events through
- * replay_device at that segment's origin, then the shift, with the stats summed on the device. */
-int uqs_replay_recentering_dev(const uqs_params* p, int n_flights, int n_frames, const float* x, const float* y,
-                               const float* yaw, const float* ranges, int8_t* grids, float* origins, int32_t* n_events,
-                               int32_t* events, int max_events, uqs_stats* stats) {
-  int rc = check_ready();
-  if (rc) return rc;
-  DevParams dp;
-  if ((rc = make_dev_params(p, &dp))) return rc;
-  if (n_flights <= 0 || n_frames <= 0 || !x || !y || !yaw || !ranges || !grids || !origins || !n_events || max_events < 0 ||
-      (max_events > 0 && !events)) {
-    set_error("uqs_replay_recentering_dev: NULL pointer or bad size");
-    return UQS_ERR_BAD_ARG;
-  }
-  if (g_ctx.engine == 2) {
-    set_error("uqs_replay_recentering_dev: engine 2 (resident) has no recentering variant; use 0, 1 or 3");
-    return UQS_ERR_BAD_ARG;
-  }
+ * replay_device at that segment's origin, then the shift, with the stats summed on the device.  Q (or nullptr): frontier
+ * queries whose flights, frames and probe count were checked (frontier_queries_begin), answered at their frame; on
+ * route A their probes are in the flights' global frames, on route B each segment's replay serves its own queries. */
+static int replay_recentering(const uqs_params* p, const DevParams& dp, int n_flights, int n_frames, const float* x,
+                              const float* y, const float* yaw, const float* ranges, int8_t* grids, float* origins,
+                              int32_t* n_events, int32_t* events, int max_events, const ProbeSet* Q, unsigned long long* dom,
+                              int32_t* scores, uqs_stats* stats) {
+  int rc;
   cudaStream_t st = g_ctx.stream();
   Work& W = *g_ctx.w;
   const size_t info_bytes = ((size_t)n_flights * kPlanInfo * sizeof(int) + 15) & ~(size_t)15;
@@ -313,9 +304,13 @@ int uqs_replay_recentering_dev(const uqs_params* p, int n_flights, int n_frames,
   const long long gw = span_x + dp.W, gh = span_y + dp.H;
   const bool route_a = !long_rays && dp.lo_min <= 0 && dp.lo_max >= 0 && slices == 1 && gw <= 0x7fff && gh <= 0x7fff &&
                        (g_ctx.engine == 0 || g_ctx.engine == 1);
+  const bool probes = Q && Q->s_max > 0;             // (a step longer than 2.5 m samples nothing: every score is 0)
+  const int* order = nullptr;                        // route B: slot j of the probes holds query order[j]
   if (route_a) {
+    if (probes && (rc = frontier_probes_recentered(dp, *Q, Q->queries, nullptr, d_ev, d_start, d_smin, (int)gw, dom)))
+      return rc;
     if ((rc = replay_device_recentering(dp, n_flights, n_frames, x, y, yaw, ranges, grids, d_ev, d_start, d_smin, (int)gw,
-                                        (int)gh)))
+                                        (int)gh, probes ? Q : nullptr)))
       return rc;
   } else {
     std::vector<PlanEvent> ev((size_t)total);
@@ -323,6 +318,20 @@ int uqs_replay_recentering_dev(const uqs_params* p, int n_flights, int n_frames,
       e = cudaMemcpyAsync(ev.data(), d_ev, (size_t)total * sizeof(PlanEvent), cudaMemcpyDeviceToHost, st);
       if (e == cudaSuccess) e = cudaStreamSynchronize(st);
       if (e != cudaSuccess) return cuda_fail(e, "events D2H");
+    }
+    // queries grouped by segment, each segment's probes in its window
+    uqs_query* local = nullptr;
+    std::vector<int> seg_start;
+    if (probes) {
+      const long long n_segments = (long long)n_flights + total;
+      if (n_segments >= INT_MAX) { set_error("more than %d recentering segments in one call", INT_MAX - 1); return UQS_ERR_BAD_ARG; }
+      if ((rc = W.probe_local.ensure((size_t)Q->n_queries * (sizeof(uqs_query) + sizeof(int))))) return rc;
+      local = (uqs_query*)W.probe_local.p;
+      order = (const int*)(local + Q->n_queries);
+      if ((rc = frontier_queries_by_segment(Q->n_queries, Q->queries, d_ev, d_start, (int)n_segments, local, (int*)order,
+                                            &seg_start)) ||
+          (rc = frontier_probes_recentered(dp, *Q, Q->queries, order, d_ev, d_start, nullptr, dp.W, dom)))
+        return rc;
     }
     const size_t cells = (size_t)p->W * p->H;
     if ((rc = W.plan_tmp.ensure(cells)) || (rc = W.counters.ensure(64 * sizeof(unsigned long long)))) return rc;
@@ -341,8 +350,18 @@ int uqs_replay_recentering_dev(const uqs_params* p, int n_flights, int n_frames,
         if (f1 > f0) {
           DevParams dq;
           if ((rc = make_dev_params(&q, &dq))) return rc;
+          ProbeSet S;                                        // the queries of segment k + f
+          if (probes) {
+            const int j0 = seg_start[(size_t)k + f], nq = seg_start[(size_t)k + f + 1] - j0;
+            const size_t s0 = (size_t)j0 * 3 * Q->s_max;
+            S.n_queries = nq;
+            S.s_max = Q->s_max;
+            S.queries = local + j0;
+            S.cells = Q->cells + s0;
+            S.values = Q->values + s0;
+          }
           if ((rc = replay_device(dq, 1, f1 - f0, x + base + f0, y + base + f0, yaw + base + f0, ranges + (base + f0) * 32,
-                                  nullptr, g, 1, 0, p->H, false)))
+                                  nullptr, g, 1, 0, p->H, false, S.n_queries ? &S : nullptr)))
             return rc;
         }
         if (k < start[f + 1]) {
@@ -358,7 +377,58 @@ int uqs_replay_recentering_dev(const uqs_params* p, int n_flights, int n_frames,
       }
     }
   }
+  if (Q) return frontier_queries_end(*Q, order, scores, dom, stats, (uint64_t)n_flights * n_frames);
   return fetch_stats(stats, (uint64_t)n_flights * n_frames);
+}
+
+int uqs_replay_recentering_dev(const uqs_params* p, int n_flights, int n_frames, const float* x, const float* y,
+                               const float* yaw, const float* ranges, int8_t* grids, float* origins, int32_t* n_events,
+                               int32_t* events, int max_events, uqs_stats* stats) {
+  int rc = check_ready();
+  if (rc) return rc;
+  DevParams dp;
+  if ((rc = make_dev_params(p, &dp))) return rc;
+  if (n_flights <= 0 || n_frames <= 0 || !x || !y || !yaw || !ranges || !grids || !origins || !n_events || max_events < 0 ||
+      (max_events > 0 && !events)) {
+    set_error("uqs_replay_recentering_dev: NULL pointer or bad size");
+    return UQS_ERR_BAD_ARG;
+  }
+  if (g_ctx.engine == 2) {
+    set_error("uqs_replay_recentering_dev: engine 2 (resident) has no recentering variant; use 0, 1 or 3");
+    return UQS_ERR_BAD_ARG;
+  }
+  return replay_recentering(p, dp, n_flights, n_frames, x, y, yaw, ranges, grids, origins, n_events, events, max_events,
+                            nullptr, nullptr, nullptr, stats);
+}
+
+/* N2 + N3: uqs_replay_recentering_dev plus frontier queries, each answered against its flight's recentred map at its
+ * frame (after that frame's recentering and update), in the window of the origin the flight had then. */
+int uqs_replay_recentering_frontier_dev(const uqs_params* p, int n_flights, int n_frames, const float* x, const float* y,
+                                        const float* yaw, const float* ranges, int8_t* grids, float* origins,
+                                        int32_t* n_events, int32_t* events, int max_events, int n_queries,
+                                        const uqs_query* queries, int32_t* scores, uqs_stats* stats) {
+  if (n_queries == 0)
+    return uqs_replay_recentering_dev(p, n_flights, n_frames, x, y, yaw, ranges, grids, origins, n_events, events, max_events,
+                                      stats);
+  int rc = check_ready();
+  if (rc) return rc;
+  DevParams dp;
+  if ((rc = make_dev_params(p, &dp))) return rc;
+  if (n_flights <= 0 || n_frames <= 0 || !x || !y || !yaw || !ranges || !grids || !origins || !n_events || max_events < 0 ||
+      (max_events > 0 && !events) || n_queries < 0 || !queries || !scores) {
+    set_error("uqs_replay_recentering_frontier_dev: NULL pointer or bad size");
+    return UQS_ERR_BAD_ARG;
+  }
+  if (g_ctx.engine == 2) {
+    set_error("uqs_replay_recentering_frontier_dev: engine 2 (resident) has no recentering variant; use 0, 1 or 3");
+    return UQS_ERR_BAD_ARG;
+  }
+  ProbeSet Q;
+  unsigned long long* dom = nullptr;
+  if ((rc = frontier_queries_begin("uqs_replay_recentering_frontier_dev", p, n_flights, n_frames, n_queries, queries, &Q, &dom)))
+    return rc;
+  return replay_recentering(p, dp, n_flights, n_frames, x, y, yaw, ranges, grids, origins, n_events, events, max_events, &Q,
+                            dom, scores, stats);
 }
 
 /* N2, one log from host buffers: uqs_replay_recentering_dev with one flight. */
@@ -398,6 +468,42 @@ int uqs_replay_recentering(const uqs_params* p, int n_frames, const float* x, co
   if (e != cudaSuccess) return cuda_fail(e, "uqs_replay_recentering D2H");
   if (origin_out) { origin_out[0] = origin[0]; origin_out[1] = origin[1]; }
   if (n_events_out) *n_events_out = n_ev;
+  return UQS_OK;
+}
+
+/* N2 + N3 from host buffers: uqs_replay_recentering_frontier_dev staged through the library's buffers. */
+int uqs_replay_recentering_frontier(const uqs_params* p, int n_flights, int n_frames, const float* x, const float* y,
+                                    const float* yaw_deg, const float* ranges, int8_t* grids_out, float* origins_out,
+                                    int n_queries, const uqs_query* queries, int32_t* scores_out, uqs_stats* stats) {
+  int rc = check_ready();
+  if (rc) return rc;
+  if (!p || n_flights <= 0 || n_frames <= 0 || !x || !y || !yaw_deg || !ranges || n_queries < 0 ||
+      (n_queries > 0 && (!queries || !scores_out))) {
+    set_error("uqs_replay_recentering_frontier: NULL pointer or bad size");
+    return UQS_ERR_BAD_ARG;
+  }
+  cudaStream_t st = g_ctx.stream();
+  const size_t n = (size_t)n_flights * n_frames, cells = (size_t)n_flights * p->W * p->H;
+  const size_t origins_at = (cells + 15) & ~(size_t)15, n_ev_at = origins_at + (size_t)n_flights * 8;
+  if ((rc = stage(g_ctx.in_x, x, n * 4)) || (rc = stage(g_ctx.in_y, y, n * 4)) || (rc = stage(g_ctx.in_yaw, yaw_deg, n * 4)) ||
+      (rc = stage(g_ctx.in_ranges, ranges, n * 128)) || (rc = g_ctx.out_grids.ensure(n_ev_at + (size_t)n_flights * 4)) ||
+      (n_queries && ((rc = stage(g_ctx.in_kind, queries, (size_t)n_queries * sizeof(uqs_query))) ||
+                     (rc = g_ctx.in_t.ensure((size_t)n_queries * 4)))))
+    return rc;
+  char* out = (char*)g_ctx.out_grids.p;
+  uqs_stats local;
+  if ((rc = uqs_replay_recentering_frontier_dev(p, n_flights, n_frames, (float*)g_ctx.in_x.p, (float*)g_ctx.in_y.p,
+                                                (float*)g_ctx.in_yaw.p, (float*)g_ctx.in_ranges.p, (int8_t*)out,
+                                                (float*)(out + origins_at), (int32_t*)(out + n_ev_at), nullptr, 0, n_queries,
+                                                n_queries ? (const uqs_query*)g_ctx.in_kind.p : nullptr,
+                                                n_queries ? (int32_t*)g_ctx.in_t.p : nullptr, stats ? stats : &local)))
+    return rc;
+  cudaError_t e = cudaSuccess;
+  if (grids_out) e = cudaMemcpyAsync(grids_out, out, cells, cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess && origins_out) e = cudaMemcpyAsync(origins_out, out + origins_at, (size_t)n_flights * 8, cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess && n_queries) e = cudaMemcpyAsync(scores_out, g_ctx.in_t.p, (size_t)n_queries * 4, cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  if (e != cudaSuccess) return cuda_fail(e, "uqs_replay_recentering_frontier D2H");
   return UQS_OK;
 }
 
