@@ -148,6 +148,14 @@ int  uqs_set_k0_bias(int steps);
 /* Experiment knob for the layouts above: row pitch of the resident box in 32-bit words, modulo 32
  * (-1 = the built-in odd pitch).  Identical bytes for any value. */
 int  uqs_set_resident_pitch_mod(int words_mod32);
+/* Schedule of device-pointer replays that take the resident engine without frontier queries: n > 0 = flights go in
+ * chunks of n waves of resident CTAs (the first chunk one wave), and the ray set-up of each chunk runs on the SMs
+ * beside the previous chunk's replay; 0 = the ray set-up of all flights, then their replay.  -1 = the built-in
+ * choice.  Calls whose replay leaves no room for a set-up block on an SM take the second schedule.  Identical bytes
+ * either way; per-kernel times (uqs_profile_collect) overlap under the first. */
+int  uqs_set_setup_overlap(int waves);
+/* Chunks of the last device-pointer replay whose ray set-up ran beside a replay (0: the serial schedule). */
+int  uqs_setup_overlap_chunks(void);
 
 /*
  * P0 -- dead-reckoning pose integration (BUILDER-DEFINED: the reference has no

@@ -80,7 +80,7 @@ _lib = None
 _EXPORTS = [
     # batch API
     "uqs_params_default", "uqs_init", "uqs_shutdown", "uqs_last_error", "uqs_device_sm_count",
-    "uqs_set_stream", "uqs_use_own_stream", "uqs_sync", "uqs_set_tuning", "uqs_set_engine", "uqs_set_fan_layout", "uqs_set_decode_warp", "uqs_set_k0_bias", "uqs_set_resident_pitch_mod", "uqs_kernel_launches",
+    "uqs_set_stream", "uqs_use_own_stream", "uqs_sync", "uqs_set_tuning", "uqs_set_engine", "uqs_set_fan_layout", "uqs_set_decode_warp", "uqs_set_k0_bias", "uqs_set_resident_pitch_mod", "uqs_set_setup_overlap", "uqs_setup_overlap_chunks", "uqs_kernel_launches",
     "uqs_set_profiling", "uqs_profile_collect", "uqs_profile_timeline", "uqs_set_host_chunk",
     "uqs_pose_integrate", "uqs_pose_integrate_dev", "uqs_replay", "uqs_replay_dev", "uqs_replay_flow",
     "uqs_beam_cells", "uqs_frame_bounds", "uqs_sincosf_batch", "uqs_measure_rmw_peak", "uqs_measure_atoms_peak",
@@ -123,6 +123,7 @@ def lib() -> C.CDLL:
     L.uqs_set_resident_pitch_mod.argtypes = [ip]
     L.uqs_set_decode_warp.argtypes = [ip]
     L.uqs_set_k0_bias.argtypes = [ip]
+    L.uqs_set_setup_overlap.argtypes = [ip]
     L.uqs_set_profiling.argtypes = [ip]
     L.uqs_profile_collect.argtypes = [C.POINTER(C.c_double), C.POINTER(C.c_int)]
     L.uqs_profile_timeline.argtypes = [C.POINTER(C.c_double), ip]
@@ -243,6 +244,17 @@ def set_k0_bias(steps: int = 0):
 
 def set_resident_pitch_mod(words_mod32: int = -1):
     _check(lib().uqs_set_resident_pitch_mod(int(words_mod32)))
+
+
+def set_setup_overlap(waves: int = -1):
+    """Resident device replays: n > 0 = chunks of n resident waves, each one's ray set-up beside the previous chunk's
+    replay; 0 = set-up of all flights, then their replay; -1 = default (identical results)."""
+    _check(lib().uqs_set_setup_overlap(int(waves)))
+
+
+def setup_overlap_chunks() -> int:
+    """Chunks of the last device replay whose ray set-up ran beside a replay (0: the serial schedule)."""
+    return int(lib().uqs_setup_overlap_chunks())
 
 
 def set_host_chunk(flights: int = 0):

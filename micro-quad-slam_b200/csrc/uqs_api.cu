@@ -287,134 +287,155 @@ int replay_device(const DevParams& dp, int n_flights, int n_frames, const float*
   if ((rc = g_ctx.w->frames.ensure((size_t)chunk * n_frames * sizeof(uint4)))) return rc;
   if ((rc = g_ctx.w->groups.ensure((size_t)chunk * gpf * sizeof(uint2)))) return rc;
   if ((rc = g_ctx.w->counters.ensure(64 * sizeof(unsigned long long)))) return rc;
-  unsigned long long* counters = (unsigned long long*)g_ctx.w->counters.p;   // [0..3] stats, [8+] job counters
+  unsigned long long* counters = (unsigned long long*)g_ctx.w->counters.p;   // [0..3] stats, [8], [9] job counters
+  uint4* const frames = (uint4*)g_ctx.w->frames.p;
+  uint2* const groups = (uint2*)g_ctx.w->groups.p;
+  uint2* const rays = (uint2*)g_ctx.w->rays.p;
   cudaError_t e;
   if (reset_stats) {
     e = zero_counted(counters, 8 * sizeof(unsigned long long), st);
     if (e != cudaSuccess) return cuda_fail(e, "memset stats");
   }
+  g_ctx.overlap_chunks = 0;
 
   int ctas_per_sm = 0;
   e = tiles_prepare(probes != nullptr, smem, &ctas_per_sm);
   if (e != cudaSuccess) return cuda_fail(e, "occupancy(k_replay_tiles)");
   if (ctas_per_sm < 1) { set_error("replay kernel does not fit on an SM (smem %zu)", smem); return UQS_ERR_CUDA; }
+  if (may_reside && (rc = g_ctx.w->boxes.ensure((size_t)chunk * sizeof(int4)))) return rc;
 
-  for (int f0 = 0; f0 < n_flights; f0 += chunk) {
-    const int nf = std::min(chunk, n_flights - f0);
-    const size_t fo = (size_t)f0 * n_frames;
-    KernelTimer t_setup(1);
-    e = ray_setup_launch(
-        dim3((unsigned)gpf, (unsigned)nf), st, dp, n_frames, x + fo, y + fo, yaw + fo,
-        dp.ranges_u16 ? reinterpret_cast<const float*>(reinterpret_cast<const uint16_t*>(ranges) + fo * 32) : ranges + fo * 32,
-        kind ? kind + fo : nullptr, may_reside ? 1 + g_ctx.k0_bias : 0,
-        (const uint32_t*)g_ctx.inv_table.p, (uint4*)g_ctx.w->frames.p, (uint2*)g_ctx.w->groups.p, (uint2*)g_ctx.w->rays.p, counters);
+  // The records of flight f0 + i of a chunk starting at flight f0 sit at record flight i: frames[i * n_frames ...],
+  // groups[i * gpf ...], rays[i * n_frames * 32 ...], boxes[i].  Each lambda below takes the chunk-relative first
+  // flight `lo` of the n flights it serves and the chunk's first flight f0.
+  auto setup = [&](int f0, int lo, int n, cudaStream_t s, bool small) -> int {
+    const size_t fo = (size_t)(f0 + lo) * n_frames, ro = (size_t)lo * n_frames;
+    const float* r = dp.ranges_u16 ? reinterpret_cast<const float*>(reinterpret_cast<const uint16_t*>(ranges) + fo * 32) : ranges + fo * 32;
+    KernelTimer t_setup(1, s);
+    e = (small ? ray_setup256_launch : ray_setup_launch)(
+        dim3((unsigned)gpf, (unsigned)n), s, dp, n_frames, x + fo, y + fo, yaw + fo, r, kind ? kind + fo : nullptr,
+        may_reside ? 1 + g_ctx.k0_bias : 0, (const uint32_t*)g_ctx.inv_table.p, frames + ro, groups + (size_t)lo * gpf,
+        rays + ro * 32, counters);
     t_setup.stop();
     if (e != cudaSuccess) return cuda_fail(e, "k_ray_setup launch");
+    return UQS_OK;
+  };
 
-    if (may_reside) {
-      // touched bounding box per flight -> shared memory per CTA -> CTAs per SM -> engine choice
-      if ((rc = g_ctx.w->boxes.ensure((size_t)nf * sizeof(int4)))) return rc;
-      int* d_dims = (int*)(counters + 32);
-      if (!g_ctx.w->h_dims) {
-        e = cudaHostAlloc((void**)&g_ctx.w->h_dims, 16, cudaHostAllocMapped);
-        if (e != cudaSuccess) { g_ctx.w->h_dims = nullptr; return cuda_fail(e, "cudaHostAlloc(dims)"); }
-      }
-      int* h_dims_dev = nullptr;
-      e = cudaHostGetDevicePointer((void**)&h_dims_dev, g_ctx.w->h_dims, 0);
-      if (e == cudaSuccess) e = zero_counted(d_dims, 2 * sizeof(int), st);
-      if (e == cudaSuccess)
-        e = flight_boxes_launch(nf, gpf, (const uint2*)g_ctx.w->groups.p, dp.W, dp.H, (int4*)g_ctx.w->boxes.p, d_dims, h_dims_dev, st);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(st);       // the launch geometry of the replay depends on the boxes
-      if (e != cudaSuccess) return cuda_fail(e, "k_flight_boxes");
-      const int dims[2] = { g_ctx.w->h_dims[0], g_ctx.w->h_dims[1] };
-      g_ctx.launches += 2;                                     // boxes, publish
-      g_ctx.w->boxes_valid = nf == n_flights;                  // one internal chunk: the boxes describe the whole call
-      g_ctx.w->boxes_n = nf; g_ctx.w->box_w = dims[0]; g_ctx.w->box_h = dims[1];
-      const int bw = std::max(dims[0], 4), bh = std::max(dims[1], 1);
-      int fpitch = (bw + 3) & ~3;
-      if (((fpitch >> 2) & 1) == 0) fpitch += 4;
-      if (g_ctx.pitch_mod >= 0)                                 // experiment knob: row pitch in words == pitch_mod (mod 32)
-        while (((fpitch >> 2) & 31) != g_ctx.pitch_mod) fpitch += 4;
-      const size_t region = (size_t)fpitch * bh;
-      // Warps per resident CTA.  Measured over box sizes from 17 KB (8 CTAs per SM) to 173 KB (one): the kernel wants
-      // >= 24 resident warps per SM from as few warps per CTA as possible (per-frame work is paid per warp), and never
-      // more than 16 per CTA (a frame has ~80-400 steps to share out).  Few flights: more warps per CTA (nw_min).
-      int ring_size = 256, f_ctas = 0, fnw = nw;
-      size_t fsmem = 0;
-      auto fit = [&](int w, int* ring, size_t* bytes, int* ctas) -> cudaError_t {
-        *ring = 256;                                        // per-warp collision table (power of two)
-        const size_t dec_bytes = (size_t)std::min(w, kDecSlotsMax) * kDecSlotBytes + 16;      // ring of decoded frames (+ alignment)
-        while (*ring > 32 && region + (size_t)(*ring + 4) * w + dec_bytes > kFlightSmemMax) *ring >>= 1;
-        *bytes = region + (size_t)(*ring + 4) * w + dec_bytes;         // + one spare word per warp
-        *ctas = 0;
-        return *bytes <= kFlightSmemMax ? flights_prepare(w, g_ctx.flight_fan, g_ctx.flight_prod, *bytes, ctas) : cudaSuccess;
-      };
-      if (g_ctx.flight_warps) {
-        e = fit(fnw, &ring_size, &fsmem, &f_ctas);
-      } else {
-        e = cudaSuccess;
-        for (int w : { 4, 8, 16 }) {
-          if (w < nw) continue;                             // nw: the minimum the flight count asks for
-          int r, c;
-          size_t bts;
-          if ((e = fit(w, &r, &bts, &c)) != cudaSuccess) break;
-          if (c < 1) break;                                 // more warps only need more shared memory
-          fnw = w; ring_size = r; fsmem = bts; f_ctas = c;
-          if (c * w >= 24) break;
-        }
-      }
-      if (e != cudaSuccess) return cuda_fail(e, "k_replay_flights attributes");
-      if (g_ctx.engine == 2 && f_ctas < 1) {
-        set_error("engine 2: the touched region %dx%d of a flight does not fit %zu B of shared memory", bw, bh, kFlightSmemMax);
-        return UQS_ERR_BAD_ARG;
-      }
-      // auto: resident when the box fits and there are at least SMs/4 flights (measured crossover; with one CTA of
-      // 16 warps per SM it still beats the sub-tile engine by 1.6x on the 668^2 and 800^2 grids of config 5);
-      // otherwise the sub-tile engine (time-sliced when flights are few)
-      // (a chunk of the host-buffer pipeline shares the chip with its neighbours: no flight-count condition there)
-      // (round 2, tools/c5_shard_engines.py: with 128 flights -- a 1/8 shard of a config-5 resolution -- the resident engine
-      // at 16 warps per CTA needs 1.8-2.8 ms against 3.3-6.9 ms for time-sliced sub-tiles on every geometry that fits; one
-      // resident flight takes ~2 ms whatever the count, the sub-tile engine ~0.9 ms + 0.04 ms per flight: crossover ~30)
-      const bool pipelined = g_ctx.chip_shared;               // other chunks of a host-buffer call share the chip
-      const bool resident = f_ctas >= 1 && (g_ctx.engine == 2 || nf * 4 >= g_ctx.sm_count || pipelined);
-      if (resident) {
-        FlightArgs FA;
-        FA.frames = (const uint4*)g_ctx.w->frames.p;
-        FA.rays = (const uint2*)g_ctx.w->rays.p;
-        FA.boxes = (const int4*)g_ctx.w->boxes.p;
-        FA.grids = grids + (size_t)f0 * dp.W * dp.H;
-        FA.job_counter = counters + 8;
-        FA.n_flights = nf; FA.n_frames = n_frames;
-        FA.W = dp.W; FA.H = dp.H; FA.pitch = fpitch; FA.max_rows = bh; FA.ring_size = ring_size;
-        FA.lo_free = dp.lo_free; FA.lo_occ = dp.lo_occ; FA.lo_min = dp.lo_min; FA.lo_max = dp.lo_max;
-        FA.end_nohit = dp.end_nohit;
-        FA.accumulate = accumulate;
-        e = zero_counted(FA.job_counter, sizeof(unsigned long long), st);
-        // cells outside a flight's box are never touched: they are zero in a fresh replay
-        if (e == cudaSuccess && !accumulate) e = zero_counted(FA.grids, (size_t)nf * dp.W * dp.H, st);
-        if (e != cudaSuccess) return cuda_fail(e, "memset before k_replay_flights");
-        if (probes) {
-          int p_ctas = 0;
-          ProbeArgs PA;
-          if ((rc = probe_buckets(*probes, f0, nf, n_frames, dp.W, 0, 0, 0, 0, 0, 0, &PA))) return rc;
-          if ((e = flights_probe_prepare(fnw, fsmem, &p_ctas)) != cudaSuccess) return cuda_fail(e, "k_replay_flights (probes) attributes");
-          if (p_ctas < 1) { set_error("resident engine (probes): %zu B of shared memory do not fit an SM", fsmem); return UQS_ERR_CUDA; }
-          KernelTimer t_rep(2);
-          e = flights_probe_launch(fnw, (unsigned)std::min<long long>(nf, (long long)p_ctas * g_ctx.sm_count), fsmem, st, FA, PA);
-          t_rep.stop();
-          if (e != cudaSuccess) return cuda_fail(e, "k_replay_flights (probes) launch");
-          g_ctx.launches += 2;
-          continue;
-        }
-        const unsigned fgrid = (unsigned)std::min<long long>(nf, (long long)f_ctas * g_ctx.sm_count);
-        KernelTimer t_rep(2);
-        e = flights_launch(fnw, g_ctx.flight_fan, g_ctx.flight_prod, fgrid, fsmem, st, FA);
-        t_rep.stop();
-        if (e != cudaSuccess) return cuda_fail(e, "k_replay_flights launch");
-        g_ctx.launches += 2;
-        continue;
+  // touched bounding box per flight -> shared memory per CTA -> CTAs per SM -> engine choice (after the set-up of
+  // flights [lo, lo + n), which ran on s: synchronises s, the launch geometry of the replay depends on the boxes)
+  struct Resident {
+    int fnw = 0, ring_size = 256, f_ctas = 0, fpitch = 0, bh = 0;
+    size_t fsmem = 0;
+    bool resident = false;
+  };
+  auto configure = [&](int lo, int n, cudaStream_t s, Resident* R) -> int {
+    int* d_dims = (int*)(counters + 32);
+    if (!g_ctx.w->h_dims) {
+      e = cudaHostAlloc((void**)&g_ctx.w->h_dims, 16, cudaHostAllocMapped);
+      if (e != cudaSuccess) { g_ctx.w->h_dims = nullptr; return cuda_fail(e, "cudaHostAlloc(dims)"); }
+    }
+    int* h_dims_dev = nullptr;
+    e = cudaHostGetDevicePointer((void**)&h_dims_dev, g_ctx.w->h_dims, 0);
+    if (e == cudaSuccess) e = zero_counted(d_dims, 2 * sizeof(int), s);
+    if (e == cudaSuccess)
+      e = flight_boxes_launch(n, gpf, groups + (size_t)lo * gpf, dp.W, dp.H, (int4*)g_ctx.w->boxes.p + lo, d_dims, h_dims_dev, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    if (e != cudaSuccess) return cuda_fail(e, "k_flight_boxes");
+    const int dims[2] = { g_ctx.w->h_dims[0], g_ctx.w->h_dims[1] };
+    g_ctx.launches += 2;                                     // boxes, publish
+    g_ctx.w->boxes_valid = n == n_flights;                   // one internal chunk: the boxes describe the whole call
+    g_ctx.w->boxes_n = n; g_ctx.w->box_w = dims[0]; g_ctx.w->box_h = dims[1];
+    const int bw = std::max(dims[0], 4), bh = std::max(dims[1], 1);
+    int fpitch = (bw + 3) & ~3;
+    if (((fpitch >> 2) & 1) == 0) fpitch += 4;
+    if (g_ctx.pitch_mod >= 0)                                 // experiment knob: row pitch in words == pitch_mod (mod 32)
+      while (((fpitch >> 2) & 31) != g_ctx.pitch_mod) fpitch += 4;
+    const size_t region = (size_t)fpitch * bh;
+    // Warps per resident CTA.  Measured over box sizes from 17 KB (8 CTAs per SM) to 173 KB (one): the kernel wants
+    // >= 24 resident warps per SM from as few warps per CTA as possible (per-frame work is paid per warp), and never
+    // more than 16 per CTA (a frame has ~80-400 steps to share out).  Few flights: more warps per CTA (nw_min).
+    int ring_size = 256, f_ctas = 0, fnw = nw;
+    size_t fsmem = 0;
+    auto fit = [&](int w, int* ring, size_t* bytes, int* ctas) -> cudaError_t {
+      *ring = 256;                                        // per-warp collision table (power of two)
+      const size_t dec_bytes = (size_t)std::min(w, kDecSlotsMax) * kDecSlotBytes + 16;      // ring of decoded frames (+ alignment)
+      while (*ring > 32 && region + (size_t)(*ring + 4) * w + dec_bytes > kFlightSmemMax) *ring >>= 1;
+      *bytes = region + (size_t)(*ring + 4) * w + dec_bytes;         // + one spare word per warp
+      *ctas = 0;
+      return *bytes <= kFlightSmemMax ? flights_prepare(w, g_ctx.flight_fan, g_ctx.flight_prod, *bytes, ctas) : cudaSuccess;
+    };
+    if (g_ctx.flight_warps) {
+      e = fit(fnw, &ring_size, &fsmem, &f_ctas);
+    } else {
+      e = cudaSuccess;
+      for (int w : { 4, 8, 16 }) {
+        if (w < nw) continue;                             // nw: the minimum the flight count asks for
+        int r, c;
+        size_t bts;
+        if ((e = fit(w, &r, &bts, &c)) != cudaSuccess) break;
+        if (c < 1) break;                                 // more warps only need more shared memory
+        fnw = w; ring_size = r; fsmem = bts; f_ctas = c;
+        if (c * w >= 24) break;
       }
     }
+    if (e != cudaSuccess) return cuda_fail(e, "k_replay_flights attributes");
+    if (g_ctx.engine == 2 && f_ctas < 1) {
+      set_error("engine 2: the touched region %dx%d of a flight does not fit %zu B of shared memory", bw, bh, kFlightSmemMax);
+      return UQS_ERR_BAD_ARG;
+    }
+    // auto: resident when the box fits and there are at least SMs/4 flights (measured crossover; with one CTA of
+    // 16 warps per SM it still beats the sub-tile engine by 1.6x on the 668^2 and 800^2 grids of config 5);
+    // otherwise the sub-tile engine (time-sliced when flights are few)
+    // (a chunk of the host-buffer pipeline shares the chip with its neighbours: no flight-count condition there)
+    // (round 2, tools/c5_shard_engines.py: with 128 flights -- a 1/8 shard of a config-5 resolution -- the resident engine
+    // at 16 warps per CTA needs 1.8-2.8 ms against 3.3-6.9 ms for time-sliced sub-tiles on every geometry that fits; one
+    // resident flight takes ~2 ms whatever the count, the sub-tile engine ~0.9 ms + 0.04 ms per flight: crossover ~30)
+    const bool pipelined = g_ctx.chip_shared;               // other chunks of a host-buffer call share the chip
+    R->resident = f_ctas >= 1 && (g_ctx.engine == 2 || n * 4 >= g_ctx.sm_count || pipelined);
+    R->fnw = fnw; R->ring_size = ring_size; R->f_ctas = f_ctas; R->fpitch = fpitch; R->bh = bh; R->fsmem = fsmem;
+    return UQS_OK;
+  };
+
+  // the resident replay of flights [lo, lo + n) on stream s with job counter jc
+  auto replay_resident = [&](const Resident& R, int f0, int lo, int n, cudaStream_t s, unsigned long long* jc) -> int {
+    FlightArgs FA;
+    FA.frames = frames + (size_t)lo * n_frames;
+    FA.rays = rays + (size_t)lo * n_frames * 32;
+    FA.boxes = (const int4*)g_ctx.w->boxes.p + lo;
+    FA.grids = grids + (size_t)(f0 + lo) * dp.W * dp.H;
+    FA.job_counter = jc;
+    FA.n_flights = n; FA.n_frames = n_frames;
+    FA.W = dp.W; FA.H = dp.H; FA.pitch = R.fpitch; FA.max_rows = R.bh; FA.ring_size = R.ring_size;
+    FA.lo_free = dp.lo_free; FA.lo_occ = dp.lo_occ; FA.lo_min = dp.lo_min; FA.lo_max = dp.lo_max;
+    FA.end_nohit = dp.end_nohit;
+    FA.accumulate = accumulate;
+    e = zero_counted(FA.job_counter, sizeof(unsigned long long), s);
+    // cells outside a flight's box are never touched: they are zero in a fresh replay
+    if (e == cudaSuccess && !accumulate) e = zero_counted(FA.grids, (size_t)n * dp.W * dp.H, s);
+    if (e != cudaSuccess) return cuda_fail(e, "memset before k_replay_flights");
+    if (probes) {
+      int p_ctas = 0;
+      ProbeArgs PA;
+      if ((rc = probe_buckets(*probes, f0 + lo, n, n_frames, dp.W, 0, 0, 0, 0, 0, 0, &PA))) return rc;
+      if ((e = flights_probe_prepare(R.fnw, R.fsmem, &p_ctas)) != cudaSuccess) return cuda_fail(e, "k_replay_flights (probes) attributes");
+      if (p_ctas < 1) { set_error("resident engine (probes): %zu B of shared memory do not fit an SM", R.fsmem); return UQS_ERR_CUDA; }
+      KernelTimer t_rep(2, s);
+      e = flights_probe_launch(R.fnw, (unsigned)std::min<long long>(n, (long long)p_ctas * g_ctx.sm_count), R.fsmem, s, FA, PA);
+      t_rep.stop();
+      if (e != cudaSuccess) return cuda_fail(e, "k_replay_flights (probes) launch");
+      g_ctx.launches += 2;
+      return UQS_OK;
+    }
+    const unsigned fgrid = (unsigned)std::min<long long>(n, (long long)R.f_ctas * g_ctx.sm_count);
+    KernelTimer t_rep(2, s);
+    e = flights_launch(R.fnw, g_ctx.flight_fan, g_ctx.flight_prod, fgrid, R.fsmem, s, FA);
+    t_rep.stop();
+    if (e != cudaSuccess) return cuda_fail(e, "k_replay_flights launch");
+    g_ctx.launches += 2;
+    return UQS_OK;
+  };
+
+  // the sub-tile replay of flights [lo, lo + n) on the library stream
+  auto replay_tiles = [&](int f0, int lo, int n) -> int {
     // sub-tiles nearest the grid centre first (trajectories stay within 60 % of the half-extent,
     // so those are the heavy ones); cached per geometry
     if (g_ctx.w->order_nsx != nsx || g_ctx.w->order_nsy != nsy) {
@@ -434,17 +455,17 @@ int replay_device(const DevParams& dp, int n_flights, int n_frames, const float*
     }
     ReplayArgs A;
     A.tile_order = (const uint32_t*)g_ctx.w->order.p;
-    A.n_flights = nf;
-    A.frames = (const uint4*)g_ctx.w->frames.p;
-    A.groups = (const uint2*)g_ctx.w->groups.p;
-    A.rays = (const uint2*)g_ctx.w->rays.p;
-    A.grids = grids + (size_t)f0 * dp.W * dp.H;
+    A.n_flights = n;
+    A.frames = frames + (size_t)lo * n_frames;
+    A.groups = groups + (size_t)lo * gpf;
+    A.rays = rays + (size_t)lo * n_frames * 32;
+    A.grids = grids + (size_t)(f0 + lo) * dp.W * dp.H;
     A.job_counter = counters + 8;
-    A.total_jobs = (unsigned long long)nf * nsx * nsy * slices;
+    A.total_jobs = (unsigned long long)n * nsx * nsy * slices;
     A.slices = slices; A.groups_per_slice = gps; A.pitch_cells = pitch_cells;
     A.maps = nullptr;
     if (slices > 1) {
-      if ((rc = g_ctx.w->maps.ensure((size_t)nf * (slices - 1) * dp.W * dp.H * sizeof(uint32_t)))) return rc;
+      if ((rc = g_ctx.w->maps.ensure((size_t)n * (slices - 1) * dp.W * dp.H * sizeof(uint32_t)))) return rc;
       A.maps = (uint32_t*)g_ctx.w->maps.p;
     }
     A.n_frames = n_frames; A.groups_per_flight = gpf;
@@ -459,21 +480,101 @@ int replay_device(const DevParams& dp, int n_flights, int n_frames, const float*
     unsigned long long want = (A.total_jobs + kReplayWarps - 1) / kReplayWarps;
     unsigned grid = (unsigned)std::min<unsigned long long>(want, (unsigned long long)ctas_per_sm * g_ctx.sm_count);
     ProbeArgs PA;
-    if (probes && (rc = probe_buckets(*probes, f0, nf, n_frames, dp.W, slices, gps, sw, sh, nsx, nsy, &PA))) return rc;
+    if (probes && (rc = probe_buckets(*probes, f0 + lo, n, n_frames, dp.W, slices, gps, sw, sh, nsx, nsy, &PA))) return rc;
     KernelTimer t_rep(2);
     e = tiles_launch(probes != nullptr, grid, smem, st, A, probes ? PA : ProbeArgs{});
     if (e == cudaSuccess && probes && slices > 1 &&     // before slice 0's values are overwritten
         (rc = probe_resolve_slices(PA, (int)probes->slots(), A.grids, A.maps, dp.W, dp.H, slices, gps)))
       return rc;
     if (e == cudaSuccess && slices > 1) {
-      const size_t cells = (size_t)dp.W * rows * nf;
-      k_compose_slices<<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(A.grids, A.maps, nf, dp.W, dp.H, slices, row0, rows);
+      const size_t cells = (size_t)dp.W * rows * n;
+      k_compose_slices<<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(A.grids, A.maps, n, dp.W, dp.H, slices, row0, rows);
       e = cudaGetLastError();
       g_ctx.launches += 1;
     }
     t_rep.stop();
     if (e != cudaSuccess) return cuda_fail(e, "k_replay_tiles launch");
     g_ctx.launches += 2;
+    return UQS_OK;
+  };
+
+  // Overlapped schedule (resident engine, no probes): the set-up of chunk k + 1 runs, in 256-thread blocks on a
+  // low-priority stream, in the SM resources and issue slots the replay of chunk k leaves over; the replays alternate
+  // between two high-priority streams, so that the next one fills the SMs as the previous one's CTAs drain.  The first
+  // chunk is about one wave of resident CTAs (its set-up is the only one exposed), the later ones `setup_overlap` waves
+  // (the last one up to twice that: a fraction of a wave replayed on its own would end on a ragged tail).  Measured on
+  // a B200 (profiles/r3_setup_overlap_ab.log): calls with less than one such later chunk lose more than they hide.
+  const bool overlap = g_ctx.setup_overlap > 0 && may_reside && !probes && !g_ctx.chip_shared;
+  // four CTAs per SM, before any box is known: the wave of config 3's resident replay (4 CTAs of 8 warps)
+  const int wave0 = g_ctx.sm_count * 4;
+
+  for (int f0 = 0; f0 < n_flights; f0 += chunk) {
+    const int nf = std::min(chunk, n_flights - f0);
+    int done = 0;                                            // flights of this chunk set up so far
+    if (overlap && nf > wave0) {
+      Resident R;
+      if ((rc = setup(f0, 0, wave0, st, false)) || (rc = configure(0, wave0, st, &R))) return rc;
+      done = wave0;
+      bool fits = false;
+      if (R.resident && (e = setup256_fits_beside(R.fnw, g_ctx.flight_fan, g_ctx.flight_prod, R.fsmem, R.f_ctas, &fits)) != cudaSuccess)
+        return cuda_fail(e, "k_ray_setup256 attributes");
+      const long long later = (long long)g_ctx.setup_overlap * R.f_ctas * g_ctx.sm_count;
+      if (fits && nf - wave0 >= later) {
+        if (!g_ctx.aux_setup) {
+          int lo_pri = 0, hi_pri = 0;
+          e = cudaDeviceGetStreamPriorityRange(&lo_pri, &hi_pri);
+          if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&g_ctx.aux_setup, cudaStreamNonBlocking, lo_pri);
+          if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&g_ctx.aux_replay[0], cudaStreamNonBlocking, hi_pri);
+          if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&g_ctx.aux_replay[1], cudaStreamNonBlocking, hi_pri);
+          if (e == cudaSuccess) e = cudaEventCreateWithFlags(&g_ctx.aux_ev, cudaEventDisableTiming);
+          if (e != cudaSuccess) return cuda_fail(e, "set-up overlap streams");
+        }
+        cudaStream_t ss = g_ctx.aux_setup, *rs = g_ctx.aux_replay;
+        // every internal stream starts after the library stream's work so far (inputs, zeroed stats)
+        e = cudaEventRecord(g_ctx.aux_ev, st);
+        for (cudaStream_t s : { ss, rs[0], rs[1] })
+          if (e == cudaSuccess) e = cudaStreamWaitEvent(s, g_ctx.aux_ev, 0);
+        if (e != cudaSuccess) return cuda_fail(e, "set-up overlap join");
+        if ((rc = replay_resident(R, f0, 0, wave0, rs[0], counters + 8))) return rc;
+        int box_w = g_ctx.w->box_w, box_h = g_ctx.w->box_h;       // the boxes of the chunk's flights, all of them
+        for (int lo = wave0, k = 1, n = 0; lo < nf; lo += n, k++) {
+          n = nf - lo < 2 * later ? nf - lo : (int)later;
+          if ((rc = setup(f0, lo, n, ss, true)) || (rc = configure(lo, n, ss, &R))) return rc;
+          box_w = std::max(box_w, g_ctx.w->box_w); box_h = std::max(box_h, g_ctx.w->box_h);
+          g_ctx.overlap_chunks += 1;
+          if (R.resident) {
+            if ((rc = replay_resident(R, f0, lo, n, rs[k & 1], counters + 8 + (k & 1)))) return rc;
+          } else {
+            // a chunk whose boxes do not fit: the sub-tile engine, after both replay streams
+            for (int i = 0; i < 2 && e == cudaSuccess; i++)
+              if ((e = cudaEventRecord(g_ctx.aux_ev, rs[i])) == cudaSuccess) e = cudaStreamWaitEvent(st, g_ctx.aux_ev, 0);
+            if (e != cudaSuccess) return cuda_fail(e, "set-up overlap join");
+            if ((rc = replay_tiles(f0, lo, n))) return rc;
+            for (int i = 0; i < 2 && e == cudaSuccess; i++)
+              if ((e = cudaEventRecord(g_ctx.aux_ev, st)) == cudaSuccess) e = cudaStreamWaitEvent(rs[i], g_ctx.aux_ev, 0);
+            if (e != cudaSuccess) return cuda_fail(e, "set-up overlap join");
+          }
+        }
+        // the library stream (and so any event the caller records on it) covers all of the call's work
+        for (cudaStream_t s : { ss, rs[0], rs[1] })
+          if (e == cudaSuccess && (e = cudaEventRecord(g_ctx.aux_ev, s)) == cudaSuccess) e = cudaStreamWaitEvent(st, g_ctx.aux_ev, 0);
+        if (e != cudaSuccess) return cuda_fail(e, "set-up overlap join");
+        g_ctx.w->boxes_valid = nf == n_flights;
+        g_ctx.w->boxes_n = nf; g_ctx.w->box_w = box_w; g_ctx.w->box_h = box_h;
+        continue;
+      }
+      // no room beside the replay's CTAs: the serial schedule, the rest of the chunk set up behind the first wave
+    }
+    if ((rc = setup(f0, done, nf - done, st, false))) return rc;
+    if (may_reside) {
+      Resident R;
+      if ((rc = configure(0, nf, st, &R))) return rc;
+      if (R.resident) {
+        if ((rc = replay_resident(R, f0, 0, nf, st, counters + 8))) return rc;
+        continue;
+      }
+    }
+    if ((rc = replay_tiles(f0, 0, nf))) return rc;
   }
   return UQS_OK;
 }
@@ -675,6 +776,12 @@ void context_shutdown(Context& c) {
   c.release_all();
   if (c.own_stream) cudaStreamDestroy(c.own_stream);
   c.own_stream = nullptr;
+  for (cudaStream_t* s : { &c.aux_setup, &c.aux_replay[0], &c.aux_replay[1] }) {
+    if (*s) cudaStreamDestroy(*s);
+    *s = nullptr;
+  }
+  if (c.aux_ev) cudaEventDestroy(c.aux_ev);
+  c.aux_ev = nullptr;
   c.ready = false;
 }
 
@@ -776,6 +883,15 @@ int uqs_set_k0_bias(int steps) {
   g_ctx.k0_bias = steps < 0 ? 0 : (steps > 8 ? 8 : steps);
   return UQS_OK;
 }
+
+/* Schedule of the resident engine's device calls: n > 0 = the ray set-up of each chunk of n resident waves runs beside
+ * the previous chunk's replay, 0 = set-up and replay in turn, -1 = the built-in choice.  Identical bytes. */
+int uqs_set_setup_overlap(int waves) {
+  g_ctx.setup_overlap = waves < 0 ? kDefaultSetupOverlap : std::min(waves, 64);
+  return UQS_OK;
+}
+
+int uqs_setup_overlap_chunks(void) { return g_ctx.overlap_chunks; }
 
 int uqs_set_fan_layout(int on) {
   g_ctx.flight_fan = on < 0 ? kDefaultFanLayout : (on ? 1 : 0);

@@ -12,6 +12,8 @@ namespace uqs {
 
 constexpr int kDefaultDecodeWarp = 0;           // resident engine: 1 = an extra warp per CTA that only decodes (measured choice)
 constexpr int kDefaultFanLayout = 0;            // resident engine: 0 = 32 beams x 1 step, 1 = 8 beams x 4 steps (measured choice)
+constexpr int kDefaultSetupOverlap = 2;         // resident engine: resident waves per chunk whose ray set-up runs beside the
+                                                //   previous chunk's replay (0 = set-up and replay in turn)
 
 // grow-only device buffer
 struct DevBuf {
@@ -57,6 +59,11 @@ struct Context {
   int pitch_mod = -1;                           // experiment: resident row pitch in words mod 32 (uqs_set_resident_pitch_mod)
   int flight_prod = kDefaultDecodeWarp;         // dedicated decode warp (uqs_set_decode_warp)
   int flight_fan = kDefaultFanLayout;           // lane layout of its free-space steps (uqs_set_fan_layout)
+  int setup_overlap = kDefaultSetupOverlap;     // uqs_set_setup_overlap
+  int overlap_chunks = 0;                       // chunks of the last device replay set up beside a replay
+  cudaStream_t aux_setup = nullptr;             // the overlapped schedule's streams (replay_device): set-up (low priority)
+  cudaStream_t aux_replay[2] = { nullptr, nullptr };   //   and replays of alternate chunks (high priority)
+  cudaEvent_t aux_ev = nullptr;
   int host_chunk = 0;                           // flights per chunk of the host-buffer pipeline (0 = auto)
   bool copy_only = false;                       // measurement: host-buffer calls skip their kernels (uqs_set_copy_only)
   bool chip_shared = false;                     // a multi-chunk host-buffer call is in flight: chunks share the chip

@@ -247,6 +247,156 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
       : "memory");
 }
 
+// The per-frame pieces of the ray set-up, shared by the 1024- and 256-thread kernels below.  A warp holds one frame,
+// lane = beam.  setup_beam_end: the beam's end point (everything that does not need the frame's start cell); the range
+// readings are read at rb (staged in shared memory after the block's bulk copy, or straight from the log).
+__device__ __forceinline__ int setup_beam_end(const DevParams& p, const float* __restrict__ x, const float* __restrict__ y,
+                                              const float* __restrict__ yaw_deg, const uint8_t* __restrict__ kind, size_t fi,
+                                              int lane, bool staged, uint32_t bar_sa, const unsigned char* rb, bool u16,
+                                              float& ex, float& ey, bool& hit, bool& raw) {
+  const float px = x[fi], py = y[fi], third = yaw_deg[fi];
+  raw = kind != nullptr && kind[fi] == 1;
+  if (staged) mbar_wait(bar_sa, 0);
+  const float* rr = reinterpret_cast<const float*>(rb);
+  if (!raw) {
+    const float dist = u16 ? range_from_mm(reinterpret_cast<const uint16_t*>(rb)[lane]) : rr[lane];
+    return beam_endpoint(p, px, py, third, dist, lane, ex, ey, hit);
+  }
+  ex = third;
+  ey = rr[0];
+  hit = rr[1] != 0.0f;
+  return (lane == 0) ? 1 : 0;
+}
+
+// The rest of frame fi once its start cell org[0..1] (and, RECENTER, org[2..5]: the origin at the frame and its offset
+// into the global frame) is known: the ray record of every beam, K0 and the frame record.  Returns the frame's touched
+// box (warp-wide) and this lane's counters.
+template <bool RECENTER>
+__device__ __forceinline__ void setup_beam_finish(const DevParams& p, const int* org, size_t fi, int lane, int st, float ex,
+                                                  float ey, bool hit, bool raw, int want_k0,
+                                                  const uint32_t* __restrict__ inv_table, uint4* __restrict__ frames,
+                                                  uint2* __restrict__ rays, int& xmin, int& xmax, int& ymin, int& ymax,
+                                                  unsigned& cells, int& accepted, int& skipped, int& domain) {
+  xmin = 0x7fff; xmax = 0; ymin = 0x7fff; ymax = 0;
+  cells = 0;
+  accepted = 0; skipped = 0; domain = 0;
+  const bool have_o = org[0] >= 0;
+  // window cells; in the global frame for RECENTER (-1 stays the off-grid mark)
+  const int gx0 = org[0] + (RECENTER && have_o ? org[RECENTER ? 4 : 0] : 0);
+  const int gy0 = org[1] + (RECENTER && have_o ? org[RECENTER ? 5 : 0] : 0);
+  uint32_t w0 = 0, w1 = 0;
+  if (st < 0) {
+    domain = 1;
+  } else if (st > 0 && have_o) {
+    int gx1, gy1;
+    const bool on_grid = RECENTER ? world_to_grid_at(p, __int_as_float(org[RECENTER ? 2 : 0]),
+                                                     __int_as_float(org[RECENTER ? 3 : 0]), ex, ey, gx1, gy1)
+                                  : world_to_grid(p, ex, ey, gx1, gy1);
+    if (on_grid) {
+      if (RECENTER) { gx1 += org[RECENTER ? 4 : 0]; gy1 += org[RECENTER ? 5 : 0]; }
+      const int dx = gx1 - gx0, dy = gy1 - gy0;
+      const int m = max(abs(dx), abs(dy));
+      if (m > kMaxRayCells) {
+        domain = 1;
+      } else {
+        w0 = ((uint32_t)dx & 0xfffu) | (((uint32_t)dy & 0xfffu) << 12) | (hit ? kRayHit : 0u) |
+             kRayValid;
+        w1 = __ldg(&inv_table[m]);                           // ceil(2^31 / m), 0 for m == 0
+        xmin = min(gx0, gx1); xmax = max(gx0, gx1);
+        ymin = min(gy0, gy1); ymax = max(gy0, gy1);
+        cells = (unsigned)m + 1u;
+        accepted = 1;
+      }
+    }
+  }
+  if (!accepted && !domain && !(raw && lane != 0)) skipped = 1;
+  rays[fi * 32 + lane] = make_uint2(w0, w1);
+
+  // K0: two accepted beams of this frame can share a cell only at steps k < K0 (DESIGN.md,
+  // "same-k lemma" and ring coordinate).  sigma = position of the beam's direction on the
+  // unit max-norm ring, in [0,8); cells of step k sit within 1/2 of k*sigma on the ring of
+  // radius k, so beams i,j are apart for every k > 1/|sigma_i - sigma_j|.  Conservative
+  // float arithmetic (K0 may only be too large) -- it gates a fast path, never a result.
+  int k0 = 0;
+  bool frame_sorted = false;
+  if (want_k0) {                       // only the grid-resident engine reads K0 and the order flag
+    const int dx = sext12(w0), dy = sext12(w0 >> 12);
+    const int adx = abs(dx), ady = abs(dy);
+    const bool xmaj = adx >= ady;
+    const int m = accepted ? (xmaj ? adx : ady) : -1;
+    const int n = xmaj ? ady : adx;
+    const bool xpos = dx >= 0, ypos = dy >= 0;
+    float ra, rb;
+    if (xmaj) { ra = xpos ? (ypos ? 0.f : 8.f) : 4.f; rb = (xpos == ypos) ? 1.f : -1.f; }
+    else      { ra = ypos ? 2.f : 6.f;                rb = (xpos == ypos) ? -1.f : 1.f; }
+    float sigma = (m > 0) ? ra + rb * __fdividef((float)n, (float)m) : 0.f;   // feeds the conservative K0 only
+    if (sigma >= 8.f) sigma -= 8.f;
+    const int mmax = __reduce_max_sync(0xffffffffu, m);
+    const unsigned any = __ballot_sync(0xffffffffu, m >= 0);
+    const unsigned dir = __ballot_sync(0xffffffffu, m >= 1);     // beams that have a direction
+    // Fast path: beams are issued in angular order, so their ring coordinates are normally sorted and the
+    // closest pair is a pair of neighbours.  Dropping the per-pair length cap only enlarges the bound.
+    const unsigned above = dir & ~(0xffffffffu >> (31 - lane));
+    const int nxt = above ? (__ffs(above) - 1) : (__ffs(dir) - 1);
+    const float sn = __shfl_sync(0xffffffffu, sigma, nxt & 31);
+    const bool has_dir = m >= 1;
+    float gap = sn - sigma;                                           // to the next beam, cyclically (K0 only)
+    // exact order test: sigma = A + s*n/m as integers (A in {0,2,4,6,8}); sigma_i <= sigma_next  <=>
+    // (A' - A)*m*m' + s'*n'*m - s*n*m' >= 0.  8 is the same direction as 0.
+    int A = (int)ra, sgn_n = (rb > 0.f) ? n : -n;
+    if (A == 8 && n == 0) A = 0;
+    const int pk = (A << 24) | ((sgn_n & 0xfff) << 12) | (max(m, 0) & 0xfff);     // m <= 1024 < 4096
+    const int pn = __shfl_sync(0xffffffffu, pk, nxt & 31);
+    const int A2 = pn >> 24, n2s = (pn << 8) >> 20, m2 = pn & 0xfff;
+    const int order = (A2 - A) * m * m2 + n2s * m - sgn_n * m2;
+    const bool wraps = has_dir && order < 0;
+    // the float gap only feeds the (conservative) K0: make it agree with the exact order first
+    if (order == 0) gap = 0.f;                     // parallel beams: shared up to the shorter one's end
+    else if (order < 0) gap += 8.f;                // the one passage through 8 -> 0
+    gap = fmaxf(gap, 0.f);
+    // circularly sorted <=> the cyclic sequence passes 8 -> 0 at most once
+    const bool sorted = __popc(__ballot_sync(0xffffffffu, wraps)) <= 1;
+    frame_sorted = sorted;
+    if (__popc(any) >= 2) {
+      if (sorted || __popc(dir) < 2) {
+        int kk = 1;                                                   // the start cell is shared by all beams
+        // no shared cell once k*gap > 1: steps 0..floor(1/gap) may collide (the float slack only enlarges it)
+        if (has_dir && __popc(dir) >= 2) kk = (gap > 1e-4f) ? (int)(1.0f / (gap - 2e-5f)) + 1 : 0x7fffffff;
+        k0 = min(__reduce_max_sync(0xffffffffu, kk), mmax + 1);
+      } else {
+        // beams out of angular order (very short rays quantise coarsely): exact all-pairs bound
+#pragma unroll 4
+        for (int j = 1; j <= 16; j++) {
+          const int pl = (lane + j) & 31;
+          const float sp = __shfl_sync(0xffffffffu, sigma, pl);
+          const int mp = __shfl_sync(0xffffffffu, m, pl);
+          float dlt = fabsf(sigma - sp);
+          dlt = fminf(dlt, 8.f - dlt);
+          int kk = (dlt > 1e-4f) ? (int)(1.0f / (dlt - 2e-5f)) + 1 : 0x7fffffff;
+          if (m < 1 || mp < 1) kk = 1;
+          kk = min(kk, min(m, mp) + 1);          // a beam has no step beyond its own length
+          if (m >= 0 && mp >= 0) k0 = max(k0, kk);
+        }
+        k0 = __reduce_max_sync(0xffffffffu, k0);
+      }
+    }
+    // want_k0 - 1: measurement bias (uqs_set_k0_bias), added after the cap at mmax + 1 so that it cannot overflow the
+    // 0x7fffffff of parallel beams, and capped the same way (a larger K0 is always safe: more collision-checked steps)
+    const int bias = want_k0 - 1;
+    k0 = min(k0, mmax + 1 - bias) + bias;
+  }
+
+  xmin = __reduce_min_sync(0xffffffffu, xmin);
+  xmax = __reduce_max_sync(0xffffffffu, xmax);
+  ymin = __reduce_min_sync(0xffffffffu, ymin);
+  ymax = __reduce_max_sync(0xffffffffu, ymax);
+  if (lane == 0)
+    frames[fi] = make_uint4(have_o ? ((uint32_t)gx0 | ((uint32_t)k0 << 16)) : 0u,
+                            have_o ? ((uint32_t)gy0 | kFrameHasOrigin | (frame_sorted ? kFrameSorted : 0u)) : 0u,
+                            (uint32_t)xmin | ((uint32_t)xmax << 16),
+                            (uint32_t)ymin | ((uint32_t)ymax << 16));
+}
+
 // grid = (groups_per_flight, n_flights); block = 1024 = 32 frames x 32 beams.
 // kind == nullptr: every entry is a frame (pose + 32 ranges).
 // kind[i] == 1   : entry i is one raw ray raycast_update(x0,y0,x1,y1,hit) stored as
@@ -328,141 +478,15 @@ k_ray_setup(const __grid_constant__ DevParams p, int n_frames, const float* __re
   float ex = 0.f, ey = 0.f;
   bool hit = false, raw = false;
   int st = 0;
-  if (live) {
-    const float px = x[fi], py = y[fi], third = yaw_deg[fi];
-    raw = kind != nullptr && kind[fi] == 1;
-    if (staged) mbar_wait(bar_sa, 0);
-    const unsigned char* rb = staged ? reinterpret_cast<const unsigned char*>(s_rng) + (size_t)w * rbytes : ranges_b + fi * rbytes;
-    const float* rr = reinterpret_cast<const float*>(rb);
-    if (!raw) {
-      const float dist = u16 ? range_from_mm(reinterpret_cast<const uint16_t*>(rb)[lane]) : rr[lane];
-      st = beam_endpoint(p, px, py, third, dist, lane, ex, ey, hit);
-    } else {
-      st = (lane == 0) ? 1 : 0;
-      ex = third;
-      ey = rr[0];
-      hit = rr[1] != 0.0f;
-    }
-  }
+  if (live)
+    st = setup_beam_end(p, x, y, yaw_deg, kind, fi, lane, staged, bar_sa,
+                        staged ? reinterpret_cast<const unsigned char*>(s_rng) + (size_t)w * rbytes : ranges_b + fi * rbytes, u16,
+                        ex, ey, hit, raw);
   __syncthreads();
 
-  if (live) {
-    const bool have_o = s_org[w][0] >= 0;
-    // window cells; in the global frame for RECENTER (-1 stays the off-grid mark)
-    const int gx0 = s_org[w][0] + (RECENTER && have_o ? s_org[w][RECENTER ? 4 : 0] : 0);
-    const int gy0 = s_org[w][1] + (RECENTER && have_o ? s_org[w][RECENTER ? 5 : 0] : 0);
-    uint32_t w0 = 0, w1 = 0;
-    if (st < 0) {
-      domain = 1;
-    } else if (st > 0 && have_o) {
-      int gx1, gy1;
-      const bool on_grid = RECENTER ? world_to_grid_at(p, __int_as_float(s_org[w][RECENTER ? 2 : 0]),
-                                                       __int_as_float(s_org[w][RECENTER ? 3 : 0]), ex, ey, gx1, gy1)
-                                    : world_to_grid(p, ex, ey, gx1, gy1);
-      if (on_grid) {
-        if (RECENTER) { gx1 += s_org[w][RECENTER ? 4 : 0]; gy1 += s_org[w][RECENTER ? 5 : 0]; }
-        const int dx = gx1 - gx0, dy = gy1 - gy0;
-        const int m = max(abs(dx), abs(dy));
-        if (m > kMaxRayCells) {
-          domain = 1;
-        } else {
-          w0 = ((uint32_t)dx & 0xfffu) | (((uint32_t)dy & 0xfffu) << 12) | (hit ? kRayHit : 0u) |
-               kRayValid;
-          w1 = __ldg(&inv_table[m]);                           // ceil(2^31 / m), 0 for m == 0
-          xmin = min(gx0, gx1); xmax = max(gx0, gx1);
-          ymin = min(gy0, gy1); ymax = max(gy0, gy1);
-          cells = (unsigned)m + 1u;
-          accepted = 1;
-        }
-      }
-    }
-    if (!accepted && !domain && !(raw && lane != 0)) skipped = 1;
-    rays[fi * 32 + lane] = make_uint2(w0, w1);
-
-    // K0: two accepted beams of this frame can share a cell only at steps k < K0 (DESIGN.md,
-    // "same-k lemma" and ring coordinate).  sigma = position of the beam's direction on the
-    // unit max-norm ring, in [0,8); cells of step k sit within 1/2 of k*sigma on the ring of
-    // radius k, so beams i,j are apart for every k > 1/|sigma_i - sigma_j|.  Conservative
-    // float arithmetic (K0 may only be too large) -- it gates a fast path, never a result.
-    int k0 = 0;
-    bool frame_sorted = false;
-    if (want_k0) {                       // only the grid-resident engine reads K0 and the order flag
-      const int dx = sext12(w0), dy = sext12(w0 >> 12);
-      const int adx = abs(dx), ady = abs(dy);
-      const bool xmaj = adx >= ady;
-      const int m = accepted ? (xmaj ? adx : ady) : -1;
-      const int n = xmaj ? ady : adx;
-      const bool xpos = dx >= 0, ypos = dy >= 0;
-      float ra, rb;
-      if (xmaj) { ra = xpos ? (ypos ? 0.f : 8.f) : 4.f; rb = (xpos == ypos) ? 1.f : -1.f; }
-      else      { ra = ypos ? 2.f : 6.f;                rb = (xpos == ypos) ? -1.f : 1.f; }
-      float sigma = (m > 0) ? ra + rb * __fdividef((float)n, (float)m) : 0.f;   // feeds the conservative K0 only
-      if (sigma >= 8.f) sigma -= 8.f;
-      const int mmax = __reduce_max_sync(0xffffffffu, m);
-      const unsigned any = __ballot_sync(0xffffffffu, m >= 0);
-      const unsigned dir = __ballot_sync(0xffffffffu, m >= 1);     // beams that have a direction
-      // Fast path: beams are issued in angular order, so their ring coordinates are normally sorted and the
-      // closest pair is a pair of neighbours.  Dropping the per-pair length cap only enlarges the bound.
-      const unsigned above = dir & ~(0xffffffffu >> (31 - lane));
-      const int nxt = above ? (__ffs(above) - 1) : (__ffs(dir) - 1);
-      const float sn = __shfl_sync(0xffffffffu, sigma, nxt & 31);
-      const bool has_dir = m >= 1;
-      float gap = sn - sigma;                                           // to the next beam, cyclically (K0 only)
-      // exact order test: sigma = A + s*n/m as integers (A in {0,2,4,6,8}); sigma_i <= sigma_next  <=>
-      // (A' - A)*m*m' + s'*n'*m - s*n*m' >= 0.  8 is the same direction as 0.
-      int A = (int)ra, sgn_n = (rb > 0.f) ? n : -n;
-      if (A == 8 && n == 0) A = 0;
-      const int pk = (A << 24) | ((sgn_n & 0xfff) << 12) | (max(m, 0) & 0xfff);     // m <= 1024 < 4096
-      const int pn = __shfl_sync(0xffffffffu, pk, nxt & 31);
-      const int A2 = pn >> 24, n2s = (pn << 8) >> 20, m2 = pn & 0xfff;
-      const int order = (A2 - A) * m * m2 + n2s * m - sgn_n * m2;
-      const bool wraps = has_dir && order < 0;
-      // the float gap only feeds the (conservative) K0: make it agree with the exact order first
-      if (order == 0) gap = 0.f;                     // parallel beams: shared up to the shorter one's end
-      else if (order < 0) gap += 8.f;                // the one passage through 8 -> 0
-      gap = fmaxf(gap, 0.f);
-      // circularly sorted <=> the cyclic sequence passes 8 -> 0 at most once
-      const bool sorted = __popc(__ballot_sync(0xffffffffu, wraps)) <= 1;
-      frame_sorted = sorted;
-      if (__popc(any) >= 2) {
-        if (sorted || __popc(dir) < 2) {
-          int kk = 1;                                                   // the start cell is shared by all beams
-          // no shared cell once k*gap > 1: steps 0..floor(1/gap) may collide (the float slack only enlarges it)
-          if (has_dir && __popc(dir) >= 2) kk = (gap > 1e-4f) ? (int)(1.0f / (gap - 2e-5f)) + 1 : 0x7fffffff;
-          k0 = min(__reduce_max_sync(0xffffffffu, kk), mmax + 1);
-        } else {
-          // beams out of angular order (very short rays quantise coarsely): exact all-pairs bound
-#pragma unroll 4
-          for (int j = 1; j <= 16; j++) {
-            const int pl = (lane + j) & 31;
-            const float sp = __shfl_sync(0xffffffffu, sigma, pl);
-            const int mp = __shfl_sync(0xffffffffu, m, pl);
-            float dlt = fabsf(sigma - sp);
-            dlt = fminf(dlt, 8.f - dlt);
-            int kk = (dlt > 1e-4f) ? (int)(1.0f / (dlt - 2e-5f)) + 1 : 0x7fffffff;
-            if (m < 1 || mp < 1) kk = 1;
-            kk = min(kk, min(m, mp) + 1);          // a beam has no step beyond its own length
-            if (m >= 0 && mp >= 0) k0 = max(k0, kk);
-          }
-          k0 = __reduce_max_sync(0xffffffffu, k0);
-        }
-      }
-      // want_k0 - 1: measurement bias (uqs_set_k0_bias), added after the cap at mmax + 1 so that it cannot overflow the
-      // 0x7fffffff of parallel beams, and capped the same way (a larger K0 is always safe: more collision-checked steps)
-      const int bias = want_k0 - 1;
-      k0 = min(k0, mmax + 1 - bias) + bias;
-    }
-
-    xmin = __reduce_min_sync(0xffffffffu, xmin);
-    xmax = __reduce_max_sync(0xffffffffu, xmax);
-    ymin = __reduce_min_sync(0xffffffffu, ymin);
-    ymax = __reduce_max_sync(0xffffffffu, ymax);
-    if (lane == 0)
-      frames[fi] = make_uint4(have_o ? ((uint32_t)gx0 | ((uint32_t)k0 << 16)) : 0u,
-                              have_o ? ((uint32_t)gy0 | kFrameHasOrigin | (frame_sorted ? kFrameSorted : 0u)) : 0u,
-                              (uint32_t)xmin | ((uint32_t)xmax << 16),
-                              (uint32_t)ymin | ((uint32_t)ymax << 16));
-  }
+  if (live)
+    setup_beam_finish<RECENTER>(p, s_org[w], fi, lane, st, ex, ey, hit, raw, want_k0, inv_table, frames, rays, xmin, xmax,
+                                ymin, ymax, cells, accepted, skipped, domain);
   // per-warp counters (two packed words), then one block-level reduce by warp 0
   const unsigned as = __reduce_add_sync(0xffffffffu, (unsigned)accepted | ((unsigned)skipped << 16));
   const unsigned cd = __reduce_add_sync(0xffffffffu, cells | ((unsigned)domain << 21));       // cells <= 32*1025 per warp
@@ -490,11 +514,110 @@ k_ray_setup(const __grid_constant__ DevParams p, int n_frames, const float* __re
   }
 }
 
+// The same records from blocks of 256 threads = 8 warps x 4 frames each (warp w holds frames w, w + 8, w + 16, w + 24
+// of the block's 32), at <= 32 registers: such a block fits beside the resident replay's CTAs on an SM, so the set-up of
+// the next chunk of flights runs in the replay's idle issue slots (replay_device).  A block still owns one 32-frame
+// group (the group boxes are per 32 frames).  The start cells take the place of warp 7's first end point before the
+// barrier, so that the barrier waits for no more than one end point per warp.  Plain frames only (no RECENTER).
+__global__ void __launch_bounds__(256, 8)
+k_ray_setup256(const __grid_constant__ DevParams p, int n_frames, const float* __restrict__ x,
+               const float* __restrict__ y, const float* __restrict__ yaw_deg,
+               const float* __restrict__ ranges, const uint8_t* __restrict__ kind, int want_k0,
+               const uint32_t* __restrict__ inv_table, uint4* __restrict__ frames, uint2* __restrict__ groups,
+               uint2* __restrict__ rays, unsigned long long* __restrict__ stats /* [4]: U, accepted, skipped, domain */) {
+  constexpr int kWarps = 8, kOrgWarp = kWarps - 1;
+  __shared__ __align__(128) float s_rng[32 * 32];
+  __shared__ __align__(8) unsigned long long s_bar;
+  __shared__ int s_box[4][32];                                    // per frame
+  __shared__ unsigned s_cnt[2][kWarps];                           // per warp
+  __shared__ int s_org[32][2];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int flight = blockIdx.y, g = blockIdx.x, groups_per_flight = gridDim.x;
+  const size_t fbase = (size_t)flight * n_frames;
+  const int nfr = min(32, n_frames - g * 32);                     // frames of this block
+
+  const bool u16 = p.ranges_u16 != 0;
+  const unsigned rbytes = u16 ? 64u : 128u;
+  const unsigned char* ranges_b = reinterpret_cast<const unsigned char*>(ranges);
+  const unsigned char* blk_ranges = ranges_b + (fbase + (size_t)g * 32) * rbytes;
+  const bool staged = (reinterpret_cast<size_t>(ranges) & 15) == 0;
+  const uint32_t bar_sa = (uint32_t)__cvta_generic_to_shared(&s_bar);
+  if (staged) {
+    if (threadIdx.x == 0) {
+      mbar_init(bar_sa, 1);
+      bulk_load_g2s((uint32_t)__cvta_generic_to_shared(s_rng), blk_ranges, (uint32_t)nfr * rbytes, bar_sa);
+    }
+    __syncthreads();
+  }
+
+  const size_t blk = fbase + (size_t)g * 32;                      // the block's first frame
+  const unsigned char* rsrc = staged ? reinterpret_cast<const unsigned char*>(s_rng) : blk_ranges;   // its range readings
+  float ex = 0.f, ey = 0.f;
+  bool hit = false, raw = false;
+  int st = 0;
+  if (w == kOrgWarp) {
+    int ox = -1, oy = -1;
+    const int fo = g * 32 + lane;
+    if (fo < n_frames && !world_to_grid(p, x[fbase + fo], y[fbase + fo], ox, oy)) ox = oy = -1;
+    s_org[lane][0] = ox;
+    s_org[lane][1] = oy;
+  } else if (w < nfr) {
+    st = setup_beam_end(p, x, y, yaw_deg, kind, blk + w, lane, staged, bar_sa, rsrc + w * rbytes, u16, ex, ey, hit, raw);
+  }
+  __syncthreads();
+
+  unsigned as = 0, cd = 0;                                         // this lane's counters, packed as below
+  auto finish = [&](int r) {
+    const size_t fi = blk + r;
+    int fx0, fx1, fy0, fy1, acc, skp, dom;
+    unsigned cl;
+    setup_beam_finish<false>(p, s_org[r], fi, lane, st, ex, ey, hit, raw, want_k0, inv_table, frames, rays, fx0, fx1, fy0,
+                             fy1, cl, acc, skp, dom);
+    if (lane == 0) { s_box[0][r] = fx0; s_box[1][r] = fx1; s_box[2][r] = fy0; s_box[3][r] = fy1; }
+    as += (unsigned)acc | ((unsigned)skp << 16);
+    cd += cl | ((unsigned)dom << 21);
+  };
+  if (w != kOrgWarp && w < nfr) finish(w);
+  for (int r = w == kOrgWarp ? w : w + kWarps; r < nfr; r += kWarps) {      // warp-uniform
+    st = setup_beam_end(p, x, y, yaw_deg, kind, blk + r, lane, staged, bar_sa, rsrc + r * rbytes, u16, ex, ey, hit, raw);
+    finish(r);
+  }
+  as = __reduce_add_sync(0xffffffffu, as);
+  cd = __reduce_add_sync(0xffffffffu, cd);                        // cells <= 4*32*1025 < 2^21 per warp
+  if (lane == 0) { s_cnt[0][w] = as; s_cnt[1][w] = cd; }
+  __syncthreads();
+  if (w == 0) {
+    const bool own = lane < kWarps, fr = lane < nfr;
+    const int gx0 = __reduce_min_sync(0xffffffffu, fr ? s_box[0][lane] : 0x7fff);
+    const int gx1 = __reduce_max_sync(0xffffffffu, fr ? s_box[1][lane] : 0);
+    const int gy0 = __reduce_min_sync(0xffffffffu, fr ? s_box[2][lane] : 0x7fff);
+    const int gy1 = __reduce_max_sync(0xffffffffu, fr ? s_box[3][lane] : 0);
+    const unsigned bas = __reduce_add_sync(0xffffffffu, own ? s_cnt[0][lane] : 0u);              // <= 1024 per field
+    const unsigned bcd = own ? s_cnt[1][lane] : 0u;
+    const unsigned bc = __reduce_add_sync(0xffffffffu, bcd & 0x1fffffu);                         // <= 1024*1025 < 2^21
+    const unsigned bd = __reduce_add_sync(0xffffffffu, bcd >> 21);
+    if (lane == 0)
+      groups[(size_t)flight * groups_per_flight + g] =
+          make_uint2((uint32_t)gx0 | ((uint32_t)gx1 << 16), (uint32_t)gy0 | ((uint32_t)gy1 << 16));
+    if (lane < 4) {
+      const unsigned long long t = lane == 0 ? bc : (lane == 1 ? (bas & 0xffffu) : (lane == 2 ? (bas >> 16) : bd));
+      if (t) atomicAdd(&stats[lane], t);
+    }
+  }
+}
+
 cudaError_t ray_setup_launch(dim3 grid, cudaStream_t st, const DevParams& p, int n_frames, const float* x, const float* y,
                              const float* yaw_deg, const float* ranges, const uint8_t* kind, int want_k0,
                              const uint32_t* inv_table, uint4* frames, uint2* groups, uint2* rays, unsigned long long* stats) {
   k_ray_setup<false><<<grid, 1024, 0, st>>>(p, n_frames, x, y, yaw_deg, ranges, kind, want_k0, inv_table, frames, groups, rays,
                                             stats, nullptr, nullptr, nullptr);
+  return cudaGetLastError();
+}
+
+cudaError_t ray_setup256_launch(dim3 grid, cudaStream_t st, const DevParams& p, int n_frames, const float* x, const float* y,
+                                const float* yaw_deg, const float* ranges, const uint8_t* kind, int want_k0,
+                                const uint32_t* inv_table, uint4* frames, uint2* groups, uint2* rays, unsigned long long* stats) {
+  k_ray_setup256<<<grid, 256, 0, st>>>(p, n_frames, x, y, yaw_deg, ranges, kind, want_k0, inv_table, frames, groups, rays, stats);
   return cudaGetLastError();
 }
 
@@ -1497,6 +1620,28 @@ cudaError_t flights_prepare(int nw, int fan, int prod, size_t smem, int* ctas_pe
   cudaError_t e = cudaFuncSetAttribute(flight_kernel(nw, fan, prod), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, flight_kernel(nw, fan, prod), flight_threads(nw, prod), smem);
+}
+
+cudaError_t setup256_fits_beside(int nw, int fan, int prod, size_t smem, int ctas, bool* fits) {
+  *fits = false;
+  int dev = 0, regs_sm = 0, smem_sm = 0, thr_sm = 0, blk_sm = 0, reserved = 0;
+  cudaFuncAttributes fr, fs;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e == cudaSuccess) e = cudaFuncGetAttributes(&fr, flight_kernel(nw, fan, prod));
+  if (e == cudaSuccess) e = cudaFuncGetAttributes(&fs, k_ray_setup256);
+  if (e == cudaSuccess) e = cudaDeviceGetAttribute(&regs_sm, cudaDevAttrMaxRegistersPerMultiprocessor, dev);
+  if (e == cudaSuccess) e = cudaDeviceGetAttribute(&smem_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, dev);
+  if (e == cudaSuccess) e = cudaDeviceGetAttribute(&thr_sm, cudaDevAttrMaxThreadsPerMultiProcessor, dev);
+  if (e == cudaSuccess) e = cudaDeviceGetAttribute(&blk_sm, cudaDevAttrMaxBlocksPerMultiprocessor, dev);
+  if (e == cudaSuccess) e = cudaDeviceGetAttribute(&reserved, cudaDevAttrReservedSharedMemoryPerBlock, dev);
+  if (e != cudaSuccess) return e;
+  auto warp_regs = [](int r) { return (long long)((r * 32 + 255) / 256) * 256; };     // allocated per warp in 256s
+  auto block_smem = [&](size_t b) { return (long long)((b + reserved + 127) / 128) * 128; };
+  const int rt = flight_threads(nw, prod);
+  const long long regs = (long long)ctas * (rt / 32) * warp_regs(fr.numRegs) + 8 * warp_regs(fs.numRegs);
+  const long long shm = (long long)ctas * block_smem(smem + fr.sharedSizeBytes) + block_smem(fs.sharedSizeBytes);
+  *fits = regs <= regs_sm && shm <= smem_sm && ctas * rt + 256 <= thr_sm && ctas + 1 <= blk_sm;
+  return cudaSuccess;
 }
 
 cudaError_t flights_launch(int nw, int fan, int prod, unsigned grid, size_t smem, cudaStream_t st, const FlightArgs& A) {

@@ -102,6 +102,13 @@ int pose_scan_threads();
 cudaError_t ray_setup_launch(dim3 grid, cudaStream_t st, const DevParams& p, int n_frames, const float* x, const float* y,
                              const float* yaw_deg, const float* ranges, const uint8_t* kind, int want_k0,
                              const uint32_t* inv_table, uint4* frames, uint2* groups, uint2* rays, unsigned long long* stats);
+// the same records from 256-thread blocks (8 warps x 4 frames), which fit beside the resident replay's CTAs on an SM
+cudaError_t ray_setup256_launch(dim3 grid, cudaStream_t st, const DevParams& p, int n_frames, const float* x, const float* y,
+                                const float* yaw_deg, const float* ranges, const uint8_t* kind, int want_k0,
+                                const uint32_t* inv_table, uint4* frames, uint2* groups, uint2* rays, unsigned long long* stats);
+// whether one k_ray_setup256 block fits on an SM beside `ctas` CTAs of the resident replay (nw, fan, prod) with `smem`
+// dynamic bytes each: registers, shared memory, threads and block slots
+cudaError_t setup256_fits_beside(int nw, int fan, int prod, size_t smem, int ctas, bool* fits);
 // the same for recentred flights: each frame is set up against its flight's origin at that frame, and its records are
 // in the flight's global frame (events, ev_start and s_min as in RecenterArgs)
 cudaError_t ray_setup_recenter_launch(dim3 grid, cudaStream_t st, const DevParams& p, int n_frames, const float* x,
